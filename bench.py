@@ -29,7 +29,10 @@ ENV_ID = "CartPoleContinuousSwingup-Gazebo-v0"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int,
+                    help="exact number of timed steps. Default 8192 for --impl b200: ~0.6 s of GPU load at the default "
+                         "size, long enough for the 100 ms clock sampler (far fewer steps give few or no clock samples); "
+                         "200 bounded samples for --impl reference")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=4 * 1048576,
@@ -42,8 +45,17 @@ def parse_args():
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the short measurements of the other BASELINE.json configurations (N=1 only)")
     ap.add_argument("--graph", action="store_true",
-                    help="replay the steps from a CUDA graph of 4 launches (for launch-bound small batches)")
-    return ap.parse_args()
+                    help="replay the steps from a CUDA graph of 4 launches (for launch-bound small batches); the "
+                         "steps of a timed block beyond whole 64-step replays run as eager rollouts")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (obs, reward, done of a fixed, seeded sample of rank "
+                         "0's envs, with their env_index) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 8192 if args.impl == "b200" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -422,6 +434,22 @@ def c3_strong(rank, world, local, peak, dist):
     return out
 
 
+def dump_outputs(env, directory, budget=48 << 20):
+    """Writes what the last step returned to its caller (obs, reward, done) as directory/<name>.npy, for all envs or, where
+    that exceeds `budget` bytes, for a fixed, seeded sample of them; env_index holds the env index of every row."""
+    import numpy as np
+    import torch
+    n = env.num_envs
+    rows = min(n, budget // (env.obs.element_size() * (env.nobs + 1) + 4 + 8))
+    idx = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    sel = torch.as_tensor(idx, device=env.obs.device)
+    out = {"obs": env.obs[sel].cpu().numpy(), "reward": env.reward[sel].cpu().numpy(),
+           "done": env.done[sel].to(torch.float32).cpu().numpy(), "env_index": idx.astype(np.float64)}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def run_b200(args):
     import numpy as np
     import torch
@@ -503,14 +531,14 @@ def run_b200(args):
 
     run_steps(args.warmup)
     barrier()
-    # One probe block sizes the repeat count: the timed region is a block of EXACTLY args.steps steps (barrier +
-    # synchronize on both sides, CUDA events, max over ranks), repeated at least 5 times and for at least 0.6 s of
-    # loaded time so that the clock sampler (100 ms period) sees the GPU under the load it is reporting on.
-    def timed_block():
+    # The timed region is EXACTLY args.steps steps, so that a run with the same arguments always ends in the same state.
+    # It is split into up to 5 blocks of whole launch groups (4 steps per rollout call, 64 per graph replay), each
+    # bracketed by barrier + synchronize and timed with CUDA events (max over ranks); the median block is reported.
+    def timed_block(count):
         barrier()
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record()
-        run_steps(args.steps)
+        run_steps(count)
         stop.record()
         barrier()
         t = torch.tensor([start.elapsed_time(stop)], dtype=torch.float64, device="cuda")
@@ -518,29 +546,31 @@ def run_b200(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    probe_ms = timed_block()
-    repeats = int(min(400, max(5, -(-600.0 // max(probe_ms, 1e-3)))))
+    unit = 64 if graph is not None else 4
+    nblocks = max(1, min(5, args.steps // unit))
+    size = args.steps // nblocks // unit * unit
+    sizes = [size] * (nblocks - 1) + [args.steps - size * (nblocks - 1)]
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     l0 = env.sim.launch_count()
-    blocks = [timed_block() for _ in range(repeats)]
-    launches = (env.sim.launch_count() - l0) // repeats
-    if graph is not None:
-        launches += 64 * (args.steps // 64)   # launches replayed from the CUDA graph are not seen by the host counter
+    blocks = [timed_block(count) for count in sizes]
+    launches = env.sim.launch_count() - l0
+    if graph is not None:     # launches replayed from the CUDA graph are not seen by the host counter
+        launches += sum(64 * (count // 64) for count in sizes)
     clocks = sampler.stop() if rank == 0 else None
-    ordered = sorted(blocks)
-    ms_max = ordered[len(ordered) // 2]           # the median block (max over ranks inside each block) is the reported one
-    ms = ms_max
-    ms_per_step = ms_max / args.steps
-    value = world * n * args.steps / (ms_max * 1e-3)
-    repeat_info = {"blocks": repeats, "steps_per_block": args.steps, "reported": "median block, max over ranks",
-                   "best_ms_per_step": ordered[0] / args.steps, "median_ms_per_step": ms_per_step,
-                   "worst_ms_per_step": ordered[-1] / args.steps, "loaded_ms": sum(blocks)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)
+    per_step = sorted(ms / count for ms, count in zip(blocks, sizes))
+    ms_per_step = per_step[len(per_step) // 2]    # the median block (max over ranks inside each block) is the reported one
+    value = world * n / (ms_per_step * 1e-3)
+    repeat_info = {"blocks": nblocks, "steps_per_block": sizes, "timed_steps": args.steps,
+                   "reported": "median block, max over ranks", "best_ms_per_step": per_step[0],
+                   "median_ms_per_step": ms_per_step, "worst_ms_per_step": per_step[-1], "loaded_ms": sum(blocks)}
 
     # dominant kernel: the step is exactly one launch of it, so its average launch duration is the CUDA-event
-    # time of the timed region (this rank) divided by the launches in it
-    kernel_avg_ms = ms / max(1, launches)     # ms: the slowest rank's time of the reported block
+    # time per step of the reported block (the slowest rank's) over the launches per step
+    kernel_avg_ms = ms_per_step * args.steps / max(1, launches)
     if args.env_id == "PandaReach-Gazebo-v0":
         kernel_name = "k_task_panda_lanes" if n <= 32768 else "k_task_panda"
     else:
@@ -653,7 +683,8 @@ def run_b200(args):
                            "l2": "inputs larger than L2 (per-step working set %.0f MB vs 126 MB L2)"
                                  % (env.bytes_per_env_step * n / 1e6),
                            "actions": "pre-generated on device, 4 buffers cycled",
-                           "timing": "median of %d blocks of %d steps, each bracketed by barrier + synchronize" % (repeats, args.steps)},
+                           "timing": "%d timed steps after %d warm-up steps, median of %d blocks, each bracketed by "
+                                     "barrier + synchronize" % (args.steps, args.warmup, nblocks)},
                 "clocks": clocks, "e2e": e2e, "gpu_launches": int(launches), "roofline": roofline, "repeats": repeat_info}
         if stats_info is not None:
             line["episode_statistics"] = stats_info
