@@ -446,67 +446,6 @@ __global__ void __launch_bounds__(256) k_task_chain(const TaskArgs<T> a)
     store_row<T, 2 * nq>(a.state, e, st);
 }
 
-// The same step for large batches as a grid-stride loop with the NEXT env's inputs already in flight: a thread of
-// k_task_chain spends most of its life in its fp64 chain (sincos + 2x2 solve) with nothing outstanding, so the bytes
-// in flight per SM follow the SM clock (0.94 of the copy bandwidth at 1.97 GHz, 0.85 under a power cap at 1.73 GHz).
-// Here every thread issues the loads of env e + stride before it computes env e, which keeps HBM requests queued during
-// the arithmetic whatever the clock. Launched with a few blocks per SM; eager launches only (host-side step index).
-template <int TASK, typename T>
-__global__ void __launch_bounds__(256) k_task_chain_stream(const TaskArgs<T> a)
-{
-    constexpr int nq = TaskTraits<TASK>::nq, nobs = TaskTraits<TASK>::nobs;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (e == 0 && a.step_counter && a.advance_counter) *a.step_counter = a.step + 1ull;
-    if (e >= a.n) return;
-    T st[2 * nq], dm[nq + 1], action;
-    unsigned el;
-    load_row<T, 2 * nq>(a.state, e, st);
-    action = __ldcs(a.actions + e);
-    el = a.elapsed[e];
-    if (a.rand) {
-#pragma unroll
-        for (int k = 0; k <= nq; ++k) dm[k] = __ldcs(a.rand + e * (nq + 1) + k);
-    }
-    for (;;) {
-        const int64_t en = e + stride;
-        const bool more = en < a.n;
-        T st_n[2 * nq], dm_n[nq + 1], action_n = T(0);
-        unsigned el_n = 0;
-        if (more) {
-            load_row<T, 2 * nq>(a.state, en, st_n);
-            action_n = __ldcs(a.actions + en);
-            el_n = a.elapsed[en];
-            if (a.rand) {
-#pragma unroll
-                for (int k = 0; k <= nq; ++k) dm_n[k] = __ldcs(a.rand + en * (nq + 1) + k);
-            }
-        }
-        ChainCoef<T> coef = a.coef;
-        if (a.rand) coef = randomized_coef(a.coef, a.basis, nq, dm, dm[nq]);
-        T obs[nobs], reward;
-        const bool done = task_env_advance<TASK, T>(a, coef, st, el, action, obs, reward);
-        store_row<T, nobs>(a.obs, e, obs);
-        __stcs(a.reward + e, reward);
-        a.done[e] = done ? 1 : 0;
-        if (a.ep_return) episode_stats_accumulate(a.ep_return, a.ep_totals, e, reward, done, el);
-        if (done && task_env_reset<TASK, T>(a, st, el, e, a.step, dm)) {
-#pragma unroll
-            for (int k = 0; k <= nq; ++k) a.rand[e * (nq + 1) + k] = dm[k];
-        }
-        a.elapsed[e] = (uint16_t)el;
-        store_row<T, 2 * nq>(a.state, e, st);
-        if (!more) break;
-#pragma unroll
-        for (int k = 0; k < 2 * nq; ++k) st[k] = st_n[k];
-#pragma unroll
-        for (int k = 0; k <= nq; ++k) dm[k] = dm_n[k];
-        action = action_n;
-        el = el_n;
-        e = en;
-    }
-}
-
 // `steps` consecutive env.steps of every env in ONE launch (open-loop action sequences: synthetic rollouts, replayed
 // trajectories). The env's state, episode counter and model parameters stay in registers between steps, so per step
 // only the action is read and the observation / reward / done are written: small batches (BASELINE config 2,
@@ -1554,6 +1493,11 @@ __global__ void __launch_bounds__(64) k_coupled_prepare(const ModelDev<T>* __res
 // model is left in place by k_coupled_dynamics and cleared by k_world_finish. k_coupled_dynamics rewrites q in the state
 // buffer with the value the other two derive on their own, so their concurrent reads see the same number either way.
 // ---------------------------------------------------------------------------------------------------------
+// Shared-memory carve-out (percent) of the three forked kernels and of k_run_tree_lanes<COUPLED>, which replaces
+// k_coupled_dynamics on small batches: they must share SMs, and an SM has one shared-memory / L1 split at a time
+// (b2_sim.cu, launch_coupled).
+constexpr int kCoupledCarveout = 25;
+
 template <typename T>
 struct CoupledDynamics {
     static constexpr bool active = true;
@@ -1791,8 +1735,6 @@ template <typename T> __device__ __forceinline__ T clamp_sel(T x, T lo, T hi) { 
 template <typename T, int NVP>
 __global__ void __launch_bounds__(64, 7) k_pgs_solve(const PgsBuffers<T> g, int iterations)
 {
-    const bool generic_loop = iterations < 0;  // a negative sweep count asks for the generic (not unrolled) sweep loop
-    if (generic_loop) iterations = -iterations;
     constexpr int EPW = 32 / NVP;  // envs per warp
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -1935,8 +1877,7 @@ __global__ void __launch_bounds__(64, 7) k_pgs_solve(const PgsBuffers<T> g, int 
                 }
             }
         };
-        if (generic_loop) sweeps(std::integral_constant<int, 0>{});  // A/B runs (B2_PGS_UNROLL=0)
-        else if (Uw == 13) sweeps(std::integral_constant<int, 13>{});
+        if (Uw == 13) sweeps(std::integral_constant<int, 13>{});
         else if (Uw == 9) sweeps(std::integral_constant<int, 9>{});
         else if (Uw == 8) sweeps(std::integral_constant<int, 8>{});  // two stacked cubes
         else if (Uw == 5) sweeps(std::integral_constant<int, 5>{});

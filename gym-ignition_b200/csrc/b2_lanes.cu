@@ -1,8 +1,6 @@
 // Translation unit of the lane-parallel kernels (sm_100a). See b2_lanes.cuh.
 #include "b2_lanes.hpp"
 
-#include <stdlib.h>
-
 #include "b2_lanes.cuh"
 
 namespace b2 {
@@ -12,11 +10,10 @@ namespace {
 // scheduling and model staging of the next (the kernels wait with griddepcontrol.wait before they touch per-env memory).
 // Measured on the B200 (PandaReach): 39.1 -> 37.5 us per step at 16,384 envs, but 14.8 -> 15.6 us at 4,096 envs (less than one
 // wave of blocks: the early blocks of the next step land on the SMs that free up first and unbalance it), so `allow` is set
-// for batches above 8,192 envs only. B2_LANES_PDL=0 / 1 forces it.
+// for batches above 8,192 envs only.
 template <typename... KArgs, typename... Args>
 cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t stream, bool allow, Args... args)
 {
-    static const char* env = getenv("B2_LANES_PDL");
     cudaLaunchConfig_t lc = {};
     lc.gridDim = dim3((unsigned)grid);
     lc.blockDim = dim3((unsigned)block);
@@ -24,52 +21,41 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t sme
     lc.stream = stream;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = env ? (atoi(env) != 0) : (allow ? 1 : 0);
+    attr[0].val.programmaticStreamSerializationAllowed = allow ? 1 : 0;
     lc.attrs = attr;
     lc.numAttrs = 1;
     return cudaLaunchKernelEx(&lc, kernel, KArgs(args)...);
 }
 
-template <typename T, int G, int MINB, int NQ, unsigned P_LO = 0u, unsigned P_HI = 0u, unsigned REV = 0u>
+template <typename T, int G, int NQ, unsigned P_LO = 0u, unsigned P_HI = 0u, unsigned REV = 0u>
 cudaError_t launch_panda_g(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a, const TreeBits& tb,
-                           cudaStream_t stream, int warps)
+                           cudaStream_t stream)
 {
     using L = LaneLayout<G>;
+    // 64-thread blocks spread small batches over more SMs (4,096 envs: 14.4 us against 16.5 us), 128-thread blocks share
+    // the staged model constants among more envs (16,384 envs: 39.0 us against 39.6 us)
+    const int warps = a.n <= 8192 ? 2 : 4;
     const int64_t envs_per_block = (int64_t)warps * L::envs_per_warp;
     const int grid = (int)((a.n + envs_per_block - 1) / envs_per_block);
     const size_t smem = ((size_t)envs_per_block * L::stride + L::table + 12) * sizeof(T);
-    cudaError_t rc = cudaFuncSetAttribute(k_task_panda_lanes<T, G, MINB, NQ, P_LO, P_HI, REV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t rc = cudaFuncSetAttribute(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (rc != cudaSuccess) return rc;
-    return launch_pdl(k_task_panda_lanes<T, G, MINB, NQ, P_LO, P_HI, REV>, grid, 32 * warps, smem, stream, a.n > 8192, tables, lane_table, a, tb);
+    return launch_pdl(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV>, grid, 32 * warps, smem, stream, a.n > 8192, tables, lane_table, a, tb);
 }
 }  // namespace
 
 template <typename T>
 cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a,
-                                    const int* parent, const int* jtype, cudaStream_t stream, int warps_per_block)
+                                    const int* parent, const int* jtype, cudaStream_t stream)
 {
     const TreeBits tb = make_tree_bits(a.nq, parent, jtype);
-    static const char* env_warps = getenv("B2_LANES_WARPS");
-    // 64-thread blocks spread small batches over more SMs (4,096 envs: 14.4 us against 16.5 us), 128-thread blocks share
-    // the staged model constants among more envs (16,384 envs: 39.0 us against 39.6 us)
-    int warps = warps_per_block > 0 ? warps_per_block : (env_warps ? atoi(env_warps) : (a.n <= 8192 ? 2 : 4));
-    if (warps < 1 || warps > 4) warps = 4;
-    static const char* env_minb = getenv("B2_LANES_MINB");
-    const int minb = env_minb ? atoi(env_minb) : 4;  // 127 registers, no spills: measured best at 4,096 and 16,384 envs
-    if (a.nq <= 8) return launch_panda_g<T, 8, 4, 0>(tables, lane_table, a, tb, stream, warps);
+    if (a.nq <= 8) return launch_panda_g<T, 8, 0>(tables, lane_table, a, tb, stream);
     // the Panda (a chain of 7 revolute joints, two prismatic fingers on the last arm body): tree known at compile time
     constexpr unsigned kPandaLo = 0x76543210u, kPandaHi = 0x7u, kPandaRev = 0x7fu;
-    static const char* env_static = getenv("B2_LANES_STATIC_TREE");
-    const bool is_panda = a.nq == 9 && tb.p_lo == kPandaLo && tb.p_hi == kPandaHi && tb.rev_mask == kPandaRev &&
-                          !(env_static && atoi(env_static) == 0);
-    if (is_panda) {
-        if (minb == 3) return launch_panda_g<T, 10, 3, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream, warps);
-        if (minb == 5) return launch_panda_g<T, 10, 5, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream, warps);
-        if (minb == 6) return launch_panda_g<T, 10, 6, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream, warps);
-        return launch_panda_g<T, 10, 4, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream, warps);
-    }
-    if (a.nq <= 10) return launch_panda_g<T, 10, 4, 0>(tables, lane_table, a, tb, stream, warps);
-    return launch_panda_g<T, 16, 4, 0>(tables, lane_table, a, tb, stream, warps);
+    if (a.nq == 9 && tb.p_lo == kPandaLo && tb.p_hi == kPandaHi && tb.rev_mask == kPandaRev)
+        return launch_panda_g<T, 10, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream);
+    if (a.nq <= 10) return launch_panda_g<T, 10, 0>(tables, lane_table, a, tb, stream);
+    return launch_panda_g<T, 16, 0>(tables, lane_table, a, tb, stream);
 }
 
 namespace {
@@ -84,13 +70,9 @@ cudaError_t launch_run_g(const ModelDev<T>* tables, const LaneTable<T>* lane_tab
     const size_t smem = ((size_t)envs_per_block * L::stride + L::table + 12) * sizeof(T);
     cudaError_t rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (rc != cudaSuccess) return rc;
-    if (COUPLED) {  // must share SMs with k_coupled_rows / k_coupled_minv: the same shared-memory carve-out (b2_sim.cu launch_coupled)
-        static const char* carve_env = getenv("B2_COUPLED_CARVEOUT");
-        const int carve = carve_env ? atoi(carve_env) : 25;
-        if (carve >= 0) {
-            rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
-            if (rc != cudaSuccess) return rc;
-        }
+    if (COUPLED) {  // must share SMs with k_coupled_rows / k_coupled_minv: the same shared-memory carve-out
+        rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED>, cudaFuncAttributePreferredSharedMemoryCarveout, kCoupledCarveout);
+        if (rc != cudaSuccess) return rc;
     }
     // a coupled step forks three kernels from one event: no programmatic overlap with the previous step's finish
     return launch_pdl(k_run_tree_lanes<T, G, CT, COUPLED>, grid, 32 * warps, smem, stream, !COUPLED && b.n > 8192, tables, lane_table,
@@ -124,8 +106,8 @@ template cudaError_t launch_run_tree_lanes<float>(const ModelDev<float>*, const 
                                                   const RunBuffers<float>&, const int*, const int*, cudaStream_t, float*, int);
 
 template cudaError_t launch_task_panda_lanes<double>(const ModelDev<double>*, const LaneTable<double>*, const PandaArgs<double>&,
-                                                     const int*, const int*, cudaStream_t, int);
+                                                     const int*, const int*, cudaStream_t);
 template cudaError_t launch_task_panda_lanes<float>(const ModelDev<float>*, const LaneTable<float>*, const PandaArgs<float>&,
-                                                    const int*, const int*, cudaStream_t, int);
+                                                    const int*, const int*, cudaStream_t);
 
 }  // namespace b2

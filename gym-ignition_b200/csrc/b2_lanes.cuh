@@ -736,15 +736,16 @@ __device__ __noinline__ void lanes_joint_constraints(T* x /* [4][G] exchange str
 // reward, TimeLimit, reset. blockDim.x = 32 * warps, each warp steps 32 / G envs; dynamic shared memory =
 // LaneLayout<G>::table + warps * (32 / G) * LaneLayout<G>::stride scalars.
 // ---------------------------------------------------------------------------------------------------------------------
-// MINB: 128-thread blocks per SM the register allocation is sized for (4: 127 registers, 5: 96, 6: 80 with ~200 bytes of spills).
+// The register allocation is sized for 4 blocks of 128 threads per SM (127 registers, no spills): measured best at 4,096
+// and 16,384 envs among budgets of 3 - 6 blocks (5: 96 registers, 6: 80 with ~200 bytes of spills).
 // NQ > 0: the tree (joint count NQ, parents P_LO / P_HI, joint types REV, encoded like TreeBits) is a compile-time
 // constant: the launcher instantiates the Panda's and dispatches on a match with the loaded model. Every `i < nq` guard,
 // parent lookup and chain / branch decision of the unrolled body loops then folds away (about a third of the kernel's
 // instructions). NQ = 0 reads the tree from the arguments.
-template <typename T, int G, int MINB, int NQ, unsigned P_LO, unsigned P_HI, unsigned REV>
-__global__ void __launch_bounds__(128, MINB) k_task_panda_lanes(const ModelDev<T>* __restrict__ tables,
-                                                          const LaneTable<T>* __restrict__ lane_table, const PandaArgs<T> a,
-                                                          const TreeBits tb_arg)
+template <typename T, int G, int NQ, unsigned P_LO, unsigned P_HI, unsigned REV>
+__global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* __restrict__ tables,
+                                                       const LaneTable<T>* __restrict__ lane_table, const PandaArgs<T> a,
+                                                       const TreeBits tb_arg)
 {
     const TreeBits tb = NQ > 0 ? TreeBits{P_LO, P_HI, REV, NQ, {0}} : tb_arg;  // the ancestor masks are read from tb_arg
     using L = LaneLayout<G>;
@@ -807,7 +808,6 @@ __global__ void __launch_bounds__(128, MINB) k_task_panda_lanes(const ModelDev<T
         dq += ddq * a.dt;
         const bool f0 = c.body && c.tab[LT_FRICTION] != T(0), f1 = c.body && q <= c.tab[LT_LOWER], f2 = c.body && q >= c.tab[LT_UPPER];
         const unsigned rows = __ballot_sync(0xffffffffu, f0 || f1 || f2);
-#ifndef B2_LANES_NO_RARE
         if (rows) {
             T dq_io = dq, ddq_io = ddq;  // copies: the out-of-line calls must not pin the kernel's registers to memory
             const bool dk = c.body && (c.tab[LT_DAMPING] != T(0) || c.tab[LT_STIFFNESS] != T(0));
@@ -819,7 +819,6 @@ __global__ void __launch_bounds__(128, MINB) k_task_panda_lanes(const ModelDev<T
             dq = dq_io;
             ddq = ddq_io;
         }
-#endif
         q += dq * a.dt;
     }
     // ---- observation: kinematics at the new positions ----

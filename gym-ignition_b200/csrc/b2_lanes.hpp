@@ -8,10 +8,10 @@
 
 namespace b2 {
 
-// Fused Panda task, G lanes per env (G chosen from the number of joints). `warps_per_block` = 0 picks the default.
+// Fused Panda task, G lanes per env (G chosen from the number of joints).
 template <typename T>
 cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a,
-                                    const int* parent, const int* jtype, cudaStream_t stream, int warps_per_block = 0);
+                                    const int* parent, const int* jtype, cudaStream_t stream);
 
 // GazeboSimulator::run of a fixed-base tree on lanes (k_run_tree_lanes): PID / force / velocity-follower joints, the
 // computed-torque controller, resets, external link wrenches. v0 != nullptr: the model belongs to a coupled world; the

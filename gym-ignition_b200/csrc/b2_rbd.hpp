@@ -143,7 +143,7 @@ B2_HD void sincos_t(double x, double* s, double* c)
 // move), so only that kernel uses it.
 B2_HD void sincos_tp(double x, double* s, double* c)
 {
-#if defined(__CUDA_ARCH__) && !defined(B2_LIB_SINCOS)
+#if defined(__CUDA_ARCH__)
     sincos_reduced(x, s, c);
 #else
     sincos_t(x, s, c);
@@ -161,7 +161,7 @@ B2_HD void sincos_t(float x, float* s, float* c)
 
 B2_HD double cos_t(double x)
 {
-#if defined(__CUDA_ARCH__) && !defined(B2_LIB_SINCOS)
+#if defined(__CUDA_ARCH__)
     double s, c;
     sincos_reduced(x, &s, &c);  // the sine polynomial is dead code here
     return c;

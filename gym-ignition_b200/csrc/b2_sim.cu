@@ -142,7 +142,6 @@ struct b2sim {
     double contact_erp = 0.01, contact_max_erv = 1e-3;
     int contact_iterations = 50;
     uint64_t launches = 0;
-    int sm_count = 0;
     bool free_wrench_dirty = false;  // the ext / ext_env block of the device world is stale
     std::vector<std::unique_ptr<ModelState>> models;
 
@@ -262,6 +261,20 @@ int tree_topology(const ModelState* ms, b2::TreeTopo* topo)
     return B2_OK;
 }
 
+// Whether a tree's dynamics run on lanes (k_run_tree_lanes, an env on G lanes of a warp) rather than one thread per env.
+// Small batches of trees with several joints (BASELINE configs 4 / 5: 16,384 / 4,096 Pandas) leave one thread per env
+// with less than a warp per scheduler and the run lasts as long as ONE env's dependent chain, so up to 16,384 envs the
+// step is spread over lanes (Pandas under position PIDs, measured on the B200: 15 us against 38 us per run at 4,096 envs,
+// 42 against 43 us at 16,384; 21 against 60 us at 4,096 envs with both fingers on their limits). By default lanes are
+// used for trees of at least `min_nq` joints. B2_RUN_KERNEL=thread / lanes forces one side (tests run both).
+bool run_on_lanes(const b2sim* s, const ModelState* ms, int min_nq)
+{
+    static const char* forced = getenv("B2_RUN_KERNEL");
+    if (!ms->d_lane_table) return false;
+    if (forced) return !strcmp(forced, "lanes");
+    return s->n <= 16384 && ms->model->t.nq >= min_nq;
+}
+
 template <typename T>
 b2::RunCfg<T> build_run_cfg(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t compute_bits, uint32_t ct_bits,
                             const int* wrench_iters)
@@ -314,16 +327,7 @@ int launch_run(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t co
     int rc = tree_topology(ms, &topo);
     if (rc != B2_OK) return rc;
     const b2::ModelDev<T>* tb = (const b2::ModelDev<T>*)ms->d_tables;
-    // Small batches of trees with several joints (BASELINE configs 4 / 5: 16,384 / 4,096 Pandas) leave one thread per env
-    // with less than a warp per scheduler and the run lasts as long as ONE env's dependent chain; up to 16,384 envs the
-    // step is spread over G lanes of a warp instead (k_run_tree_lanes, b2_lanes.cuh; Pandas under position PIDs, measured
-    // on the B200: 15 us against 38 us per run at 4,096 envs, 42 against 43 us at 16,384; 21 against 60 us at 4,096 envs
-    // with both fingers on their limits).
-    // B2_RUN_KERNEL=thread / lanes forces one of them (A/B runs, tests).
-    static const char* run_variant = getenv("B2_RUN_KERNEL");
-    const bool lanes_ok = nq >= 1 && nq <= b2::kMaxDofs && ms->d_lane_table;
-    const bool lanes = lanes_ok && (run_variant ? !strcmp(run_variant, "lanes") : (nq >= 4 && s->n <= 16384));
-    if (lanes) {
+    if (nq >= 1 && nq <= b2::kMaxDofs && run_on_lanes(s, ms, 4)) {
         B2_CUDA(b2::launch_run_tree_lanes<T>(tb, (const b2::LaneTable<T>*)ms->d_lane_table, cfg, b, ms->model->t.parent,
                                              ms->model->t.jtype, s->stream));
         ++s->launches;
@@ -409,32 +413,18 @@ int launch_task(b2sim* s, ModelState* ms, const void* actions, int traj_steps = 
         return B2_OK;
     }
     // 128-thread blocks (measured on the B200 with eager launches, 64 / 128 / 256 threads: 131,072 envs 4.9 / 4.9 / 5.1 us,
-    // 1,048,576 envs 18.9 / 18.9 / 20.0 us, 4,194,304 envs - / 74.1 / 74.7 us per step). B2_CHAIN_BLOCK overrides.
-    static const char* chain_block = getenv("B2_CHAIN_BLOCK");
-    int block = chain_block ? atoi(chain_block) : 128;
-    if (block != 64 && block != 128 && block != 256) block = 128;
-    const int grid = grid_for(wn, block);
-    // B2_CHAIN_KERNEL=stream runs an eager step as a grid-stride loop that keeps the next env's loads in flight during
-    // the arithmetic (k_task_chain_stream, B2_CHAIN_BLOCKS_PER_SM blocks per SM). Measured on the B200 at 4,194,304
-    // envs: 82 - 103 us for 2 - 8 blocks per SM against 78 us for the plain kernel (identical results), so it is not
-    // the default: one pass with 131 k warps queued already keeps HBM busier than 1,184 resident warps that prefetch.
-    static const char* chain_variant = getenv("B2_CHAIN_KERNEL");
-    static const char* chain_blocks = getenv("B2_CHAIN_BLOCKS_PER_SM");
-    const bool stream_kernel = !capturing && chain_variant && !strcmp(chain_variant, "stream");
-    if (stream_kernel) {
-        if (s->sm_count == 0) B2_CUDA(cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, s->device));
-        const int per_sm = chain_blocks ? std::max(1, atoi(chain_blocks)) : 4;
-        const int sgrid = std::min(grid, s->sm_count * per_sm);
-        b2::k_task_chain_stream<TASK, T><<<sgrid, block, 0, s->stream>>>(a);
-    } else if (capturing) {
+    // 1,048,576 envs 18.9 / 18.9 / 20.0 us, 4,194,304 envs - / 74.1 / 74.7 us per step).
+    // One pass over all envs: a grid-stride variant that keeps the next env's loads in flight during the arithmetic was
+    // measured on the B200 at 4,194,304 envs at 82 - 103 us for 2 - 8 blocks per SM against 78 us for this launch (131 k
+    // warps queued keep HBM busier than 1,184 resident warps that prefetch).
+    const int block = 128, grid = grid_for(wn, block);
+    if (capturing) {
         if ((grid + b2::kTicketGroup - 1) / b2::kTicketGroup > b2::kTicketWords - 1)
             return fail(B2_ERR_UNSUPPORTED, "too many envs for a graph-captured step (%lld)", (long long)wn);
         b2::k_task_chain<TASK, T, true><<<grid, block, 0, s->stream>>>(a);
     } else {
         // eager steps follow each other on the stream: programmatic dependent launch hides the launch-to-launch gap
-        // (k_task_chain waits with griddepcontrol.wait before it touches memory). B2_CHAIN_PDL=0 disables it.
-        static const char* pdl_env = getenv("B2_CHAIN_PDL");
-        const bool pdl = !(pdl_env && atoi(pdl_env) == 0);
+        // (k_task_chain waits with griddepcontrol.wait before it touches memory)
         cudaLaunchConfig_t lc = {};
         lc.gridDim = dim3((unsigned)grid);
         lc.blockDim = dim3((unsigned)block);
@@ -442,7 +432,7 @@ int launch_task(b2sim* s, ModelState* ms, const void* actions, int traj_steps = 
         lc.stream = s->stream;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
         lc.attrs = attr;
         lc.numAttrs = 1;
         B2_CUDA(cudaLaunchKernelEx(&lc, b2::k_task_chain<TASK, T, false>, a));
@@ -490,7 +480,7 @@ int launch_panda(b2sim* s, ModelState* ms, const void* actions, int observe_only
     // Up to 32,768 envs an env's step is spread over G lanes of a warp (b2_lanes.cuh): measured on the B200 at 4,096 /
     // 16,384 / 65,536 / 262,144 envs, lanes 18 / 46 / 149 / 550 us against 46 / 51 / 137 / 480 us for one thread per env
     // (the lane kernel executes ~1.4x the thread-instruction slots per env, so it loses once the batch fills the
-    // schedulers). B2_PANDA_KERNEL=thread / lanes forces one of them (A/B runs).
+    // schedulers). B2_PANDA_KERNEL=thread / lanes forces one of them (tests run both).
     static const char* variant = getenv("B2_PANDA_KERNEL");
     const bool lanes = variant ? strcmp(variant, "thread") != 0 : wn <= 32768;
     if (lanes) {
@@ -870,10 +860,7 @@ int launch_solve_finish(b2sim* s, ModelState* robot, bool clear_robot_mask = fal
     if (g.nvp == 16) {
         constexpr int smem = 4 * b2::pgs_smem_per_env<T, 16>() * (int)sizeof(T);
         B2_CUDA(cudaFuncSetAttribute(b2::k_pgs_solve<T, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        // B2_PGS_UNROLL=0: the generic sweep loop instead of the unrolled ones (A/B; a negative count tells the kernel)
-        static const char* unroll_env = getenv("B2_PGS_UNROLL");
-        const int iters = (unroll_env && atoi(unroll_env) == 0) ? -s->contact_iterations : s->contact_iterations;
-        b2::k_pgs_solve<T, 16><<<grid_for(s->n, 4), 64, smem, s->stream>>>(g, iters);
+        b2::k_pgs_solve<T, 16><<<grid_for(s->n, 4), 64, smem, s->stream>>>(g, s->contact_iterations);
     } else {
         constexpr int smem = 2 * b2::pgs_smem_per_env<T, 32>() * (int)sizeof(T);
         B2_CUDA(cudaFuncSetAttribute(b2::k_pgs_solve<T, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -935,13 +922,10 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
             // different split for each of them (from the blocks per SM their registers would allow), so a kernel could only
             // start on SMs the others had left (measured: rows ended 360 us and M^-1 290 us after the fork instead of 94
             // and 65 us). The same explicit split for all three (64 KB shared, the rest L1 for their per-thread scratch).
-            static const char* carve_env = getenv("B2_COUPLED_CARVEOUT");
-            const int carve = carve_env ? atoi(carve_env) : 25;
-            if (carve >= 0) {
-                B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_dynamics<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-                B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_rows<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-                B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_minv<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-            }
+            const int carve = b2::kCoupledCarveout;
+            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_dynamics<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_rows<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_minv<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
         }
         const b2::RunBuffers<T> rb = run_buffers<T>(s, ms);
         const b2::PgsBuffers<T> g = pgs_buffers<T>(s);
@@ -964,10 +948,8 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
         b2::k_coupled_minv<T><<<grid_for(s->n, 32), 32, 0, s->fork[1]>>>(tb, rb, g);
         if (tr) cudaEventRecord(tev[3], s->fork[1]);
         // the articulated model's controllers + forward dynamics: on lanes for the small batches of this configuration
-        // (k_run_tree_lanes<COUPLED>), one thread per env otherwise (B2_RUN_KERNEL forces one of them)
-        static const char* dyn_variant = getenv("B2_RUN_KERNEL");
-        const bool dyn_lanes = ms->d_lane_table && (dyn_variant ? !strcmp(dyn_variant, "lanes") : s->n <= 16384);
-        if (dyn_lanes) {
+        // (k_run_tree_lanes<COUPLED>), one thread per env otherwise; unlike launch_run, whatever the joint count
+        if (run_on_lanes(s, ms, 0)) {
             B2_CUDA(b2::launch_run_tree_lanes<T>(tb, (const b2::LaneTable<T>*)ms->d_lane_table, cfg, rb, ms->model->t.parent,
                                                  ms->model->t.jtype, s->stream, g.v, g.nvp));
         } else {
@@ -2118,12 +2100,10 @@ int b2sim_task_step_host(b2sim* s, int model, const void* actions_host, void* ob
     const size_t nact = panda ? (size_t)ms->model->t.nq : 1;
     // The env range is cut into chunks; chunk c's actions go host->device on one stream while chunk c-1 is stepped
     // and chunk c-2's outputs go device->host on another, so the two PCIe directions and the kernels overlap.
-    // Measured at 4,194,304 envs (B2_HOST_CHUNKS): 2 / 4 / 8 / 16 / 32 chunks -> 1.18 / 1.24 / 1.23 / 1.19 / 1.11e9 env-steps/s.
+    // Measured at 4,194,304 envs: 2 / 4 / 8 / 16 / 32 chunks -> 1.18 / 1.24 / 1.23 / 1.19 / 1.11e9 env-steps/s.
     // Letting the kernel read the actions and write the outputs straight through mapped pinned memory instead of the copy
     // engines was measured too: 4.5e8 env-steps/s (22 GB/s on the link), so the copies stay.
-    const int64_t min_chunk = 65536;
-    static const char* chunks_env = getenv("B2_HOST_CHUNKS");
-    const int max_chunks = chunks_env ? std::max(1, std::min(64, atoi(chunks_env))) : 8;
+    const int64_t min_chunk = 65536, max_chunks = 8;
     const int chunks = (int)std::max<int64_t>(1, std::min<int64_t>(max_chunks, s->n / min_chunk));
     if (!s->copy_in) {
         B2_CUDA(cudaStreamCreateWithFlags(&s->copy_in, cudaStreamNonBlocking));

@@ -42,7 +42,7 @@ def child(n, dtype, out):
         b.record()
         torch.cuda.synchronize()
         best = min(best, a.elapsed_time(b) / 100)
-    print(f"{os.environ.get('B2_PANDA_KERNEL', 'lanes'):7s} fingers={os.environ.get('PROBE_FINGERS', 'free')} warps/block={os.environ.get('B2_LANES_WARPS', '-')} minb={os.environ.get('B2_LANES_MINB', '-')} n={n} {dtype}: "
+    print(f"{os.environ.get('B2_PANDA_KERNEL', 'lanes'):7s} fingers={os.environ.get('PROBE_FINGERS', 'free')} n={n} {dtype}: "
           f"{best * 1e3:8.1f} us/launch  {n / best * 1e3:.3e} env-steps/s", flush=True)
 
 
@@ -55,14 +55,10 @@ if __name__ == "__main__":
     dtype = sys.argv[2] if len(sys.argv) > 2 else "float64"
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     outs = {}
-    for variant, warps, minb in (("thread", None, None), ("lanes", "2", "3"), ("lanes", "4", "3"), ("lanes", "2", "4"), ("lanes", "3", "4"),
-                                 ("lanes", "4", "4")):
-        envv = dict(os.environ, B2_PANDA_KERNEL=variant)
-        if warps:
-            envv["B2_LANES_WARPS"] = warps
-            envv["B2_LANES_MINB"] = minb
+    for variant in ("thread", "lanes"):
         out = os.path.join(ROOT, "gpurun_out", f"panda_{variant}.npz")
-        subprocess.check_call([sys.executable, os.path.abspath(__file__), "--child", str(n), dtype, out], env=envv)
+        subprocess.check_call([sys.executable, os.path.abspath(__file__), "--child", str(n), dtype, out],
+                              env=dict(os.environ, B2_PANDA_KERNEL=variant))
         outs[variant] = np.load(out)
     a, b = outs["thread"], outs["lanes"]
     for k in ("obs", "rew", "state"):

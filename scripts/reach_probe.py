@@ -1,4 +1,4 @@
-"""PandaReach (BASELINE config 4) fused step time at several env counts; B2_PANDA_STORES=direct|tiled selects the store path."""
+"""PandaReach (BASELINE config 4) fused step time at several env counts."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import __graft_entry__; __graft_entry__.load_package()
@@ -19,5 +19,5 @@ for n in [int(a) for a in sys.argv[1:]] or (4096, 16384, 65536, 262144):
         env.step(tg)
     b.record(); torch.cuda.synchronize()
     ms = a.elapsed_time(b) / 100
-    print(f"n={n}: {ms * 1e3:.1f} us/step -> {n / ms * 1e3:.3e} env-steps/s  (stores: {os.environ.get('B2_PANDA_STORES', 'auto')})", flush=True)
+    print(f"n={n}: {ms * 1e3:.1f} us/step -> {n / ms * 1e3:.3e} env-steps/s", flush=True)
     env.close()

@@ -1,20 +1,15 @@
 """One GPU's share of BASELINE config 3 as written (1,048,576 cart-pole envs split over 8 / 4 / 2 GPUs = 131,072 / 262,144 /
-524,288 envs per GPU), timed on ONE B200: eager launches and a CUDA graph of 64 launches, for each thread-block size of
-k_task_chain (B2_CHAIN_BLOCK, read once per process).
+524,288 envs per GPU), timed on ONE B200: eager launches and a CUDA graph of 64 launches.
 
     python scripts/strong_probe.py
 """
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
-def child(n):
-    sys.path.insert(0, ROOT)
-    import __graft_entry__
-    __graft_entry__.load_package()
+def probe(n):
     import torch
     import b2sim
     env = b2sim.BatchedTaskEnv("CartPoleContinuousSwingup-Gazebo-v0", n, seed=0, env_offset=n)
@@ -51,15 +46,13 @@ def child(n):
         graph.replay()
     gr = timed(graph.replay, 8, 64)
     hbm = n * env.bytes_per_env_step / 6547.2e9 * 1e6
-    print(f"block={os.environ.get('B2_CHAIN_BLOCK', 'default'):7s} n={n}: eager {eager * 1e3:6.2f} us/step ({hbm / (eager * 1e3):.2f} of the HBM "
+    print(f"n={n}: eager {eager * 1e3:6.2f} us/step ({hbm / (eager * 1e3):.2f} of the HBM "
           f"roofline), graph {gr * 1e3:6.2f} us/step ({hbm / (gr * 1e3):.2f}); HBM time {hbm:.2f} us", flush=True)
 
 
 if __name__ == "__main__":
-    if len(sys.argv) > 1 and sys.argv[1] == "--child":
-        child(int(sys.argv[2]))
-        sys.exit(0)
+    sys.path.insert(0, ROOT)
+    import __graft_entry__
+    __graft_entry__.load_package()
     for n in (131072, 262144, 524288, 1048576):
-        for block in ("64", "128", "256"):
-            subprocess.check_call([sys.executable, os.path.abspath(__file__), "--child", str(n)],
-                                  env=dict(os.environ, B2_CHAIN_BLOCK=block))
+        probe(n)

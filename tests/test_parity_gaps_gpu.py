@@ -230,25 +230,45 @@ def test_batched_runtime_reset_returns_the_observation(torch):
     rp.close()
 
 
-@pytest.mark.parametrize("variant", ["lanes", "thread"])
-def test_run_path_on_lanes_and_on_threads(variant):
-    """GazeboSimulator::run of a fixed-base tree has two kernels: k_run_tree (one thread per env) and k_run_tree_lanes (an
-    env on G lanes of a warp, the default for trees of >= 4 joints up to 32,768 envs). The tests of the run path use small
-    env counts and models of 1, 2 and 9 joints, so each kernel is forced here (B2_RUN_KERNEL is read once per process) for
-    the same oracle comparisons: force / PID / velocity-follower joints, the computed-torque controller, deferred resets,
-    the PID rate gate, limits and Coulomb friction rows, external link wrenches, link kinematics after a run."""
+def _run_gpu_tests_with(switches, files, sel):
+    """Runs the GPU tests of `files` selected by `sel` in a fresh process with the environment variables `switches` set
+    (the engine reads its kernel switches once per process)."""
     import os
     import subprocess
     import sys
-    env = dict(os.environ, B2_RUN_KERNEL=variant)
     here = os.path.dirname(os.path.abspath(__file__))
-    files = [os.path.join(here, f) for f in ("test_parity_gpu.py", "test_parity_gaps_gpu.py", "test_scenario_gpu.py")]
+    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu"] + [os.path.join(here, f) for f in files] +
+                       ["-k", sel], env=dict(os.environ, **switches), capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
+
+
+@pytest.mark.parametrize("variant", ["lanes", "thread", "local"])
+def test_run_path_on_lanes_and_on_threads(variant):
+    """GazeboSimulator::run of a fixed-base tree has three kernels: k_run_tree_lanes (an env on G lanes of a warp, the
+    default for trees of >= 4 joints up to 16,384 envs), and one thread per env with its scratch in shared memory
+    (k_run_tree) or, from 65,536 envs, in local memory (k_run_tree_local). The tests of the run path use small env counts
+    and models of 1, 2 and 9 joints, so each kernel is forced here ("local": B2_RUN_KERNEL=thread and
+    B2_TREE_SCRATCH=local) for the same oracle comparisons: force / PID / velocity-follower joints, the computed-torque
+    controller, deferred resets, the PID rate gate, limits and Coulomb friction rows, external link wrenches, link
+    kinematics after a run."""
+    switches = {"lanes": {"B2_RUN_KERNEL": "lanes"}, "thread": {"B2_RUN_KERNEL": "thread"},
+                "local": {"B2_RUN_KERNEL": "thread", "B2_TREE_SCRATCH": "local"}}[variant]
     sel = ("test_run_force_mode_matches_oracle or test_panda_position_pid or test_tree_kernel_constraint_paths or "
            "test_pid_rate_gate or test_chain_closed_form_equals_tree_kernel or test_fp32_fast_mode_tree or wrench or "
            "test_model_joint_api or test_velocity or test_link or friction or pid or computed_torque")
-    r = subprocess.run([sys.executable, "-m", "pytest", "-q", "-x", "-m", "gpu"] + files + ["-k", sel], env=env,
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
+    _run_gpu_tests_with(switches, ("test_parity_gpu.py", "test_parity_gaps_gpu.py", "test_scenario_gpu.py"), sel)
+
+
+@pytest.mark.parametrize("variant", ["lanes", "thread"])
+def test_panda_task_on_lanes_and_on_threads(variant):
+    """The fused PandaReach step has two kernels: k_task_panda_lanes (an env on G lanes of a warp, the default up to
+    32,768 envs) and k_task_panda (one thread per env, above that). The PandaReach task tests run at <= 16,384 envs, so
+    each kernel is forced here (B2_PANDA_KERNEL) for the same comparisons: the oracle trajectory with resets, limit rows
+    against the oracle's dense LCP, CUDA-graph replay against eager steps, and the kernel-side episode statistics."""
+    sel = ("test_panda_fused_task_matches_oracle or test_panda_task_limit_rows_one_step_matches_oracle or "
+           "test_panda_task_steps_replayed_from_a_cuda_graph or test_panda_task_statistics")
+    _run_gpu_tests_with({"B2_PANDA_KERNEL": variant},
+                        ("test_parity_gpu.py", "test_parity_gaps_gpu.py", "test_episode_stats_gpu.py"), sel)
 
 
 def test_panda_task_limit_rows_one_step_matches_oracle(torch, oracle, model_files):
