@@ -831,19 +831,26 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
     B2_MARK(12);
     lanes_forward_kinematics(c, m, warp_strips, live_envs, ee_body + 1);
     B2_MARK(13);
-    const unsigned on_chain = tb_arg.anc[ee_body];
+    // an end effector welded to the base (ee_body = -1) has an empty chain: lane 0 places it from the base pose
+    const int ee_lane = max(ee_body, 0);
+    const unsigned on_chain = ee_body >= 0 ? tb_arg.anc[ee_body] : 0u;
     T* out = c.sm + L::oP1;  // the joint placements are dead once the forward kinematics has run
     V3<T> aw = v3(T(0), T(0), T(0)), po = aw, pe = aw;
     const T bx = m.basep[0], by = m.basep[1], bz = m.basep[2];
     const bool chain_lane = c.body && ((on_chain >> c.l) & 1u);
-    if (chain_lane) {
+    if (chain_lane || (c.body && c.l == ee_lane)) {
         T R[9];
-        lanes_load_placement(c, R, po);
-        const T* t = c.tab;
-        aw = v3(R[0] * t[LT_AXIS] + R[1] * t[LT_AXIS + 1] + R[2] * t[LT_AXIS + 2],
-                R[3] * t[LT_AXIS] + R[4] * t[LT_AXIS + 1] + R[5] * t[LT_AXIS + 2],
-                R[6] * t[LT_AXIS] + R[7] * t[LT_AXIS + 1] + R[8] * t[LT_AXIS + 2]);
-        if (c.l == ee_body) {
+        if (chain_lane) {
+            lanes_load_placement(c, R, po);
+            const T* t = c.tab;
+            aw = v3(R[0] * t[LT_AXIS] + R[1] * t[LT_AXIS + 1] + R[2] * t[LT_AXIS + 2],
+                    R[3] * t[LT_AXIS] + R[4] * t[LT_AXIS + 1] + R[5] * t[LT_AXIS + 2],
+                    R[6] * t[LT_AXIS] + R[7] * t[LT_AXIS + 1] + R[8] * t[LT_AXIS + 2]);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 9; ++k) R[k] = m.baseR[k];
+        }
+        if (c.l == ee_lane) {
             const T* ee = table + L::table;  // link_R (9), link_p (3)
             pe = v3(po.x + R[0] * ee[9] + R[1] * ee[10] + R[2] * ee[11], po.y + R[3] * ee[9] + R[4] * ee[10] + R[5] * ee[11],
                     po.z + R[6] * ee[9] + R[7] * ee[10] + R[8] * ee[11]);
@@ -870,7 +877,7 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
             out[k + 3] = qw; out[k + 4] = qx; out[k + 5] = qy; out[k + 6] = qz;
         }
     }
-    const int src = c.slot * G + ee_body;
+    const int src = c.slot * G + ee_lane;
     pe.x = __shfl_sync(0xffffffffu, pe.x, src);
     pe.y = __shfl_sync(0xffffffffu, pe.y, src);
     pe.z = __shfl_sync(0xffffffffu, pe.z, src);
