@@ -21,7 +21,7 @@ SHAPE_BOX, SHAPE_SPHERE, SHAPE_CYLINDER, SHAPE_PLANE = 0, 1, 2, 3
 (BUF_STATE, BUF_ACCELERATION, BUF_FORCE_CMD, BUF_POS_TARGET, BUF_VEL_TARGET, BUF_PID_STATE,
  BUF_RESET_STATE, BUF_RESET_MASK, BUF_OBS, BUF_REWARD, BUF_DONE, BUF_ELAPSED, BUF_ACTION,
  BUF_LINK_POSE, BUF_BASE_STATE, BUF_BASE_RESET, BUF_ACC_TARGET, BUF_RAND_PARAMS, BUF_EP_RETURN,
- BUF_BASE_ACCEL) = range(20)
+ BUF_BASE_ACCEL, BUF_BODY_INERTIA, BUF_JOINT_DYNAMICS, BUF_GRAVITY) = range(23)
 STAT_STRIPES = 32  # B2_STAT_STRIPES
 
 (FIELD_POSITION, FIELD_VELOCITY, FIELD_ACCELERATION, FIELD_FORCE, FIELD_FORCE_TARGET,
@@ -116,6 +116,7 @@ SYMBOLS = {
     "b2sim_controller_period": (_d, [_vp, _i]),
     "b2sim_set_max_generalized_force": (_i, [_vp, _i, _i, _d]),
     "b2sim_set_joint_friction": (_i, [_vp, _i, _i, _d, _d]),
+    "b2sim_enable_env_params": (_i, [_vp, _i, _i]),
     "b2sim_set_computed_torque": (_i, [_vp, _i, _dp, _dp, _dp]),
     "b2sim_apply_link_wrench": (_i, [_vp, _i, _i64, _i, _dp, _d]),
     "b2sim_get_joint": (_i, [_vp, _i, _i, _i64, _i, _dp]),

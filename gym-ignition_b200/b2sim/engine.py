@@ -244,6 +244,24 @@ class Simulator:
     def tensor(self, model, which):
         return self.buffer(model, which).torch(self.device)
 
+    # ---- per-env physical parameters ----
+    def enable_env_params(self, model, enable: bool = True):
+        """Gives every env of `model` its own body inertias, joint damping / Coulomb friction and gravity, starting from
+        the model's current values. Returns zero-copy views (body_inertia [N, nq, 10]: mass, centre of mass xyz, inertia
+        about it xx xy xz yy yz zz in the body frame; joint_dynamics [N, nq, 2]: damping, friction; gravity [N, 3]) that
+        the caller writes between runs, e.g. at its resets; every unpaused run reads them. enable=False returns the model
+        to its shared tables and returns None. The views do not own their memory: disabling, removing the model or
+        closing the simulator frees it, and a view kept from before must not be used afterwards (enable again for new
+        views). The computed-torque controller, the KinDyn queries and the link-level inertial data (ModelInfo tables,
+        the centre of mass used by the scenario module's wrench-at-CoM) stay nominal."""
+        check(self.lib.b2sim_enable_env_params(self.handle, model, 1 if enable else 0))
+        if not enable:
+            return None
+        nq = self.buffer(model, _lib.BUF_JOINT_DYNAMICS).cols // 2
+        inertia = self.tensor(model, _lib.BUF_BODY_INERTIA).view(self.num_envs, nq, 10)
+        dynamics = self.tensor(model, _lib.BUF_JOINT_DYNAMICS).view(self.num_envs, nq, 2)
+        return inertia, dynamics, self.tensor(model, _lib.BUF_GRAVITY)
+
     # ---- fused task path ----
     def set_task(self, model, task, seed=0, env_offset=0, max_episode_steps=5000):
         self.run_count = getattr(self, "run_count", 0) + 1  # the per-object view drops what it cached

@@ -616,9 +616,9 @@ __device__ __forceinline__ T pid_update(const T* g, T* st /* iErr, pErrLast, cmd
 
 // Joint-space constraint stage (joint limits, Coulomb friction, velocity servo): boxed LCP on
 // w = Minv lambda + b solved by projected Gauss-Seidel, Minv from CRBA + Cholesky.
-template <typename T, int NB>
+template <typename T, int NB, typename P = NominalParams<T>>
 __device__ void joint_constraints(const ModelDev<T>& m, T dt, const T* q, T* dq, const uint8_t* servo,
-                                  const T* servo_target, T* ddq)
+                                  const T* servo_target, T* ddq, const P& prm = P())
 {
     int rj[3 * NB];
     T rb[3 * NB], rlo[3 * NB], rhi[3 * NB], lam[3 * NB];
@@ -630,13 +630,14 @@ __device__ void joint_constraints(const ModelDev<T>& m, T dt, const T* q, T* dq,
             rj[nr] = j; rb[nr] = dq[j] - servo_target[j]; rlo[nr] = -m.effort[j] * dt; rhi[nr] = m.effort[j] * dt; ++nr;
             continue;
         }
-        if (m.friction[j] != T(0)) { rj[nr] = j; rb[nr] = dq[j]; rlo[nr] = -m.friction[j] * dt; rhi[nr] = m.friction[j] * dt; ++nr; }
+        const T friction = prm.friction(m, j);
+        if (friction != T(0)) { rj[nr] = j; rb[nr] = dq[j]; rlo[nr] = -friction * dt; rhi[nr] = friction * dt; ++nr; }
         if (q[j] <= m.lower[j]) { rj[nr] = j; rb[nr] = dq[j]; rlo[nr] = T(0); rhi[nr] = inf; ++nr; }
         if (q[j] >= m.upper[j]) { rj[nr] = j; rb[nr] = dq[j]; rlo[nr] = -inf; rhi[nr] = T(0); ++nr; }
     }
     if (nr == 0) return;
     T M[NB * NB], Minv[NB * NB];
-    mass_matrix<T, NB>(m, q, M);
+    mass_matrix<T, NB>(m, q, M, prm);
     spd_inverse(nq, M, Minv);
     for (int a = 0; a < nr; ++a) lam[a] = T(0);
     for (int it = 0; it < 200; ++it) {
@@ -688,10 +689,10 @@ __device__ __forceinline__ void stage_world(const WorldDev<T>* __restrict__ worl
 }
 
 // Rare path: some joint sits on a limit, has Coulomb friction or is velocity-servoed. Kept out of line so the
-// common path stays lean; works on local copies of q / dq.
-template <typename T, typename W>
+// common path stays lean; works on local copies of q / dq. `prm`: an env's EnvParams, or nothing for the model's tables.
+template <typename T, typename W, typename... P>
 __device__ __noinline__ void constraints_from_scratch(const ModelDev<T>& m, T dt, const W& w, uint32_t servo_bits,
-                                                      const T* __restrict__ vel_target_row)
+                                                      const T* __restrict__ vel_target_row, P... prm)
 {
     T q[kMaxDofs], dq[kMaxDofs], ddq[kMaxDofs], target[kMaxDofs];
     uint8_t servo[kMaxDofs];
@@ -703,7 +704,7 @@ __device__ __noinline__ void constraints_from_scratch(const ModelDev<T>& m, T dt
         servo[j] = (servo_bits >> j) & 1u;
         target[j] = servo[j] ? vel_target_row[j] : T(0);
     }
-    joint_constraints<T, kMaxDofs>(m, dt, q, dq, servo, target, ddq);
+    joint_constraints<T, kMaxDofs>(m, dt, q, dq, servo, target, ddq, prm...);
     for (int j = 0; j < nq; ++j) {
         w[kSlotsPerBody * j + SL_DQ] = dq[j];
         w[kSlotsPerBody * j + SL_TAU] = ddq[j];
@@ -727,13 +728,15 @@ template <typename T, typename C> __device__ __forceinline__ T* mass_matrix_slot
 
 // One physics iteration on the scratch state: ABA -> dq += ddq dt -> joint constraints -> q += dq dt.
 // SL_TAU holds the applied force on entry and the joint acceleration on return.
-template <typename T, typename W, typename C>
+// P: NominalParams, or the env's EnvParams (then topo.impulse_ok only covers the stiffness; the env's damping decides too).
+template <typename T, typename W, typename C, typename P = NominalParams<T>>
 __device__ __forceinline__ void tree_physics_iteration(const ModelDev<T>& m, const TreeTopo& topo, T dt, const W& w,
-                                                       uint32_t servo_bits, const T* __restrict__ vel_target_row, C& coupling)
+                                                       uint32_t servo_bits, const T* __restrict__ vel_target_row, C& coupling,
+                                                       const P& prm = P())
 {
     const int nq = m.nq;
     clear_parking_t<T>(nq, topo.nbranch, w);
-    forward_dynamics_fast(m, topo.slot, dt, w);
+    forward_dynamics_fast(m, topo.slot, dt, w, prm);
     for (int j = 0; j < nq; ++j) {
         const int o = kSlotsPerBody * j;
         w[o + SL_DQ] += w[o + SL_TAU] * dt;
@@ -743,9 +746,14 @@ __device__ __forceinline__ void tree_physics_iteration(const ModelDev<T>& m, con
     } else {
         int rj[kMaxRows];
         T rb[kMaxRows], rlo[kMaxRows], rhi[kMaxRows];
-        const int nr = collect_rows(m, dt, w, servo_bits, vel_target_row, rj, rb, rlo, rhi);
-        if (nr > 0 && topo.impulse_ok) constraints_fast(m, dt, w, nr, rj, rb, rlo, rhi);
-        else if (nr != 0) constraints_from_scratch(m, dt, w, servo_bits, vel_target_row);
+        const int nr = collect_rows(m, dt, w, servo_bits, vel_target_row, rj, rb, rlo, rhi, prm);
+        if constexpr (P::nominal) {
+            if (nr > 0 && topo.impulse_ok) constraints_fast(m, dt, w, nr, rj, rb, rlo, rhi);
+            else if (nr != 0) constraints_from_scratch(m, dt, w, servo_bits, vel_target_row);
+        } else {
+            if (nr > 0 && topo.impulse_ok && prm.undamped(m)) constraints_fast(m, dt, w, nr, rj, rb, rlo, rhi);
+            else if (nr != 0) constraints_from_scratch(m, dt, w, servo_bits, vel_target_row, prm);
+        }
     }
     if constexpr (!C::deferred) {  // deferred: the finishing kernel integrates after the warp-cooperative solve
         for (int j = 0; j < nq; ++j) {
@@ -842,10 +850,11 @@ __device__ __noinline__ void add_wrench_torques(const ModelDev<T>& m, const RunC
 }
 
 // GazeboSimulator::run for every env of a fixed-base tree. One thread per env; per-thread scratch columns in
-// dynamic shared memory (scratch_slots(nq, nbranch) * blockDim.x scalars).
-template <typename T, typename W, typename C>
+// dynamic shared memory (scratch_slots(nq, nbranch) * blockDim.x scalars). `prm` feeds the physics only: the
+// computed-torque controller keeps the nominal model (it loads its own copy of the model file in the reference).
+template <typename T, typename W, typename C, typename P = NominalParams<T>>
 __device__ __forceinline__ void run_tree_env(const ModelDev<T>& m, const RunCfg<T>& cfg, const RunBuffers<T>& b,
-                                             const TreeTopo& topo, int64_t e, const W& w, C& coupling)
+                                             const TreeTopo& topo, int64_t e, const W& w, C& coupling, const P& prm = P())
 {
     const int nq = cfg.nq;
     for (int j = 0; j < nq; ++j) {
@@ -891,7 +900,7 @@ __device__ __forceinline__ void run_tree_env(const ModelDev<T>& m, const RunCfg<
         }
         if (!cfg.paused) {
             if (cfg.nwrench) add_wrench_torques(m, cfg, e, it, w);
-            tree_physics_iteration(m, topo, cfg.dt, w, servo_bits, b.vel_target + e * nq, coupling);
+            tree_physics_iteration(m, topo, cfg.dt, w, servo_bits, b.vel_target + e * nq, coupling, prm);
             stepped = true;
         }
     }
@@ -902,10 +911,31 @@ __device__ __forceinline__ void run_tree_env(const ModelDev<T>& m, const RunCfg<
     }
 }
 
-// Shared-memory scratch: 64 threads per block, scratch_slots * 64 scalars of dynamic shared memory.
+// Per-env physical parameters of a model (b2sim_enable_env_params): B2_BUF_BODY_INERTIA [N][nq][10],
+// B2_BUF_JOINT_DYNAMICS [N][nq][2], B2_BUF_GRAVITY [N][3] (layouts: EnvParams, b2_rbd.hpp).
 template <typename T>
+struct EnvRows {
+    const T* inertia = nullptr;
+    const T* dyn = nullptr;
+    const T* grav = nullptr;
+    __host__ __device__ EnvParams<T> env(int64_t e, int nq) const
+    {
+        return EnvParams<T>{inertia + e * kEnvInertiaCols * nq, dyn + e * kEnvJointCols * nq, grav + 3 * e};
+    }
+};
+template <typename T, bool ENV> struct ParamsOf { using type = NominalParams<T>; };
+template <typename T> struct ParamsOf<T, true> { using type = EnvParams<T>; };
+template <bool ENV, typename T> __device__ __forceinline__ typename ParamsOf<T, ENV>::type params_of(const EnvRows<T>& rows, int64_t e, int nq)
+{
+    if constexpr (ENV) return rows.env(e, nq);
+    else return NominalParams<T>{};
+}
+
+// Shared-memory scratch: 64 threads per block, scratch_slots * 64 scalars of dynamic shared memory.
+// ENV: the physics reads every env's own inertias, damping, friction and gravity from `rows`.
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(64) k_run_tree(const ModelDev<T>* __restrict__ tables, const RunCfg<T> cfg,
-                                                 const RunBuffers<T> b, const TreeTopo topo)
+                                                 const RunBuffers<T> b, const TreeTopo topo, const EnvRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -913,13 +943,14 @@ __global__ void __launch_bounds__(64) k_run_tree(const ModelDev<T>* __restrict__
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= b.n) return;
     NoCoupling none;
-    run_tree_env(m, cfg, b, topo, e, Scratch<T>{reinterpret_cast<T*>(smem_raw) + threadIdx.x, (int)blockDim.x}, none);
+    run_tree_env(m, cfg, b, topo, e, Scratch<T>{reinterpret_cast<T*>(smem_raw) + threadIdx.x, (int)blockDim.x}, none,
+                 params_of<ENV>(rows, e, cfg.nq));
 }
 
 // Local-memory scratch (L1 / L2 backed): more resident threads per SM, for large env counts.
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(128) k_run_tree_local(const ModelDev<T>* __restrict__ tables, const RunCfg<T> cfg,
-                                                        const RunBuffers<T> b, const TreeTopo topo)
+                                                        const RunBuffers<T> b, const TreeTopo topo, const EnvRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     stage_model(tables, m);
@@ -927,7 +958,7 @@ __global__ void __launch_bounds__(128) k_run_tree_local(const ModelDev<T>* __res
     if (e >= b.n) return;
     T buf[kSlotsPerBody * kMaxDofs + kSlotsPerBranch * kMaxBranch];
     NoCoupling none;
-    run_tree_env(m, cfg, b, topo, e, Scratch<T, 1>{buf, 1}, none);
+    run_tree_env(m, cfg, b, topo, e, Scratch<T, 1>{buf, 1}, none, params_of<ENV>(rows, e, cfg.nq));
 }
 
 // ---------------------------------------------------------------------------------------------------------

@@ -59,51 +59,57 @@ cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T
 }
 
 namespace {
-template <typename T, int G, bool CT, bool COUPLED>
+template <typename T, int G, bool CT, bool COUPLED, bool ENV = false>
 cudaError_t launch_run_g(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const RunCfg<T>& cfg, const RunBuffers<T>& b,
-                         const TreeBits& tb, cudaStream_t stream, T* v0, int nvp)
+                         const TreeBits& tb, cudaStream_t stream, T* v0, int nvp, const EnvRows<T>& env)
 {
     using L = LaneLayout<G>;
     const int warps = b.n <= 8192 ? 2 : 4;
     const int64_t envs_per_block = (int64_t)warps * L::envs_per_warp;
     const int grid = (int)((b.n + envs_per_block - 1) / envs_per_block);
     const size_t smem = ((size_t)envs_per_block * L::stride + L::table + 12) * sizeof(T);
-    cudaError_t rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED, ENV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (rc != cudaSuccess) return rc;
     if (COUPLED) {  // must share SMs with k_coupled_rows / k_coupled_minv: the same shared-memory carve-out
-        rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED>, cudaFuncAttributePreferredSharedMemoryCarveout, kCoupledCarveout);
+        rc = cudaFuncSetAttribute(k_run_tree_lanes<T, G, CT, COUPLED, ENV>, cudaFuncAttributePreferredSharedMemoryCarveout, kCoupledCarveout);
         if (rc != cudaSuccess) return rc;
     }
     // a coupled step forks three kernels from one event: no programmatic overlap with the previous step's finish
-    return launch_pdl(k_run_tree_lanes<T, G, CT, COUPLED>, grid, 32 * warps, smem, stream, !COUPLED && b.n > 8192, tables, lane_table,
-                      cfg, b, tb, v0, nvp);
+    return launch_pdl(k_run_tree_lanes<T, G, CT, COUPLED, ENV>, grid, 32 * warps, smem, stream, !COUPLED && b.n > 8192, tables, lane_table,
+                      cfg, b, tb, v0, nvp, env);
 }
 template <typename T, int G>
 cudaError_t launch_run_v(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const RunCfg<T>& cfg, const RunBuffers<T>& b,
-                         const TreeBits& tb, cudaStream_t stream, T* v0, int nvp)
+                         const TreeBits& tb, cudaStream_t stream, T* v0, int nvp, const EnvRows<T>& env)
 {
     const bool ct = cfg.ct_active && !cfg.paused;
-    if (v0) return ct ? launch_run_g<T, G, true, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp)
-                      : launch_run_g<T, G, false, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp);
-    return ct ? launch_run_g<T, G, true, false>(tables, lane_table, cfg, b, tb, stream, v0, nvp)
-              : launch_run_g<T, G, false, false>(tables, lane_table, cfg, b, tb, stream, v0, nvp);
+    if (v0) return ct ? launch_run_g<T, G, true, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env)
+                      : launch_run_g<T, G, false, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
+    if (env.inertia) return ct ? launch_run_g<T, G, true, false, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env)
+                               : launch_run_g<T, G, false, false, true>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
+    return ct ? launch_run_g<T, G, true, false>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env)
+              : launch_run_g<T, G, false, false>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
 }
 }  // namespace
 
 template <typename T>
 cudaError_t launch_run_tree_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const RunCfg<T>& cfg,
-                                  const RunBuffers<T>& b, const int* parent, const int* jtype, cudaStream_t stream, T* v0, int nvp)
+                                  const RunBuffers<T>& b, const int* parent, const int* jtype, cudaStream_t stream, T* v0, int nvp,
+                                  const EnvRows<T>& env)
 {
+    if (v0 && env.inertia) return cudaErrorInvalidValue;  // no coupled variant with per-env parameters
     const TreeBits tb = make_tree_bits(cfg.nq, parent, jtype);
-    if (cfg.nq <= 8) return launch_run_v<T, 8>(tables, lane_table, cfg, b, tb, stream, v0, nvp);
-    if (cfg.nq <= 10) return launch_run_v<T, 10>(tables, lane_table, cfg, b, tb, stream, v0, nvp);
-    return launch_run_v<T, 16>(tables, lane_table, cfg, b, tb, stream, v0, nvp);
+    if (cfg.nq <= 8) return launch_run_v<T, 8>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
+    if (cfg.nq <= 10) return launch_run_v<T, 10>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
+    return launch_run_v<T, 16>(tables, lane_table, cfg, b, tb, stream, v0, nvp, env);
 }
 
 template cudaError_t launch_run_tree_lanes<double>(const ModelDev<double>*, const LaneTable<double>*, const RunCfg<double>&,
-                                                   const RunBuffers<double>&, const int*, const int*, cudaStream_t, double*, int);
+                                                   const RunBuffers<double>&, const int*, const int*, cudaStream_t, double*, int,
+                                                   const EnvRows<double>&);
 template cudaError_t launch_run_tree_lanes<float>(const ModelDev<float>*, const LaneTable<float>*, const RunCfg<float>&,
-                                                  const RunBuffers<float>&, const int*, const int*, cudaStream_t, float*, int);
+                                                  const RunBuffers<float>&, const int*, const int*, cudaStream_t, float*, int,
+                                                  const EnvRows<float>&);
 
 template cudaError_t launch_task_panda_lanes<double>(const ModelDev<double>*, const LaneTable<double>*, const PandaArgs<double>&,
                                                      const int*, const int*, cudaStream_t);

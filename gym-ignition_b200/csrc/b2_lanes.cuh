@@ -295,11 +295,22 @@ __device__ __forceinline__ void lanes_suffix(const TreeBits& tb, T* mine)
     }
 }
 
+// The lane's share of its env's rows of per-env parameters (k_run_tree_lanes<ENV>, EnvRows in b2_kernels.cuh): its body's
+// inertia record (mass, com, inertia about the com: 10 scalars, 16-byte aligned in fp64), its joint's damping and Coulomb
+// friction, the env's gravity.
+template <typename T>
+struct LaneRows {
+    const T* body = nullptr;
+    const T* joint = nullptr;
+    const T* g = nullptr;
+};
+
 // ---- forward dynamics of one env on its G lanes ----------------------------------------------------------------------
 // In: q, dq, tau of the lane's joint; (S|V) = world placements (lanes_forward_kinematics). Returns ddq of the lane's joint.
-template <typename T, int G>
+// ENV: inertia, damping and gravity come from `env` instead of the packed model constants.
+template <typename T, int G, bool ENV = false>
 __device__ __forceinline__ T lanes_forward_dynamics(const LaneCtx<T, G>& c, const ModelDev<T>& m, T dt, T q, T dq, T tau,
-                                                    T* inv_d_out = nullptr)
+                                                    T* inv_d_out = nullptr, const LaneRows<T>& env = LaneRows<T>())
 {
     using L = LaneLayout<G>;
     constexpr int NB = G;
@@ -319,10 +330,17 @@ __device__ __forceinline__ T lanes_forward_dynamics(const LaneCtx<T, G>& c, cons
         lanes_load_placement(c, R, p);
         T ax0, ax1, ax2, mass, ic[6], cm[3];
         ld2(t + LT_AXIS, ax0, ax1);
-        ld2(t + LT_AXIS + 2, ax2, mass);
-        ld2(t + LT_ICOM, ic[0], ic[1]); ld2(t + LT_ICOM + 2, ic[2], ic[3]); ld2(t + LT_ICOM + 4, ic[4], ic[5]);
-        ld2(t + LT_COM, cm[0], cm[1]);
-        cm[2] = t[LT_COM + 2];
+        if constexpr (ENV) {  // mass, com (3), inertia about the com (6)
+            const T* r = env.body;
+            ax2 = t[LT_AXIS + 2];
+            ld2(r, mass, cm[0]); ld2(r + 2, cm[1], cm[2]);
+            ld2(r + 4, ic[0], ic[1]); ld2(r + 6, ic[2], ic[3]); ld2(r + 8, ic[4], ic[5]);
+        } else {
+            ld2(t + LT_AXIS + 2, ax2, mass);
+            ld2(t + LT_ICOM, ic[0], ic[1]); ld2(t + LT_ICOM + 2, ic[2], ic[3]); ld2(t + LT_ICOM + 4, ic[4], ic[5]);
+            ld2(t + LT_COM, cm[0], cm[1]);
+            cm[2] = t[LT_COM + 2];
+        }
         const V3<T> aw = v3(R[0] * ax0 + R[1] * ax1 + R[2] * ax2, R[3] * ax0 + R[4] * ax1 + R[5] * ax2,
                             R[6] * ax0 + R[7] * ax1 + R[8] * ax2);
         if (rev) {
@@ -387,7 +405,7 @@ __device__ __forceinline__ T lanes_forward_dynamics(const LaneCtx<T, G>& c, cons
     __syncwarp();
     B2_MARK(6);
     // ---- F: accelerations without the joint accelerations, a_i = a_parent + c_i, gravity as base acceleration -g ----
-    if (c.live && c.l < 6) lanes_prefix<T, G, 6>(c.tb, PV + c.l, c.l >= 3 ? -m.g[c.l - 3] : T(0));
+    if (c.live && c.l < 6) lanes_prefix<T, G, 6>(c.tb, PV + c.l, c.l >= 3 ? -(ENV ? env.g[c.l - 3] : m.g[c.l - 3]) : T(0));
     __syncwarp();
     B2_MARK(7);
     // ---- G: net force on the body f = I a + V x* (I V); the lane's row of the mass matrix M[l][j] = F_l . S_j ----
@@ -402,7 +420,7 @@ __device__ __forceinline__ T lanes_forward_dynamics(const LaneCtx<T, G>& c, cons
         const V3<T> bn = cross(w, n) + cross(v, f), bf = cross(w, f);
         const T fo[6] = {Ia[0] + bn.x, Ia[1] + bn.y, Ia[2] + bn.z, Ia[3] + bf.x, Ia[4] + bf.y, Ia[5] + bf.z};
         st6(myV, fo);
-        D = c.tab[LT_DAMPING];
+        D = ENV ? env.joint[0] : c.tab[LT_DAMPING];
         ld2(c.tab + LT_STIFFNESS, K, rest);
     }
     T row[NB];
@@ -705,10 +723,11 @@ __device__ __noinline__ bool lanes_constraints_fast(const T* LT, T inv_d, int sl
 // of each such env runs the dense boxed LCP of the one-thread-per-env kernels on its env (b2_kernels.cuh joint_constraints).
 // Everything is passed by value: a reference to the lane context would force it (and the shared-memory pointer in it)
 // into local memory for the whole kernel.
-template <typename T, int G>
+// `prm`: the env's EnvParams (k_run_tree_lanes<ENV>), or nothing for the model's tables.
+template <typename T, int G, typename... P>
 __device__ __noinline__ void lanes_joint_constraints(T* x /* [4][G] exchange strip */, int l, int nq, bool body, bool solve,
                                                      const ModelDev<T>* m, T dt, T q, T* dq_io, T* ddq_io,
-                                                     unsigned servo_bits = 0u, T servo_target = T(0))
+                                                     unsigned servo_bits = 0u, T servo_target = T(0), P... prm)
 {
     T dq = *dq_io, ddq = *ddq_io;
     __syncwarp();
@@ -722,7 +741,7 @@ __device__ __noinline__ void lanes_joint_constraints(T* x /* [4][G] exchange str
             servo[j] = (servo_bits >> j) & 1u;
             target[j] = servo[j] ? x[3 * G + j] : T(0);
         }
-        joint_constraints<T, kMaxDofs>(*m, dt, qa, dqa, servo, target, ddqa);
+        joint_constraints<T, kMaxDofs>(*m, dt, qa, dqa, servo, target, ddqa, prm...);
         for (int j = 0; j < nq; ++j) { x[G + j] = dqa[j]; x[2 * G + j] = ddqa[j]; }
     }
     __syncwarp();
@@ -968,11 +987,15 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
 // COUPLED: the model belongs to a world with contacts (k_coupled_dynamics): the joint rows are solved together with the
 //   contacts by k_pgs_solve, so this kernel stops after the unconstrained velocity update, hands dq to the solver (v0),
 //   leaves the positions unintegrated and the pending-reset mask in place (k_world_finish integrates and clears it).
-template <typename T, int G, bool CT, bool COUPLED>
+// ENV (not with COUPLED): the physics reads every env's own inertias, damping, Coulomb friction and gravity from `rows`
+//   (b2sim_enable_env_params); the computed-torque controller keeps the packed nominal constants.
+template <typename T, int G, bool CT, bool COUPLED, bool ENV = false>
 __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __restrict__ tables,
                                                            const LaneTable<T>* __restrict__ lane_table, const RunCfg<T> cfg,
-                                                           const RunBuffers<T> b, const TreeBits tb, T* __restrict__ v0, int nvp)
+                                                           const RunBuffers<T> b, const TreeBits tb, T* __restrict__ v0, int nvp,
+                                                           const EnvRows<T> env_rows)
 {
+    static_assert(!(ENV && COUPLED), "per-env parameters are not supported in a coupled world");
     using L = LaneLayout<G>;
     constexpr int EPW = L::envs_per_warp;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1002,6 +1025,12 @@ __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __
     const bool pid_joint = cfg.controller_loaded && pid_mode;
     const bool control = !cfg.paused && cfg.controller_loaded && pid_mode;
     const bool has_fc = cfg.has_force_cmd[jl] != 0;
+    LaneRows<T> env;
+    if constexpr (ENV) {  // pointers only: lanes without a body never dereference theirs
+        env.body = env_rows.inertia + (e * nq + jl) * kEnvInertiaCols;
+        env.joint = env_rows.dyn + (e * nq + jl) * kEnvJointCols;
+        env.g = env_rows.grav + 3 * e;
+    }
     asm volatile("griddepcontrol.launch_dependents;");  // see k_task_panda_lanes
     lanes_stage_table<T, G>(lane_table, table);
     asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -1097,7 +1126,7 @@ __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __
                 }
             }
             T inv_d;
-            T ddq = lanes_forward_dynamics(c, m, cfg.dt, q, dq, tau, &inv_d);
+            T ddq = lanes_forward_dynamics<T, G, ENV>(c, m, cfg.dt, q, dq, tau, &inv_d, env);
             dq += ddq * cfg.dt;
             if (COUPLED) {  // the solver owns the constraint stage and k_world_finish the integration
                 acc = ddq;
@@ -1105,18 +1134,27 @@ __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __
                 continue;
             }
             // rows of joint_constraints: a servoed joint has its servo row only
-            const bool f0 = c.body && (servo || c.tab[LT_FRICTION] != T(0));
+            T env_friction = T(0), env_damping = T(0);  // ENV: the joint's row (read once, used below)
+            if (ENV && c.body) { env_damping = env.joint[0]; env_friction = env.joint[1]; }
+            const bool f0 = c.body && (servo || (ENV ? env_friction : c.tab[LT_FRICTION]) != T(0));
             const bool f1 = c.body && !servo && q <= c.tab[LT_LOWER], f2 = c.body && !servo && q >= c.tab[LT_UPPER];
             const unsigned rows = __ballot_sync(0xffffffffu, f0 || f1 || f2);
             if (rows) {
                 T dq_io = dq, ddq_io = ddq;
-                const bool dk = c.body && (c.tab[LT_DAMPING] != T(0) || c.tab[LT_STIFFNESS] != T(0));
+                const bool dk = c.body && ((ENV ? env_damping : c.tab[LT_DAMPING]) != T(0) || c.tab[LT_STIFFNESS] != T(0));
                 if (!lanes_constraints_fast<T, G>(c.sm + L::oP1 + L::oLT, inv_d, c.slot, c.l, nq, c.body, cfg.dt, f0, f1, f2, servo, vel_t,
-                                                  servo ? c.tab[LT_EFFORT] : c.tab[LT_FRICTION], dk, &dq_io, &ddq_io)) {
+                                                  servo ? c.tab[LT_EFFORT] : (ENV ? env_friction : c.tab[LT_FRICTION]), dk, &dq_io,
+                                                  &ddq_io)) {
                     const unsigned env_bits = (1u << G) - 1u;
                     const unsigned servos = __ballot_sync(0xffffffffu, servo);
-                    lanes_joint_constraints<T, G>(c.sm + L::oV, c.l, nq, c.body, c.l == 0 && ((rows >> (c.slot * G)) & env_bits) != 0u,
-                                                  tables, cfg.dt, q, &dq_io, &ddq_io, (servos >> (c.slot * G)) & env_bits, vel_t);
+                    // ENV: lane 0 solves its env with the env's own inertias and friction (the pack holds its EnvParams)
+                    const auto dense = [&](auto... prm) {
+                        lanes_joint_constraints<T, G>(c.sm + L::oV, c.l, nq, c.body, c.l == 0 && ((rows >> (c.slot * G)) & env_bits) != 0u,
+                                                      tables, cfg.dt, q, &dq_io, &ddq_io, (servos >> (c.slot * G)) & env_bits, vel_t,
+                                                      prm...);
+                    };
+                    if constexpr (ENV) dense(env_rows.env(e, nq));
+                    else dense();
                 }
                 dq = dq_io;
                 ddq = ddq_io;

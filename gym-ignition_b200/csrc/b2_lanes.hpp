@@ -17,9 +17,10 @@ cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T
 // computed-torque controller, resets, external link wrenches. v0 != nullptr: the model belongs to a coupled world; the
 // kernel stops after the unconstrained velocity update and writes the joint velocities into the solver's v0 rows
 // ([N, nvp]), leaving constraint solve, integration and the pending-reset mask to k_pgs_solve / k_world_finish.
+// env.inertia != nullptr: the physics reads every env's own parameters (b2sim_enable_env_params); not with v0.
 template <typename T>
 cudaError_t launch_run_tree_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const RunCfg<T>& cfg,
                                   const RunBuffers<T>& b, const int* parent, const int* jtype, cudaStream_t stream,
-                                  T* v0 = nullptr, int nvp = 0);
+                                  T* v0 = nullptr, int nvp = 0, const EnvRows<T>& env = EnvRows<T>());
 
 }  // namespace b2

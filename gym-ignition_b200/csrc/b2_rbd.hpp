@@ -261,6 +261,57 @@ template <typename T> B2_HD M3<T> ld9(const T* p)
     return A;
 }
 
+// Where the run path reads a body's inertia, a joint's viscous damping and Coulomb friction, and the gravity.
+// NominalParams: the model's shared tables. EnvParams: one env's rows of B2_BUF_BODY_INERTIA / B2_BUF_JOINT_DYNAMICS /
+// B2_BUF_GRAVITY (b2sim_enable_env_params); the first moment and the inertia about the body origin are derived from the
+// row where they are used, so no per-env copy of the model exists.
+template <typename T>
+struct NominalParams {
+    static constexpr bool nominal = true;
+    B2_HD T mass(const ModelDev<T>& m, int i) const { return m.mass[i]; }
+    B2_HD V3<T> mc(const ModelDev<T>& m, int i) const { return ld3(m.mc[i]); }
+    B2_HD M3<T> Io(const ModelDev<T>& m, int i) const { return ld9(m.Io[i]); }
+    B2_HD T damping(const ModelDev<T>& m, int i) const { return m.damping[i]; }
+    B2_HD T friction(const ModelDev<T>& m, int i) const { return m.friction[i]; }
+    B2_HD V3<T> g(const ModelDev<T>& m) const { return ld3(m.g); }
+    B2_HD bool undamped(const ModelDev<T>&) const { return true; }  // the host folded the tables' damping into the topology
+};
+
+// Row layouts: inertia [nq][10] = mass, centre of mass (x, y, z), rotational inertia about it (xx, xy, xz, yy, yz, zz),
+// body frame; dynamics [nq][2] = viscous damping, Coulomb friction; gravity [3], world frame.
+constexpr int kEnvInertiaCols = 10;
+constexpr int kEnvJointCols = 2;
+
+template <typename T>
+struct EnvParams {
+    static constexpr bool nominal = false;
+    const T* inertia;
+    const T* dyn;
+    const T* grav;
+    B2_HD T mass(const ModelDev<T>&, int i) const { return inertia[kEnvInertiaCols * i]; }
+    B2_HD V3<T> com(int i) const { return ld3(inertia + kEnvInertiaCols * i + 1); }
+    B2_HD V3<T> mc(const ModelDev<T>& m, int i) const { return mass(m, i) * com(i); }
+    // Ic + m (c.c 1 - c c^T), as the loader forms the shared tables (b2_model.cpp to_device_tables)
+    B2_HD M3<T> Io(const ModelDev<T>& m, int i) const
+    {
+        const T* r = inertia + kEnvInertiaCols * i;
+        const T mi = r[0], cx = r[1], cy = r[2], cz = r[3];
+        const T cc = cx * cx + cy * cy + cz * cz;
+        const T xy = r[5] - mi * (cx * cy), xz = r[6] - mi * (cx * cz), yz = r[8] - mi * (cy * cz);
+        return M3<T>{{r[4] + mi * (cc - cx * cx), xy, xz, xy, r[7] + mi * (cc - cy * cy), yz, xz, yz,
+                      r[9] + mi * (cc - cz * cz)}};
+    }
+    B2_HD T damping(const ModelDev<T>&, int i) const { return dyn[kEnvJointCols * i]; }
+    B2_HD T friction(const ModelDev<T>&, int i) const { return dyn[kEnvJointCols * i + 1]; }
+    B2_HD V3<T> g(const ModelDev<T>&) const { return ld3(grav); }
+    B2_HD bool undamped(const ModelDev<T>& m) const
+    {
+        bool z = true;
+        for (int i = 0; i < m.nq; ++i) z = z && dyn[kEnvJointCols * i] == T(0);
+        return z;
+    }
+};
+
 // Pose of the child frame of joint i in its parent body frame at position q.
 template <typename T> B2_HD void joint_pose(const ModelDev<T>& m, int i, T q, M3<T>& R, V3<T>& p)
 {
@@ -462,8 +513,9 @@ B2_HD void inverse_dynamics(const ModelDev<T>& m, const T* q, const T* dq, const
 }
 
 // Composite-rigid-body algorithm: joint-space mass matrix, row-major nq x nq (full, symmetric).
-template <typename T, int NB>
-B2_HD void mass_matrix(const ModelDev<T>& m, const T* q, T* M)
+// P: where the inertias come from (NominalParams / EnvParams); the controllers and KinDyn queries use the nominal model.
+template <typename T, int NB, typename Prm = NominalParams<T>>
+B2_HD void mass_matrix(const ModelDev<T>& m, const T* q, T* M, const Prm& prm = Prm())
 {
     M3<T> R[NB];
     V3<T> p[NB];
@@ -472,9 +524,9 @@ B2_HD void mass_matrix(const ModelDev<T>& m, const T* q, T* M)
     for (int k = 0; k < nq * nq; ++k) M[k] = T(0);  // entries between different branches stay zero
     for (int i = 0; i < nq; ++i) {
         joint_pose(m, i, q[i], R[i], p[i]);
-        const T mass = m.mass[i];
-        IC[i].A = ld9(m.Io[i]);
-        IC[i].B = skew(ld3(m.mc[i]));
+        const T mass = prm.mass(m, i);
+        IC[i].A = prm.Io(m, i);
+        IC[i].B = skew(prm.mc(m, i));
         IC[i].C = M3<T>{{mass, T(0), T(0), T(0), mass, T(0), T(0), T(0), mass}};
     }
     for (int i = nq - 1; i >= 0; --i) {

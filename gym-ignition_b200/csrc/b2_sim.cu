@@ -97,6 +97,7 @@ struct ModelState {
     uint64_t seed = 0, env_offset = 0, task_steps = 0;
     int max_episode_steps = 5000;
     double rand_mass_delta = 0, rand_gravity_sigma = 0;
+    bool env_params = false;  // B2_BUF_BODY_INERTIA / JOINT_DYNAMICS / GRAVITY allocated (b2sim_enable_env_params)
     unsigned long long* d_step = nullptr;  // device-side step counter of the fused task (next Philox step index)
     unsigned int* d_ticket = nullptr;
     bool graph_recorded = false;
@@ -217,6 +218,9 @@ void buffer_shape(const b2sim* s, const ModelState* ms, int which, int64_t* cols
     case B2_BUF_BASE_RESET: *cols = ms->kind == B2_KIND_FREE ? 13 : 0; break;
     case B2_BUF_EP_RETURN: *cols = ms->d_ep_totals ? 1 : 0; break;
     case B2_BUF_BASE_ACCEL: *cols = ms->kind == B2_KIND_FREE ? 6 : 0; break;
+    case B2_BUF_BODY_INERTIA: *cols = ms->env_params ? b2::kEnvInertiaCols * nq : 0; break;
+    case B2_BUF_JOINT_DYNAMICS: *cols = ms->env_params ? b2::kEnvJointCols * nq : 0; break;
+    case B2_BUF_GRAVITY: *cols = ms->env_params ? 3 : 0; break;
     default: *cols = 0; break;
     }
 }
@@ -316,6 +320,19 @@ b2::RunCfg<T> build_run_cfg(b2sim* s, ModelState* ms, int paused, int iterations
     return cfg;
 }
 
+// One thread per env: k_run_tree (scratch in shared memory, 64-thread blocks) or k_run_tree_local; ENV = the model's
+// per-env parameter rows are allocated.
+template <typename T, bool ENV>
+cudaError_t launch_run_thread(b2sim* s, const b2::ModelDev<T>* tb, const b2::RunCfg<T>& cfg, const b2::RunBuffers<T>& b,
+                              const b2::TreeTopo& topo, const b2::EnvRows<T>& env, size_t smem, bool local)
+{
+    cudaError_t rc = cudaFuncSetAttribute(b2::k_run_tree<T, ENV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (rc != cudaSuccess) return rc;
+    if (local) b2::k_run_tree_local<T, ENV><<<grid_for(s->n, 128), 128, 0, s->stream>>>(tb, cfg, b, topo, env);
+    else b2::k_run_tree<T, ENV><<<grid_for(s->n, 64), 64, smem, s->stream>>>(tb, cfg, b, topo, env);
+    return cudaGetLastError();
+}
+
 template <typename T>
 int launch_run(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t compute_bits, uint32_t ct_bits,
                const int* wrench_iters)
@@ -327,26 +344,30 @@ int launch_run(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t co
     int rc = tree_topology(ms, &topo);
     if (rc != B2_OK) return rc;
     const b2::ModelDev<T>* tb = (const b2::ModelDev<T>*)ms->d_tables;
+    b2::EnvRows<T> env;
+    if (ms->env_params) {
+        env.inertia = (const T*)ms->buf[B2_BUF_BODY_INERTIA];
+        env.dyn = (const T*)ms->buf[B2_BUF_JOINT_DYNAMICS];
+        env.grav = (const T*)ms->buf[B2_BUF_GRAVITY];
+        // the impulse path needs undamped joints: the tables' stiffness decides here, every env's damping row in the kernel
+        topo.impulse_ok = 1;
+        for (int j = 0; j < nq; ++j)
+            if (ms->model->t.stiffness[j] != 0.0) topo.impulse_ok = 0;
+    }
     if (nq >= 1 && nq <= b2::kMaxDofs && run_on_lanes(s, ms, 4)) {
         B2_CUDA(b2::launch_run_tree_lanes<T>(tb, (const b2::LaneTable<T>*)ms->d_lane_table, cfg, b, ms->model->t.parent,
-                                             ms->model->t.jtype, s->stream));
+                                             ms->model->t.jtype, s->stream, nullptr, 0, env));
         ++s->launches;
         return B2_OK;
     }
-    const int block = 64, grid = grid_for(s->n, block);
-    const size_t smem = (size_t)b2::scratch_slots(nq, topo.nbranch) * block * sizeof(T);
-    B2_CUDA(cudaFuncSetAttribute(b2::k_run_tree<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = (size_t)b2::scratch_slots(nq, topo.nbranch) * 64 * sizeof(T);  // 64-thread blocks
     // Scratch placement: shared memory keeps small batches fastest (two 64-thread blocks per SM); from ~64 k envs on,
     // L1/L2-backed local memory wins because more threads stay resident (1.4x at 1 M envs). B2_TREE_SCRATCH overrides.
     static const char* variant = getenv("B2_TREE_SCRATCH");
     const bool local = variant ? !strcmp(variant, "local") : s->n >= 65536;
-    if (local) {
-        b2::k_run_tree_local<T><<<grid_for(s->n, 128), 128, 0, s->stream>>>(tb, cfg, b, topo);
-    } else {
-        b2::k_run_tree<T><<<grid, block, smem, s->stream>>>(tb, cfg, b, topo);
-    }
+    B2_CUDA((ms->env_params ? launch_run_thread<T, true>(s, tb, cfg, b, topo, env, smem, local)
+                            : launch_run_thread<T, false>(s, tb, cfg, b, topo, env, smem, local)));
     ++s->launches;
-    B2_CUDA(cudaGetLastError());
     return B2_OK;
 }
 
@@ -1184,6 +1205,7 @@ int b2sim_set_gravity(b2sim* s, const double g[3])
     for (auto& ms : s->models)
         if (!ms->removed) {
             int rc = refresh_tables(s, ms.get());
+            for (int k = 0; k < 3 && rc == B2_OK && ms->env_params; ++k) rc = col_fill_any(s, ms->buf[B2_BUF_GRAVITY], 3, k, g[k]);
             if (rc != B2_OK) return rc;
         }
     s->world_dirty = true;  // the free-body world description carries the gravity vector too
@@ -1298,6 +1320,11 @@ int b2sim_run(b2sim* s, int paused)
         int rc = s->dtype == B2_F64 ? upload_world<double>(s) : upload_world<float>(s);
         if (rc != B2_OK) return rc;
     }
+    if (!s->free_models.empty())  // a free body inserted after b2sim_enable_env_params
+        for (auto& ms : s->models)
+            if (!ms->removed && ms->env_params)
+                return fail(B2_ERR_UNSUPPORTED, "model '%s' has per-env parameters and the world has free bodies",
+                            ms->name.c_str());
     // An articulated model with link collision shapes shares its constraint solve with the free bodies of the world
     const int coupled = (s->robot_model >= 0 && !s->free_models.empty()) ? s->robot_model : -1;
     uint32_t c_bits = 0, c_ct_bits = 0;
@@ -1599,6 +1626,15 @@ int b2sim_set_joint_friction(b2sim* s, int model, int joint, double coulomb, dou
     DeviceGuard guard__(s->device);
     if (coulomb >= 0) ms->model->t.friction[joint] = coulomb;  // negative: leave unchanged
     if (viscous >= 0) ms->model->t.damping[joint] = viscous;
+    if (ms->env_params) {  // "every env": the per-env rows follow
+        int rc = B2_OK;
+        if (viscous >= 0) rc = col_fill_any(s, ms->buf[B2_BUF_JOINT_DYNAMICS], b2::kEnvJointCols * ms->model->t.nq,
+                                            b2::kEnvJointCols * joint, viscous);
+        if (rc == B2_OK && coulomb >= 0)
+            rc = col_fill_any(s, ms->buf[B2_BUF_JOINT_DYNAMICS], b2::kEnvJointCols * ms->model->t.nq, b2::kEnvJointCols * joint + 1,
+                              coulomb);
+        if (rc != B2_OK) return rc;
+    }
     return refresh_tables(s, ms);  // the closed-form fit depends on the damping; Coulomb friction needs the tree path
 }
 
@@ -1860,6 +1896,54 @@ int b2sim_momentum_jacobian(b2sim* s, int model, void* momentum_jacobian, void* 
     return B2_OK;
 }
 
+// ---- per-env physical parameters ----------------------------------------------------------------------------------
+int b2sim_enable_env_params(b2sim* s, int model, int enable)
+{
+    ModelState* ms = get_model(s, model);
+    if (!ms) return fail(B2_ERR_NOT_FOUND, "model %d not found", model);
+    DeviceGuard guard__(s->device);
+    const int bufs[3] = {B2_BUF_BODY_INERTIA, B2_BUF_JOINT_DYNAMICS, B2_BUF_GRAVITY};
+    if (!enable) {
+        if (ms->env_params) B2_CUDA(cudaStreamSynchronize(s->stream));  // runs still queued read the rows
+        for (int which : bufs)
+            if (ms->buf[which]) { cudaFree(ms->buf[which]); ms->buf[which] = nullptr; }
+        ms->env_params = false;
+        return B2_OK;
+    }
+    const b2_model_tables& t = ms->model->t;
+    const int nq = t.nq;
+    if (nq == 0 || ms->kind == B2_KIND_FREE || ms->kind == B2_KIND_STATIC)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' is not a fixed-base articulated model", ms->name.c_str());
+    if (ms->task != B2_TASK_NONE)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' has a fused task, whose kernels read the shared tables only", ms->name.c_str());
+    for (auto& other : s->models)
+        if (!other->removed && other->kind == B2_KIND_FREE)
+            return fail(B2_ERR_UNSUPPORTED, "the world has free bodies: the coupled contact pipeline has no per-env parameters");
+    if (ms->env_params) return B2_OK;
+    ms->env_params = true;
+    int rc = B2_OK;
+    for (int which : bufs)
+        if (rc == B2_OK) rc = ensure_buffer(s, ms, which);
+    // every row starts from the model's current values: loader tables, set_joint_friction edits, world gravity
+    const int sym[6] = {0, 1, 2, 4, 5, 8};
+    for (int b = 0; b < nq && rc == B2_OK; ++b) {
+        double v[b2::kEnvInertiaCols] = {t.mass[b], t.com[b][0], t.com[b][1], t.com[b][2]};
+        for (int k = 0; k < 6; ++k) v[4 + k] = t.Ic[b][sym[k]];
+        for (int k = 0; k < b2::kEnvInertiaCols && rc == B2_OK; ++k)
+            rc = col_fill_any(s, ms->buf[B2_BUF_BODY_INERTIA], b2::kEnvInertiaCols * nq, b2::kEnvInertiaCols * b + k, v[k]);
+        if (rc == B2_OK) rc = col_fill_any(s, ms->buf[B2_BUF_JOINT_DYNAMICS], b2::kEnvJointCols * nq, b2::kEnvJointCols * b, t.damping[b]);
+        if (rc == B2_OK)
+            rc = col_fill_any(s, ms->buf[B2_BUF_JOINT_DYNAMICS], b2::kEnvJointCols * nq, b2::kEnvJointCols * b + 1, t.friction[b]);
+    }
+    for (int k = 0; k < 3 && rc == B2_OK; ++k) rc = col_fill_any(s, ms->buf[B2_BUF_GRAVITY], 3, k, s->gravity[k]);
+    if (rc != B2_OK) {
+        std::string msg = g_error;
+        b2sim_enable_env_params(s, model, 0);
+        return fail(rc, "%s", msg.c_str());
+    }
+    return B2_OK;
+}
+
 // ---- zero-copy view --------------------------------------------------------------------------------------------
 int b2sim_buffer(b2sim* s, int model, int which, b2_buffer* out)
 {
@@ -1901,6 +1985,9 @@ int b2sim_set_task(b2sim* s, int model, int task, uint64_t seed, uint64_t env_of
     if (!ms) return fail(B2_ERR_NOT_FOUND, "model %d not found", model);
     if (b2sim_task_nobs(task) == 0) return fail(B2_ERR_UNSUPPORTED, "unknown task %d", task);
     if (max_episode_steps <= 0 || max_episode_steps > 65535) return fail(B2_ERR_INVALID, "max_episode_steps out of range");
+    if (ms->env_params)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' has per-env parameters: the fused task kernels read the shared tables only",
+                    ms->name.c_str());
     DeviceGuard guard__(s->device);
     const b2_model_tables& t = ms->model->t;
     if (task == B2_TASK_PANDA_REACH) {

@@ -121,9 +121,10 @@ B2_HD void joint_pose_sc(const ModelDev<T>& m, int i, T s, T c, T q, M3<T>& R, V
 
 // Forward dynamics (implicit damping/spring). On entry the SL_Q / SL_DQ / SL_TAU slots of every body hold
 // q, dq and the applied joint force, and the parking slots are zero (clear_parking). On return SL_TAU holds
-// the joint acceleration of the body; SL_Q / SL_DQ are untouched.
-template <typename T, typename W>
-B2_HD void forward_dynamics_fast(const ModelDev<T>& m, const int* branch_slot, T dt, const W& w)
+// the joint acceleration of the body; SL_Q / SL_DQ are untouched. P: where inertias, damping and gravity come from
+// (NominalParams: the model's tables, EnvParams: one env's rows).
+template <typename T, typename W, typename P = NominalParams<T>>
+B2_HD void forward_dynamics_fast(const ModelDev<T>& m, const int* branch_slot, T dt, const W& w, const P& prm = P())
 {
     const int nq = m.nq;
     const int park0 = kSlotsPerBody * nq;
@@ -165,10 +166,13 @@ B2_HD void forward_dynamics_fast(const ModelDev<T>& m, const int* branch_slot, T
         const Sv<T> V = {{w[o + SL_V], w[o + SL_V + 1], w[o + SL_V + 2]},
                          {w[o + SL_V + 3], w[o + SL_V + 4], w[o + SL_V + 5]}};
         // rigid-body part
-        const T mass = m.mass[i];
-        const V3<T> mc = ld3(m.mc[i]);
+        const T mass = prm.mass(m, i);
+        const V3<T> mc = prm.mc(m, i);
         AiS<T> IA;
-        IA.A = {m.Io[i][0], m.Io[i][1], m.Io[i][2], m.Io[i][4], m.Io[i][5], m.Io[i][8]};
+        {
+            const M3<T> Io = prm.Io(m, i);
+            IA.A = {Io.m[0], Io.m[1], Io.m[2], Io.m[4], Io.m[5], Io.m[8]};
+        }
         IA.B = skew(mc);
         IA.C = {mass, T(0), T(0), mass, T(0), mass};
         Sv<T> pA;
@@ -211,10 +215,11 @@ B2_HD void forward_dynamics_fast(const ModelDev<T>& m, const int* branch_slot, T
             U = {mul(IA.B, a), mul(IA.C, a)};
             d = dot(a, U.l);
         }
-        d += dt * m.damping[i] + dt * dt * m.stiffness[i];
+        const T damping = prm.damping(m, i);
+        d += dt * damping + dt * dt * m.stiffness[i];
         const T psi = T(1) / d;
         const Sv<T> pa = {mul(IA.A, eta.a) + mul(IA.B, eta.l) + pA.a, mulT(IA.B, eta.a) + mul(IA.C, eta.l) + pA.l};
-        const T u = w[o + SL_TAU] - m.damping[i] * dq - m.stiffness[i] * (q - m.rest[i] + dt * dq) -
+        const T u = w[o + SL_TAU] - damping * dq - m.stiffness[i] * (q - m.rest[i] + dt * dq) -
                     (rev ? dot(a, pa.a) : dot(a, pa.l));
         w[o + SL_U + 0] = U.a.x; w[o + SL_U + 1] = U.a.y; w[o + SL_U + 2] = U.a.z;
         w[o + SL_U + 3] = U.l.x; w[o + SL_U + 4] = U.l.y; w[o + SL_U + 5] = U.l.z;
@@ -272,7 +277,7 @@ B2_HD void forward_dynamics_fast(const ModelDev<T>& m, const int* branch_slot, T
     }
 
     // ---- pass 3: accelerations, root to leaves (the V slots are overwritten by spatial accelerations) ----
-    const V3<T> g_base = mulT(ld9(m.baseR), ld3(m.g));
+    const V3<T> g_base = mulT(ld9(m.baseR), prm.g(m));
     for (int i = 0; i < nq; ++i) {
         const int o = kSlotsPerBody * i, par = m.parent[i];
         const bool rev = m.jtype[i] == kRevolute;
@@ -379,9 +384,9 @@ B2_HD void impulse_response(const ModelDev<T>& m, const W& w, int nr, const int*
 
 // Collects the active rows (joint, b, lo, hi). Returns the row count, or -1 when more than kMaxRows are active.
 // servo_bits: joints under a velocity servo (VelocityFollowerDart), servo_target: their target velocities.
-template <typename T, typename W>
+template <typename T, typename W, typename P = NominalParams<T>>
 B2_HD int collect_rows(const ModelDev<T>& m, T dt, const W& w, unsigned servo_bits, const T* servo_target,
-                       int* rj, T* rb, T* rlo, T* rhi)
+                       int* rj, T* rb, T* rlo, T* rhi, const P& prm = P())
 {
     int nr = 0;
     const T inf = T(INFINITY);
@@ -392,9 +397,10 @@ B2_HD int collect_rows(const ModelDev<T>& m, T dt, const W& w, unsigned servo_bi
             rj[nr] = j; rb[nr] = dq - servo_target[j]; rlo[nr] = -m.effort[j] * dt; rhi[nr] = m.effort[j] * dt; ++nr;
             continue;
         }
-        if (m.friction[j] != T(0)) {
+        const T friction = prm.friction(m, j);
+        if (friction != T(0)) {
             if (nr >= kMaxRows) return -1;
-            rj[nr] = j; rb[nr] = dq; rlo[nr] = -m.friction[j] * dt; rhi[nr] = m.friction[j] * dt; ++nr;
+            rj[nr] = j; rb[nr] = dq; rlo[nr] = -friction * dt; rhi[nr] = friction * dt; ++nr;
         }
         if (q <= m.lower[j]) {
             if (nr >= kMaxRows) return -1;

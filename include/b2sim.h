@@ -100,7 +100,12 @@ enum {
     B2_BUF_BASE_ACCEL = 19,  /* [N, 6] B2_KIND_FREE: world linear acceleration of the base frame origin and angular acceleration
                               * over the last step, constraint impulses included (Link::world{Linear,Angular}Acceleration,
                               * Link.cpp:240-294; DART adds the velocity change of the constraint stage / dt to the accelerations) */
-    B2_BUF_COUNT = 20
+    /* Per-env physical parameters (b2sim_enable_env_params), read by every unpaused b2sim_run of the model: */
+    B2_BUF_BODY_INERTIA = 20,   /* [N, 10*nq] per body j (child of joint j, welded links lumped in as in b2_model_tables):
+                                 * mass, centre of mass xyz, inertia about it Ixx Ixy Ixz Iyy Iyz Izz, both in the body frame */
+    B2_BUF_JOINT_DYNAMICS = 21, /* [N, 2*nq] per joint: viscous damping, Coulomb friction */
+    B2_BUF_GRAVITY = 22,        /* [N, 3] gravity this model's dynamics sees in the env, world frame */
+    B2_BUF_COUNT = 23
 };
 
 typedef struct {
@@ -221,6 +226,21 @@ int b2sim_set_max_generalized_force(b2sim* s, int model, int joint, double f); /
  * joint, for every env; a negative value leaves that parameter unchanged. The caller enforces the reference's
  * "only while the model has just been created" rule (helpers.cpp:131-157). */
 int b2sim_set_joint_friction(b2sim* s, int model, int joint, double coulomb, double viscous);
+/* Per-env physical parameters (domain randomisation of articulated models: the batched counterpart of editing the SDF and
+ * re-inserting the model at a reset, gym_ignition/randomizers/gazebo_env_randomizer.py). enable != 0 allocates
+ * B2_BUF_BODY_INERTIA, B2_BUF_JOINT_DYNAMICS and B2_BUF_GRAVITY in the simulator dtype and fills every row with the
+ * model's current values (loader tables, b2sim_set_joint_friction edits, world gravity). The caller owns the rows: a write
+ * on the simulator stream between runs acts from the next run on. b2sim_set_joint_friction and b2sim_set_gravity keep
+ * their "every env" meaning and overwrite their column in every row. enable = 0 frees the buffers and the model returns to
+ * the shared tables; pointers from b2sim_buffer taken before are then invalid. What stays nominal: the computed-torque
+ * controller (the reference's ComputedTorqueFixedBase loads its own copy of the model file), the KinDyn queries
+ * (b2sim_kindyn, b2sim_centroidal, b2sim_momentum_jacobian, b2sim_update_kinematics, b2sim_link_motion:
+ * KinDynComputations is built from the model file), and the per-link inertial data of the loader (b2model_tables:
+ * link_mass, link_com, which a wrench applied at a link's centre of mass uses): the rows describe lumped bodies, not
+ * links, so a per-link centre of mass cannot be derived from them. B2_ERR_UNSUPPORTED for a
+ * free-floating or static model, a model with a fused task, and a world with free bodies (also from b2sim_run when a free
+ * body is inserted later); b2sim_set_task refuses a model with per-env parameters. */
+int b2sim_enable_env_params(b2sim* s, int model, int enable);
 
 /* ---- custom controller: ComputedTorqueFixedBase run by ControllerRunner -------------------------------- */
 /* Model::insertModelPlugin("ControllerRunner", ...) with a <controller name="ComputedTorqueFixedBase"> context

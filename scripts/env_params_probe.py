@@ -1,0 +1,92 @@
+"""Cost of per-env physical parameters (Simulator.enable_env_params) on GazeboSimulator::run of Pandas under position PIDs.
+
+Two simulators with the same Pandas, targets and gains (those of run_probe.py), one with its own random rows per env
+(masses x U(0.8, 1.2), inertias alike, damping U(0, 0.1), gravity tilted by up to ~3 degrees), the other on the shared
+tables. Blocks of `runs` b2sim_run calls alternate between the two in one process and are timed with CUDA events; the
+median of 5 blocks per variant is reported. The batch size selects the kernel: 4,096 and 16,384 envs run on lanes
+(k_run_tree_lanes), 20,001 on k_run_tree and 65,536 on k_run_tree_local.
+
+    python scripts/env_params_probe.py [runs_per_block]
+"""
+import os
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+SIZES = {4096: "k_run_tree_lanes", 16384: "k_run_tree_lanes", 20001: "k_run_tree", 65536: "k_run_tree_local"}
+GAINS = [(50, 0, 20), (10000, 0, 500), (100, 0, 10), (1000, 0, 50), (100, 0, 10), (100, 0, 10), (10, 0.5, 0.1), (100, 0, 50),
+         (100, 0, 50)]
+
+
+def card():
+    out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
+                         text=True, check=True).stdout
+    return out.strip().splitlines()[0]
+
+
+def panda_sim(n, env_params, seed):
+    import torch
+    import b2sim
+    import gym_ignition_models
+    from b2sim import _lib as L
+    from b2sim.batched import PANDA_Q0
+    sim = b2sim.Simulator(n, 0.001, 1)
+    mid = sim.insert_model_file(gym_ignition_models.get_model_file("panda"))
+    for j in range(9):
+        sim.set_joint(mid, L.FIELD_POSITION_RESET, -1, j, PANDA_Q0[j])
+    sim.run(paused=True)
+    big = 1.7976931348623157e308
+    sim.set_controller_period(mid, 0.001)
+    for j, (p, i, d) in enumerate(GAINS):
+        sim.set_pid(mid, j, p, i, d, big, -big, big, -big, 0.0)
+        sim.set_control_mode(mid, j, 5)
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(seed)
+    f64 = dict(device="cuda", dtype=torch.float64)
+    tg = sim.tensor(mid, L.BUF_POS_TARGET)
+    tg.copy_(torch.tensor(PANDA_Q0, **f64) + 0.1 * torch.sin(torch.rand(n, 1, generator=gen, **f64) * 6.28))
+    tg[:, 7:] = 0.02
+    if env_params:
+        inertia, dyn, g = sim.enable_env_params(mid)
+        s = 0.8 + 0.4 * torch.rand(n, 9, 1, generator=gen, **f64)
+        inertia[:, :, 0:1] *= s
+        inertia[:, :, 4:] *= s
+        dyn[:, :, 0] = 0.1 * torch.rand(n, 9, generator=gen, **f64)
+        g[:, :2] = 0.5 * (torch.rand(n, 2, generator=gen, **f64) - 0.5)
+    return sim
+
+
+def main():
+    sys.path.insert(0, ROOT)
+    import __graft_entry__
+    __graft_entry__.load_package()
+    import numpy as np
+    import torch
+    runs = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
+    print(f"card: {card()}", flush=True)
+    for n, kernel in SIZES.items():
+        sims = {"off": panda_sim(n, False, 3), "on": panda_sim(n, True, 3)}
+        for sim in sims.values():  # warm-up: module loads, clocks
+            for _ in range(200):
+                sim.run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in sims}
+        for block in range(5):
+            for name, sim in sims.items():
+                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                a.record()
+                for _ in range(runs):
+                    sim.run()
+                b.record()
+                torch.cuda.synchronize()
+                times[name].append(a.elapsed_time(b) / runs * 1e3)
+        off, on = (float(np.median(times[k])) for k in ("off", "on"))
+        spread = {k: (min(v), max(v)) for k, v in times.items()}
+        print(f"n={n:6d} {kernel:17s} off {off:7.2f} us/run (blocks {spread['off'][0]:.2f}-{spread['off'][1]:.2f})  "
+              f"on {on:7.2f} us/run (blocks {spread['on'][0]:.2f}-{spread['on'][1]:.2f})  on/off {on / off:.3f}", flush=True)
+        for sim in sims.values():
+            sim.close()
+
+
+if __name__ == "__main__":
+    main()
