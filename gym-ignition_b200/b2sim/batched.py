@@ -71,6 +71,8 @@ class BatchedTaskEnv:
         self.nobs = self.obs.shape[1]
         self.nact = self.sim.buffer(self.model, _lib.BUF_ACTION).cols
         self.bytes_per_env_step = ALGORITHMIC_BYTES[self.task][dtype]
+        self.rand_params = self.env_params = None
+        self.episode_stats_enabled = False
 
     def randomize(self, mass_delta: float = 0.2, gravity_sigma: float = 0.2):
         """Per-env domain randomisation (randomizers/cartpole.py:51-56,100-135): at every reset an env draws link
@@ -85,14 +87,32 @@ class BatchedTaskEnv:
                 (8 if self.dtype == "float64" else 4) * self.rand_params.shape[1]
         return self.rand_params
 
+    def enable_env_params(self, enable: bool = True):
+        """Per-env body inertias, joint damping / Coulomb friction and gravity for the reach task
+        (``Simulator.enable_env_params``; the pendulum and cart-pole tasks raise B2Error and have ``randomize``). Returns
+        the views (body_inertia [N, nq, 10], joint_dynamics [N, nq, 2], gravity [N, 3]), or None when disabling. Every
+        step reads them (+(12 nq + 3) scalars of traffic per env-step). For new parameters per episode, write the rows of
+        the envs whose ``done`` is set (e.g. with torch.where on the done mask) after the step that reports it and before
+        the next one: the terminal step ran with the old rows, the new episode runs with the new ones. The reach task
+        ends at its TimeLimit only, so its envs finish together unless ``elapsed`` is staggered."""
+        self.env_params = self.sim.enable_env_params(self.model, enable)
+        self._count_bytes()
+        return self.env_params
+
     def enable_episode_stats(self, enable: bool = True) -> None:
         """Let the step kernels accumulate [sum of returns, sum of lengths, finished episodes, non-finite rewards] on
         the device (two extra scalars of traffic per env-step). Read them with ``episode_stats()`` or hand them to
         ``b2sim.distributed.EpisodeStats`` for the end-of-rollout sum over ranks."""
         self.sim.episode_stats_enable(self.model, enable)
+        self.episode_stats_enabled = enable
+        self._count_bytes()
+
+    def _count_bytes(self) -> None:
+        """bytes_per_env_step: the task's traffic plus what the enabled per-env extras read or write per env-step."""
         es = 8 if self.dtype == "float64" else 4
-        self.bytes_per_env_step = ALGORITHMIC_BYTES[self.task][self.dtype] + (2 * es if enable else 0) + \
-            (es * self.rand_params.shape[1] if getattr(self, "rand_params", None) is not None else 0)
+        self.bytes_per_env_step = ALGORITHMIC_BYTES[self.task][self.dtype] + (2 * es if self.episode_stats_enabled else 0) + \
+            (es * self.rand_params.shape[1] if self.rand_params is not None else 0) + \
+            (es * sum(v[0].numel() for v in self.env_params) if self.env_params is not None else 0)
 
     def episode_stats(self, clear: bool = False):
         """Host copy of the four totals (synchronises the stream)."""

@@ -1046,8 +1046,11 @@ __device__ __forceinline__ void warp_store_rows(T* __restrict__ g, int64_t row0,
     }
 }
 
-template <typename T>
-__global__ void __launch_bounds__(128) k_task_panda(const ModelDev<T>* __restrict__ tables, const PandaArgs<T> a, const TreeTopo topo)
+// ENV: the physics reads every env's own inertias, damping, Coulomb friction and gravity from `rows`
+// (b2sim_enable_env_params); the observation is kinematic and reads none of them.
+template <typename T, bool ENV = false>
+__global__ void __launch_bounds__(128) k_task_panda(const ModelDev<T>* __restrict__ tables, const PandaArgs<T> a, const TreeTopo topo,
+                                                    const EnvRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     __shared__ T tiles[4][32 * (kTileCols + 1)];
@@ -1078,7 +1081,7 @@ __global__ void __launch_bounds__(128) k_task_panda(const ModelDev<T>* __restric
                 w[kSlotsPerBody * j + SL_TAU] = pid_update(a.pid[j], pst + 3 * j, w[kSlotsPerBody * j + SL_Q] - target, a.dt);
             }
             NoCoupling none;
-            tree_physics_iteration(m, topo, a.dt, w, 0u, (const T*)nullptr, none);
+            tree_physics_iteration(m, topo, a.dt, w, 0u, (const T*)nullptr, none, params_of<ENV>(rows, e, nq));
         }
         // ---- forward kinematics along the chain to the end effector (world axis / origin go to the V slots) ----
         const int body = m.link_body[a.ee_link];

@@ -27,9 +27,9 @@ cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t sme
     return cudaLaunchKernelEx(&lc, kernel, KArgs(args)...);
 }
 
-template <typename T, int G, int NQ, unsigned P_LO = 0u, unsigned P_HI = 0u, unsigned REV = 0u>
+template <typename T, int G, int NQ, unsigned P_LO = 0u, unsigned P_HI = 0u, unsigned REV = 0u, bool ENV = false>
 cudaError_t launch_panda_g(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a, const TreeBits& tb,
-                           cudaStream_t stream)
+                           cudaStream_t stream, const EnvRows<T>& env)
 {
     using L = LaneLayout<G>;
     // 64-thread blocks spread small batches over more SMs (4,096 envs: 14.4 us against 16.5 us), 128-thread blocks share
@@ -38,24 +38,34 @@ cudaError_t launch_panda_g(const ModelDev<T>* tables, const LaneTable<T>* lane_t
     const int64_t envs_per_block = (int64_t)warps * L::envs_per_warp;
     const int grid = (int)((a.n + envs_per_block - 1) / envs_per_block);
     const size_t smem = ((size_t)envs_per_block * L::stride + L::table + 12) * sizeof(T);
-    cudaError_t rc = cudaFuncSetAttribute(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t rc = cudaFuncSetAttribute(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV, ENV>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem);
     if (rc != cudaSuccess) return rc;
-    return launch_pdl(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV>, grid, 32 * warps, smem, stream, a.n > 8192, tables, lane_table, a, tb);
+    return launch_pdl(k_task_panda_lanes<T, G, NQ, P_LO, P_HI, REV, ENV>, grid, 32 * warps, smem, stream, a.n > 8192, tables, lane_table,
+                      a, tb, env);
+}
+// env.inertia != nullptr selects the per-env parameter variant of the same specialisation
+template <typename T, int G, int NQ, unsigned P_LO = 0u, unsigned P_HI = 0u, unsigned REV = 0u>
+cudaError_t launch_panda_v(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a, const TreeBits& tb,
+                           cudaStream_t stream, const EnvRows<T>& env)
+{
+    return env.inertia ? launch_panda_g<T, G, NQ, P_LO, P_HI, REV, true>(tables, lane_table, a, tb, stream, env)
+                       : launch_panda_g<T, G, NQ, P_LO, P_HI, REV>(tables, lane_table, a, tb, stream, env);
 }
 }  // namespace
 
 template <typename T>
 cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a,
-                                    const int* parent, const int* jtype, cudaStream_t stream)
+                                    const int* parent, const int* jtype, cudaStream_t stream, const EnvRows<T>& env)
 {
     const TreeBits tb = make_tree_bits(a.nq, parent, jtype);
-    if (a.nq <= 8) return launch_panda_g<T, 8, 0>(tables, lane_table, a, tb, stream);
+    if (a.nq <= 8) return launch_panda_v<T, 8, 0>(tables, lane_table, a, tb, stream, env);
     // the Panda (a chain of 7 revolute joints, two prismatic fingers on the last arm body): tree known at compile time
     constexpr unsigned kPandaLo = 0x76543210u, kPandaHi = 0x7u, kPandaRev = 0x7fu;
     if (a.nq == 9 && tb.p_lo == kPandaLo && tb.p_hi == kPandaHi && tb.rev_mask == kPandaRev)
-        return launch_panda_g<T, 10, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream);
-    if (a.nq <= 10) return launch_panda_g<T, 10, 0>(tables, lane_table, a, tb, stream);
-    return launch_panda_g<T, 16, 0>(tables, lane_table, a, tb, stream);
+        return launch_panda_v<T, 10, 9, kPandaLo, kPandaHi, kPandaRev>(tables, lane_table, a, tb, stream, env);
+    if (a.nq <= 10) return launch_panda_v<T, 10, 0>(tables, lane_table, a, tb, stream, env);
+    return launch_panda_v<T, 16, 0>(tables, lane_table, a, tb, stream, env);
 }
 
 namespace {
@@ -112,8 +122,8 @@ template cudaError_t launch_run_tree_lanes<float>(const ModelDev<float>*, const 
                                                   const EnvRows<float>&);
 
 template cudaError_t launch_task_panda_lanes<double>(const ModelDev<double>*, const LaneTable<double>*, const PandaArgs<double>&,
-                                                     const int*, const int*, cudaStream_t);
+                                                     const int*, const int*, cudaStream_t, const EnvRows<double>&);
 template cudaError_t launch_task_panda_lanes<float>(const ModelDev<float>*, const LaneTable<float>*, const PandaArgs<float>&,
-                                                    const int*, const int*, cudaStream_t);
+                                                    const int*, const int*, cudaStream_t, const EnvRows<float>&);
 
 }  // namespace b2

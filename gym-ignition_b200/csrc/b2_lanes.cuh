@@ -761,10 +761,12 @@ __device__ __noinline__ void lanes_joint_constraints(T* x /* [4][G] exchange str
 // constant: the launcher instantiates the Panda's and dispatches on a match with the loaded model. Every `i < nq` guard,
 // parent lookup and chain / branch decision of the unrolled body loops then folds away (about a third of the kernel's
 // instructions). NQ = 0 reads the tree from the arguments.
-template <typename T, int G, int NQ, unsigned P_LO, unsigned P_HI, unsigned REV>
+// ENV: the physics reads every env's own inertias, damping, Coulomb friction and gravity from `env_rows`
+// (b2sim_enable_env_params), as k_run_tree_lanes<ENV> does; the observation is kinematic and reads none of them.
+template <typename T, int G, int NQ, unsigned P_LO, unsigned P_HI, unsigned REV, bool ENV = false>
 __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* __restrict__ tables,
                                                        const LaneTable<T>* __restrict__ lane_table, const PandaArgs<T> a,
-                                                       const TreeBits tb_arg)
+                                                       const TreeBits tb_arg, const EnvRows<T> env_rows)
 {
     const TreeBits tb = NQ > 0 ? TreeBits{P_LO, P_HI, REV, NQ, {0}} : tb_arg;  // the ancestor masks are read from tb_arg
     using L = LaneLayout<G>;
@@ -793,6 +795,12 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
     c.tab = table + L::REC * jl;
     c.anc = c.l < c.nq ? tb_arg.anc[c.l] : 0u;
     const int nobs = panda_obs_size(nq);
+    LaneRows<T> env;
+    if constexpr (ENV) {  // pointers only: lanes without a body never dereference theirs
+        env.body = env_rows.inertia + (e * nq + jl) * kEnvInertiaCols;
+        env.joint = env_rows.dyn + (e * nq + jl) * kEnvJointCols;
+        env.g = env_rows.grav + 3 * e;
+    }
 
     // Programmatic dependent launch (the launcher sets the stream-serialization attribute): the next step's blocks are
     // scheduled while this grid drains and stage the model constants (written at set-up, never by a step) before they
@@ -823,18 +831,27 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
         lanes_forward_kinematics(c, m, warp_strips, live_envs);
         B2_MARK(3);
         T inv_d;
-        T ddq = lanes_forward_dynamics(c, m, a.dt, q, dq, tau, &inv_d);
+        T ddq = lanes_forward_dynamics<T, G, ENV>(c, m, a.dt, q, dq, tau, &inv_d, env);
         dq += ddq * a.dt;
-        const bool f0 = c.body && c.tab[LT_FRICTION] != T(0), f1 = c.body && q <= c.tab[LT_LOWER], f2 = c.body && q >= c.tab[LT_UPPER];
+        T env_friction = T(0), env_damping = T(0);  // ENV: the joint's row (read once, used below)
+        if (ENV && c.body) { env_damping = env.joint[0]; env_friction = env.joint[1]; }
+        const bool f0 = c.body && (ENV ? env_friction : c.tab[LT_FRICTION]) != T(0), f1 = c.body && q <= c.tab[LT_LOWER],
+                   f2 = c.body && q >= c.tab[LT_UPPER];
         const unsigned rows = __ballot_sync(0xffffffffu, f0 || f1 || f2);
         if (rows) {
             T dq_io = dq, ddq_io = ddq;  // copies: the out-of-line calls must not pin the kernel's registers to memory
-            const bool dk = c.body && (c.tab[LT_DAMPING] != T(0) || c.tab[LT_STIFFNESS] != T(0));
+            const bool dk = c.body && ((ENV ? env_damping : c.tab[LT_DAMPING]) != T(0) || c.tab[LT_STIFFNESS] != T(0));
             if (!lanes_constraints_fast<T, G>(c.sm + L::oP1 + L::oLT, inv_d, c.slot, c.l, nq, c.body, a.dt, f0, f1, f2, false, T(0),
-                                              c.tab[LT_FRICTION], dk, &dq_io, &ddq_io))
-                lanes_joint_constraints<T, G>(c.sm + L::oV, c.l, nq, c.body,
-                                              c.l == 0 && ((rows >> (c.slot * G)) & ((1u << G) - 1u)) != 0u, tables, a.dt, q,
-                                              &dq_io, &ddq_io);
+                                              ENV ? env_friction : c.tab[LT_FRICTION], dk, &dq_io, &ddq_io)) {
+                // ENV: lane 0 solves its env with the env's own inertias and friction (the pack holds its EnvParams)
+                const auto dense = [&](auto... prm) {
+                    lanes_joint_constraints<T, G>(c.sm + L::oV, c.l, nq, c.body,
+                                                  c.l == 0 && ((rows >> (c.slot * G)) & ((1u << G) - 1u)) != 0u, tables, a.dt, q,
+                                                  &dq_io, &ddq_io, 0u, T(0), prm...);
+                };
+                if constexpr (ENV) dense(env_rows.env(e, nq));
+                else dense();
+            }
             dq = dq_io;
             ddq = ddq_io;
         }

@@ -8,10 +8,11 @@
 
 namespace b2 {
 
-// Fused Panda task, G lanes per env (G chosen from the number of joints).
+// Fused Panda task, G lanes per env (G chosen from the number of joints). env.inertia != nullptr: the physics reads every
+// env's own parameters (b2sim_enable_env_params).
 template <typename T>
 cudaError_t launch_task_panda_lanes(const ModelDev<T>* tables, const LaneTable<T>* lane_table, const PandaArgs<T>& a,
-                                    const int* parent, const int* jtype, cudaStream_t stream);
+                                    const int* parent, const int* jtype, cudaStream_t stream, const EnvRows<T>& env);
 
 // GazeboSimulator::run of a fixed-base tree on lanes (k_run_tree_lanes): PID / force / velocity-follower joints, the
 // computed-torque controller, resets, external link wrenches. v0 != nullptr: the model belongs to a coupled world; the

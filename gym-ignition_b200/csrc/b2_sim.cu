@@ -320,6 +320,24 @@ b2::RunCfg<T> build_run_cfg(b2sim* s, ModelState* ms, int paused, int iterations
     return cfg;
 }
 
+// The model's per-env parameter rows from env w0 on (all null while b2sim_enable_env_params is off). With rows, the impulse
+// path of the constraint stage needs undamped joints: the tables' stiffness decides in `topo`, every env's damping row in
+// the kernel.
+template <typename T>
+b2::EnvRows<T> env_rows(const ModelState* ms, int64_t w0, b2::TreeTopo* topo)
+{
+    b2::EnvRows<T> env;
+    if (!ms->env_params) return env;
+    const int nq = ms->model->t.nq;
+    env.inertia = (const T*)ms->buf[B2_BUF_BODY_INERTIA] + w0 * b2::kEnvInertiaCols * nq;
+    env.dyn = (const T*)ms->buf[B2_BUF_JOINT_DYNAMICS] + w0 * b2::kEnvJointCols * nq;
+    env.grav = (const T*)ms->buf[B2_BUF_GRAVITY] + w0 * 3;
+    topo->impulse_ok = 1;
+    for (int j = 0; j < nq; ++j)
+        if (ms->model->t.stiffness[j] != 0.0) topo->impulse_ok = 0;
+    return env;
+}
+
 // One thread per env: k_run_tree (scratch in shared memory, 64-thread blocks) or k_run_tree_local; ENV = the model's
 // per-env parameter rows are allocated.
 template <typename T, bool ENV>
@@ -344,16 +362,7 @@ int launch_run(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t co
     int rc = tree_topology(ms, &topo);
     if (rc != B2_OK) return rc;
     const b2::ModelDev<T>* tb = (const b2::ModelDev<T>*)ms->d_tables;
-    b2::EnvRows<T> env;
-    if (ms->env_params) {
-        env.inertia = (const T*)ms->buf[B2_BUF_BODY_INERTIA];
-        env.dyn = (const T*)ms->buf[B2_BUF_JOINT_DYNAMICS];
-        env.grav = (const T*)ms->buf[B2_BUF_GRAVITY];
-        // the impulse path needs undamped joints: the tables' stiffness decides here, every env's damping row in the kernel
-        topo.impulse_ok = 1;
-        for (int j = 0; j < nq; ++j)
-            if (ms->model->t.stiffness[j] != 0.0) topo.impulse_ok = 0;
-    }
+    const b2::EnvRows<T> env = env_rows<T>(ms, 0, &topo);
     if (nq >= 1 && nq <= b2::kMaxDofs && run_on_lanes(s, ms, 4)) {
         B2_CUDA(b2::launch_run_tree_lanes<T>(tb, (const b2::LaneTable<T>*)ms->d_lane_table, cfg, b, ms->model->t.parent,
                                              ms->model->t.jtype, s->stream, nullptr, 0, env));
@@ -498,6 +507,7 @@ int launch_panda(b2sim* s, ModelState* ms, const void* actions, int observe_only
     int rc = tree_topology(ms, &topo);
     if (rc != B2_OK) return rc;
     if (b2::panda_obs_size(nq) > b2::kPandaObs) return fail(B2_ERR_UNSUPPORTED, "the reach task supports up to 9 joints");
+    const b2::EnvRows<T> env = env_rows<T>(ms, w0, &topo);  // offset by the window like every per-env pointer above
     // Up to 32,768 envs an env's step is spread over G lanes of a warp (b2_lanes.cuh): measured on the B200 at 4,096 /
     // 16,384 / 65,536 / 262,144 envs, lanes 18 / 46 / 149 / 550 us against 46 / 51 / 137 / 480 us for one thread per env
     // (the lane kernel executes ~1.4x the thread-instruction slots per env, so it loses once the batch fills the
@@ -506,7 +516,7 @@ int launch_panda(b2sim* s, ModelState* ms, const void* actions, int observe_only
     const bool lanes = variant ? strcmp(variant, "thread") != 0 : wn <= 32768;
     if (lanes) {
         B2_CUDA(b2::launch_task_panda_lanes<T>((const b2::ModelDev<T>*)ms->d_tables, (const b2::LaneTable<T>*)ms->d_lane_table, a,
-                                               ms->model->t.parent, ms->model->t.jtype, s->stream));
+                                               ms->model->t.parent, ms->model->t.jtype, s->stream, env));
         ++s->launches;
         return B2_OK;
     }
@@ -516,7 +526,8 @@ int launch_panda(b2sim* s, ModelState* ms, const void* actions, int observe_only
     // registers) was measured on the B200 and does not help at any batch size (16 k envs: 53 / 58 / 68 / 93 us,
     // 1 M envs: 1.82 / 1.82 / 1.94 / 2.51 ms): the kernel is bound by the dependent fp64 chain at small batches and by
     // the L1 / L2 traffic of the per-thread scratch at large ones, not by occupancy.
-    b2::k_task_panda<T><<<grid, block, 0, s->stream>>>((const b2::ModelDev<T>*)ms->d_tables, a, topo);
+    if (ms->env_params) b2::k_task_panda<T, true><<<grid, block, 0, s->stream>>>((const b2::ModelDev<T>*)ms->d_tables, a, topo, env);
+    else b2::k_task_panda<T><<<grid, block, 0, s->stream>>>((const b2::ModelDev<T>*)ms->d_tables, a, topo, env);
     ++s->launches;
     B2_CUDA(cudaGetLastError());
     return B2_OK;
@@ -1914,8 +1925,9 @@ int b2sim_enable_env_params(b2sim* s, int model, int enable)
     const int nq = t.nq;
     if (nq == 0 || ms->kind == B2_KIND_FREE || ms->kind == B2_KIND_STATIC)
         return fail(B2_ERR_UNSUPPORTED, "model '%s' is not a fixed-base articulated model", ms->name.c_str());
-    if (ms->task != B2_TASK_NONE)
-        return fail(B2_ERR_UNSUPPORTED, "model '%s' has a fused task, whose kernels read the shared tables only", ms->name.c_str());
+    if (ms->task != B2_TASK_NONE && ms->task != B2_TASK_PANDA_REACH)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' has a pendulum / cart-pole task, whose kernels read the shared tables only",
+                    ms->name.c_str());
     for (auto& other : s->models)
         if (!other->removed && other->kind == B2_KIND_FREE)
             return fail(B2_ERR_UNSUPPORTED, "the world has free bodies: the coupled contact pipeline has no per-env parameters");
@@ -1985,9 +1997,9 @@ int b2sim_set_task(b2sim* s, int model, int task, uint64_t seed, uint64_t env_of
     if (!ms) return fail(B2_ERR_NOT_FOUND, "model %d not found", model);
     if (b2sim_task_nobs(task) == 0) return fail(B2_ERR_UNSUPPORTED, "unknown task %d", task);
     if (max_episode_steps <= 0 || max_episode_steps > 65535) return fail(B2_ERR_INVALID, "max_episode_steps out of range");
-    if (ms->env_params)
-        return fail(B2_ERR_UNSUPPORTED, "model '%s' has per-env parameters: the fused task kernels read the shared tables only",
-                    ms->name.c_str());
+    if (ms->env_params && task != B2_TASK_PANDA_REACH)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' has per-env parameters: the pendulum / cart-pole task kernels read the shared "
+                                        "tables only", ms->name.c_str());
     DeviceGuard guard__(s->device);
     const b2_model_tables& t = ms->model->t;
     if (task == B2_TASK_PANDA_REACH) {

@@ -100,7 +100,8 @@ enum {
     B2_BUF_BASE_ACCEL = 19,  /* [N, 6] B2_KIND_FREE: world linear acceleration of the base frame origin and angular acceleration
                               * over the last step, constraint impulses included (Link::world{Linear,Angular}Acceleration,
                               * Link.cpp:240-294; DART adds the velocity change of the constraint stage / dt to the accelerations) */
-    /* Per-env physical parameters (b2sim_enable_env_params), read by every unpaused b2sim_run of the model: */
+    /* Per-env physical parameters (b2sim_enable_env_params), read by every unpaused b2sim_run of the model and every
+     * step of its reach task: */
     B2_BUF_BODY_INERTIA = 20,   /* [N, 10*nq] per body j (child of joint j, welded links lumped in as in b2_model_tables):
                                  * mass, centre of mass xyz, inertia about it Ixx Ixy Ixz Iyy Iyz Izz, both in the body frame */
     B2_BUF_JOINT_DYNAMICS = 21, /* [N, 2*nq] per joint: viscous damping, Coulomb friction */
@@ -237,9 +238,14 @@ int b2sim_set_joint_friction(b2sim* s, int model, int joint, double coulomb, dou
  * (b2sim_kindyn, b2sim_centroidal, b2sim_momentum_jacobian, b2sim_update_kinematics, b2sim_link_motion:
  * KinDynComputations is built from the model file), and the per-link inertial data of the loader (b2model_tables:
  * link_mass, link_com, which a wrench applied at a link's centre of mass uses): the rows describe lumped bodies, not
- * links, so a per-link centre of mass cannot be derived from them. B2_ERR_UNSUPPORTED for a
- * free-floating or static model, a model with a fused task, and a world with free bodies (also from b2sim_run when a free
- * body is inserted later); b2sim_set_task refuses a model with per-env parameters. */
+ * links, so a per-link centre of mass cannot be derived from them. B2_TASK_PANDA_REACH reads the rows too, on every
+ * step that runs physics (b2sim_task_step, b2sim_task_rollout, steps replayed from a CUDA graph, b2sim_task_step_host);
+ * its observation is kinematic, so b2sim_task_observe and b2sim_task_reset_all do not read them. To draw new parameters
+ * per episode, write the rows of the envs whose B2_BUF_DONE is set (or all of them: the reach task only ends at its
+ * TimeLimit, so its envs finish together unless B2_BUF_ELAPSED is staggered) after that step and before the next: the
+ * terminal step ran with the old rows, the new episode runs with the new ones. B2_ERR_UNSUPPORTED for a free-floating
+ * or static model, a model with a pendulum / cart-pole task, and a world with free bodies (also from b2sim_run when a
+ * free body is inserted later); b2sim_set_task refuses a pendulum / cart-pole task on a model with per-env parameters. */
 int b2sim_enable_env_params(b2sim* s, int model, int enable);
 
 /* ---- custom controller: ComputedTorqueFixedBase run by ControllerRunner -------------------------------- */
@@ -286,7 +292,8 @@ int b2sim_buffer(b2sim* s, int model, int which, b2_buffer* out);
 
 /* ---- fused task path: the env.step hot path for all envs in one launch ----------------------------- */
 /* Attaches a task to a model: allocates obs/reward/done, stores the Philox seed and the global index of
- * env 0 (multi-GPU sharding: env e on this device is global env env_offset + e). */
+ * env 0 (multi-GPU sharding: env e on this device is global env env_offset + e). B2_TASK_PANDA_REACH may be attached to a
+ * model with per-env parameters (b2sim_enable_env_params, before or after); the pendulum / cart-pole tasks may not. */
 int b2sim_set_task(b2sim* s, int model, int task, uint64_t seed, uint64_t env_offset,
                    int max_episode_steps);
 /* Parameters of B2_TASK_PANDA_REACH (any pointer may be NULL, ee_link < 0 keeps the current one): reach goal in the

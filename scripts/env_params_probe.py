@@ -1,10 +1,16 @@
-"""Cost of per-env physical parameters (Simulator.enable_env_params) on GazeboSimulator::run of Pandas under position PIDs.
+"""Cost of per-env physical parameters (Simulator.enable_env_params) on GazeboSimulator::run of Pandas under position PIDs,
+and on the fused PandaReach step (BatchedTaskEnv.enable_env_params).
 
 Two simulators with the same Pandas, targets and gains (those of run_probe.py), one with its own random rows per env
 (masses x U(0.8, 1.2), inertias alike, damping U(0, 0.1), gravity tilted by up to ~3 degrees), the other on the shared
 tables. Blocks of `runs` b2sim_run calls alternate between the two in one process and are timed with CUDA events; the
 median of 5 blocks per variant is reported. The batch size selects the kernel: 4,096 and 16,384 envs run on lanes
 (k_run_tree_lanes), 20,001 on k_run_tree and 65,536 on k_run_tree_local.
+
+The reach step is timed the same way (blocks of `runs` env.step calls): 4,096 and 16,384 envs on k_task_panda_lanes with
+the fingers held mid-range, 16,384 envs with the fingers driven into their lower limits (limit rows on every step) with
+damped rows (the dense constraint solve) and with undamped ones (the lane-parallel stage), 65,536 envs on k_task_panda. Last, the cost of redrawing every row of 16,384 envs once (the per-episode pattern: new
+rows after the step that reports done) with torch, against the step it precedes.
 
     python scripts/env_params_probe.py [runs_per_block]
 """
@@ -56,6 +62,87 @@ def panda_sim(n, env_params, seed):
     return sim
 
 
+def draw_rows(views, nominal, gen, damped=True):
+    """New random rows from the nominal ones, written in place (what a caller does at its resets)."""
+    import torch
+    inertia, dyn, g = views
+    n = inertia.shape[0]
+    f64 = dict(device="cuda", dtype=torch.float64)
+    s = 0.8 + 0.4 * torch.rand(n, 9, 1, generator=gen, **f64)
+    inertia[:, :, 0:1] = nominal[:, :, 0:1] * s
+    inertia[:, :, 1:4] = nominal[:, :, 1:4]
+    inertia[:, :, 4:] = nominal[:, :, 4:] * s
+    dyn[:, :, 0] = 0.1 * torch.rand(n, 9, generator=gen, **f64) if damped else 0.0
+    g[:, :2] = 0.5 * (torch.rand(n, 2, generator=gen, **f64) - 0.5)
+
+
+def reach_env(n, env_params, fingers, seed, damped=True):
+    import torch
+    import b2sim
+    from b2sim.batched import PANDA_Q0
+    env = b2sim.BatchedTaskEnv("PandaReach-Gazebo-v0", n)
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(seed)
+    f64 = dict(device="cuda", dtype=torch.float64)
+    tg = (torch.tensor(PANDA_Q0, **f64) + 0.1 * torch.sin(torch.rand(n, 1, generator=gen, **f64) * 6.28)).contiguous()
+    tg[:, 7:] = 0.02 if fingers == "mid" else -0.05
+    if env_params:
+        views = env.enable_env_params()
+        draw_rows(views, views[0].clone(), gen, damped)
+    return env, tg
+
+
+def timed(fn, runs):
+    """Microseconds per call of fn over `runs` calls, CUDA events."""
+    import torch
+    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    a.record()
+    for _ in range(runs):
+        fn()
+    b.record()
+    torch.cuda.synchronize()
+    return a.elapsed_time(b) / runs * 1e3
+
+
+def reach(runs):
+    import numpy as np
+    import torch
+    # damped=False: the rows keep the Panda's zero joint damping, so limit rows stay on the lane-parallel constraint stage
+    for n, kernel, fingers, damped in ((4096, "k_task_panda_lanes", "mid", True), (16384, "k_task_panda_lanes", "mid", True),
+                                       (16384, "k_task_panda_lanes", "limits", True),
+                                       (16384, "k_task_panda_lanes", "limits", False), (65536, "k_task_panda", "mid", True)):
+        envs = {"off": reach_env(n, False, fingers, 3), "on": reach_env(n, True, fingers, 3, damped)}
+        for env, tg in envs.values():  # warm-up: module loads, clocks
+            for _ in range(200):
+                env.step(tg)
+        torch.cuda.synchronize()
+        times = {k: [] for k in envs}
+        for block in range(5):
+            for name, (env, tg) in envs.items():
+                times[name].append(timed(lambda: env.step(tg), runs))
+        off, on = (float(np.median(times[k])) for k in ("off", "on"))
+        spread = {k: (min(v), max(v)) for k, v in times.items()}
+        print(f"reach n={n:6d} {kernel:18s} fingers {fingers:6s} {'damped' if damped else 'undamped':8s} off {off:7.2f} us/step (blocks {spread['off'][0]:.2f}-"
+              f"{spread['off'][1]:.2f})  on {on:7.2f} us/step (blocks {spread['on'][0]:.2f}-{spread['on'][1]:.2f})  "
+              f"on/off {on / off:.3f}", flush=True)
+        for env, _ in envs.values():
+            env.close()
+    n = 16384
+    env, tg = reach_env(n, False, "mid", 3)
+    views = env.enable_env_params()
+    nominal = views[0].clone()
+    gen = torch.Generator(device="cuda")
+    gen.manual_seed(5)
+    for _ in range(200):
+        draw_rows(views, nominal, gen)
+        env.step(tg)
+    torch.cuda.synchronize()
+    draw = float(np.median([timed(lambda: draw_rows(views, nominal, gen), runs) for _ in range(5)]))
+    step = float(np.median([timed(lambda: env.step(tg), runs) for _ in range(5)]))
+    print(f"reach n={n:6d} redraw of every row {draw:7.2f} us  (one step {step:7.2f} us)", flush=True)
+    env.close()
+
+
 def main():
     sys.path.insert(0, ROOT)
     import __graft_entry__
@@ -86,6 +173,7 @@ def main():
               f"on {on:7.2f} us/run (blocks {spread['on'][0]:.2f}-{spread['on'][1]:.2f})  on/off {on / off:.3f}", flush=True)
         for sim in sims.values():
             sim.close()
+    reach(runs)
 
 
 if __name__ == "__main__":
