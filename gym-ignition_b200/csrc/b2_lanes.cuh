@@ -141,16 +141,28 @@ struct LaneCtx {
     unsigned anc;   // bit j: body j is l or one of its ancestors
 };
 
-// Stages the packed model constants into shared memory (all threads of the block; ends with the block barrier).
-template <typename T, int G>
-__device__ __forceinline__ void lanes_stage_table(const LaneTable<T>* __restrict__ lane_table, T* table)
+struct NoStaging {
+    __device__ void operator()() const {}
+};
+
+// Stages the packed model constants into shared memory (all threads of the block), then waits for the previous grid on
+// the stream. `also`: further staging by the block's threads, published with the table by the same block barrier.
+// Programmatic dependent launch (the launcher sets the stream-serialization attribute): the next step's blocks are
+// scheduled while this grid drains and stage the model constants (written at set-up, never by a step) before they wait
+// for the previous step's state. Without the attribute both griddepcontrol instructions are no-ops.
+template <typename T, int G, typename Also = NoStaging>
+__device__ __forceinline__ void lanes_stage_table_then_wait(const LaneTable<T>* __restrict__ lane_table, T* table,
+                                                            Also also = Also())
 {
+    asm volatile("griddepcontrol.launch_dependents;");
+    also();
     using V = typename Pair<T>::type;
     const V* src = reinterpret_cast<const V*>(lane_table);
     V* dst = reinterpret_cast<V*>(table);
     for (int k = threadIdx.x; k < G * LT_SIZE / 2; k += blockDim.x)
         dst[(k / (LT_SIZE / 2)) * (LaneLayout<G>::REC / 2) + (k % (LT_SIZE / 2))] = __ldg(src + k);
     __syncthreads();
+    asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 // ---- phase A: sine / cosine and joint placement of the lane's joint -> P1[l][12] -------------------------------------
@@ -255,6 +267,24 @@ __device__ __forceinline__ void lanes_load_placement(const LaneCtx<T, G>& c, T* 
     ld2(rp + 8, R[6], R[7]); ld2(rp + 10, R[8], p.z);
 }
 
+// World axis of the lane's joint, R axis, from its body's world orientation R.
+template <typename T, int G>
+__device__ __forceinline__ V3<T> lanes_joint_axis(const LaneCtx<T, G>& c, const T* R)
+{
+    const T* t = c.tab;
+    return v3(R[0] * t[LT_AXIS] + R[1] * t[LT_AXIS + 1] + R[2] * t[LT_AXIS + 2],
+              R[3] * t[LT_AXIS] + R[4] * t[LT_AXIS + 1] + R[5] * t[LT_AXIS + 2],
+              R[6] * t[LT_AXIS] + R[7] * t[LT_AXIS + 1] + R[8] * t[LT_AXIS + 2]);
+}
+
+// A point given at x in a body's frame, placed from the body's world placement (R, p): p + R x.
+template <typename T>
+__device__ __forceinline__ V3<T> place_point(const T* R, const V3<T>& p, const T* x)
+{
+    return v3(p.x + R[0] * x[0] + R[1] * x[1] + R[2] * x[2], p.y + R[3] * x[0] + R[4] * x[1] + R[5] * x[2],
+              p.z + R[6] * x[0] + R[7] * x[1] + R[8] * x[2]);
+}
+
 // Sum over the tree towards the leaves (lane = component): x_i += x_parent(i), roots start from `root`.
 // `mine` points at the lane's component of body 0; PER scalars per body.
 template <typename T, int G, int PER>
@@ -349,8 +379,7 @@ __device__ __forceinline__ T lanes_forward_dynamics(const LaneCtx<T, G>& c, cons
         } else {
             S[0] = S[1] = S[2] = T(0); S[3] = aw.x; S[4] = aw.y; S[5] = aw.z;
         }
-        const V3<T> cw = v3(p.x + R[0] * cm[0] + R[1] * cm[1] + R[2] * cm[2], p.y + R[3] * cm[0] + R[4] * cm[1] + R[5] * cm[2],
-                            p.z + R[6] * cm[0] + R[7] * cm[1] + R[8] * cm[2]);
+        const V3<T> cw = place_point(R, p, cm);
         const Sym3<T> Iw = rot_sym(M3<T>{{R[0], R[1], R[2], R[3], R[4], R[5], R[6], R[7], R[8]}},
                                    Sym3<T>{ic[0], ic[1], ic[2], ic[3], ic[4], ic[5]});
         const T cc = dot(cw, cw);
@@ -530,8 +559,7 @@ __device__ __forceinline__ T lanes_inverse_dynamics(const LaneCtx<T, G>& c, cons
         } else {
             S[0] = S[1] = S[2] = T(0); S[3] = aw.x; S[4] = aw.y; S[5] = aw.z;
         }
-        const V3<T> cw = v3(p.x + R[0] * cm[0] + R[1] * cm[1] + R[2] * cm[2], p.y + R[3] * cm[0] + R[4] * cm[1] + R[5] * cm[2],
-                            p.z + R[6] * cm[0] + R[7] * cm[1] + R[8] * cm[2]);
+        const V3<T> cw = place_point(R, p, cm);
         const Sym3<T> Iw = rot_sym(M3<T>{{R[0], R[1], R[2], R[3], R[4], R[5], R[6], R[7], R[8]}},
                                    Sym3<T>{ic[0], ic[1], ic[2], ic[3], ic[4], ic[5]});
         const T cc = dot(cw, cw);
@@ -802,14 +830,10 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
         env.g = env_rows.grav + 3 * e;
     }
 
-    // Programmatic dependent launch (the launcher sets the stream-serialization attribute): the next step's blocks are
-    // scheduled while this grid drains and stage the model constants (written at set-up, never by a step) before they
-    // wait for the previous step's state. Without the attribute both instructions are no-ops.
-    asm volatile("griddepcontrol.launch_dependents;");
-    if (threadIdx.x < 9) table[L::table + threadIdx.x] = m.link_R[a.ee_link][threadIdx.x];
-    else if (threadIdx.x < 12) table[L::table + threadIdx.x] = m.link_p[a.ee_link][threadIdx.x - 9];
-    lanes_stage_table<T, G>(lane_table, table);
-    asm volatile("griddepcontrol.wait;" ::: "memory");
+    lanes_stage_table_then_wait<T, G>(lane_table, table, [&] {
+        if (threadIdx.x < 9) table[L::table + threadIdx.x] = m.link_R[a.ee_link][threadIdx.x];
+        else if (threadIdx.x < 12) table[L::table + threadIdx.x] = m.link_p[a.ee_link][threadIdx.x - 9];
+    });
     T q = T(0), dq = T(0), target = T(0), st[3] = {T(0), T(0), T(0)};
     unsigned el = 0;
     if (c.live && c.l == 0) el = a.elapsed[e];  // needed at the very end: in flight with the state loads
@@ -878,18 +902,14 @@ __global__ void __launch_bounds__(128, 4) k_task_panda_lanes(const ModelDev<T>* 
         T R[9];
         if (chain_lane) {
             lanes_load_placement(c, R, po);
-            const T* t = c.tab;
-            aw = v3(R[0] * t[LT_AXIS] + R[1] * t[LT_AXIS + 1] + R[2] * t[LT_AXIS + 2],
-                    R[3] * t[LT_AXIS] + R[4] * t[LT_AXIS + 1] + R[5] * t[LT_AXIS + 2],
-                    R[6] * t[LT_AXIS] + R[7] * t[LT_AXIS + 1] + R[8] * t[LT_AXIS + 2]);
+            aw = lanes_joint_axis(c, R);
         } else {
 #pragma unroll
             for (int k = 0; k < 9; ++k) R[k] = m.baseR[k];
         }
         if (c.l == ee_lane) {
             const T* ee = table + L::table;  // link_R (9), link_p (3)
-            pe = v3(po.x + R[0] * ee[9] + R[1] * ee[10] + R[2] * ee[11], po.y + R[3] * ee[9] + R[4] * ee[10] + R[5] * ee[11],
-                    po.z + R[6] * ee[9] + R[7] * ee[10] + R[8] * ee[11]);
+            pe = place_point(R, po, ee + 9);
             T E[9];
 #pragma unroll
             for (int r = 0; r < 3; ++r)
@@ -1048,9 +1068,7 @@ __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __
         env.joint = env_rows.dyn + (e * nq + jl) * kEnvJointCols;
         env.g = env_rows.grav + 3 * e;
     }
-    asm volatile("griddepcontrol.launch_dependents;");  // see k_task_panda_lanes
-    lanes_stage_table<T, G>(lane_table, table);
-    asm volatile("griddepcontrol.wait;" ::: "memory");
+    lanes_stage_table_then_wait<T, G>(lane_table, table);
     T q = T(0), dq = T(0), fc = T(0), ref = T(0), vel_t = T(0), st[3] = {T(0), T(0), T(0)};
     T ct_pos = T(0), ct_vel = T(0), ct_acc = T(0), ct_tau = T(0);
     const bool ct = CT && !cfg.paused && cfg.ct_active;
@@ -1122,15 +1140,8 @@ __global__ void __launch_bounds__(128, 4) k_run_tree_lanes(const ModelDev<T>* __
                 if (c.body) {
                     T R[9];
                     lanes_load_placement(c, R, po);
-                    const T* t = c.tab;
-                    aw = v3(R[0] * t[LT_AXIS] + R[1] * t[LT_AXIS + 1] + R[2] * t[LT_AXIS + 2],
-                            R[3] * t[LT_AXIS] + R[4] * t[LT_AXIS + 1] + R[5] * t[LT_AXIS + 2],
-                            R[6] * t[LT_AXIS] + R[7] * t[LT_AXIS + 1] + R[8] * t[LT_AXIS + 2]);
-                    if (c.l == wb) {
-                        const T* lp = m.link_p[link];
-                        pl = v3(po.x + R[0] * lp[0] + R[1] * lp[1] + R[2] * lp[2], po.y + R[3] * lp[0] + R[4] * lp[1] + R[5] * lp[2],
-                                po.z + R[6] * lp[0] + R[7] * lp[1] + R[8] * lp[2]);
-                    }
+                    aw = lanes_joint_axis(c, R);
+                    if (c.l == wb) pl = place_point(R, po, m.link_p[link]);
                 }
                 const int src = c.slot * G + wb;
                 pl.x = __shfl_sync(0xffffffffu, pl.x, src);

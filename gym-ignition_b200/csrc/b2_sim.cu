@@ -279,6 +279,14 @@ bool run_on_lanes(const b2sim* s, const ModelState* ms, int min_nq)
     return s->n <= 16384 && ms->model->t.nq >= min_nq;
 }
 
+// A joint's PID gains in the kernels' order: p, i, d, i_max, i_min, cmd_max, cmd_min, cmd_offset.
+template <typename T>
+void pack_pid(const b2_pid& p, T* gains)
+{
+    const double g[8] = {p.p, p.i, p.d, p.i_max, p.i_min, p.cmd_max, p.cmd_min, p.cmd_offset};
+    for (int k = 0; k < 8; ++k) gains[k] = (T)g[k];
+}
+
 template <typename T>
 b2::RunCfg<T> build_run_cfg(b2sim* s, ModelState* ms, int paused, int iterations, uint32_t compute_bits, uint32_t ct_bits,
                             const int* wrench_iters)
@@ -296,9 +304,7 @@ b2::RunCfg<T> build_run_cfg(b2sim* s, ModelState* ms, int paused, int iterations
         cfg.mode[j] = (uint8_t)ms->mode[j];
         cfg.has_force_cmd[j] = ms->has_force_cmd[j];
         cfg.has_vel_cmd[j] = ms->has_vel_cmd[j];
-        const b2_pid& p = ms->pid[j];
-        const double g[8] = {p.p, p.i, p.d, p.i_max, p.i_min, p.cmd_max, p.cmd_min, p.cmd_offset};
-        for (int k = 0; k < 8; ++k) cfg.pid[j][k] = (T)g[k];
+        pack_pid(ms->pid[j], cfg.pid[j]);
         cfg.ct_kp[j] = (T)ms->ct_kp[j];
         cfg.ct_kd[j] = (T)ms->ct_kd[j];
     }
@@ -455,17 +461,7 @@ int launch_task(b2sim* s, ModelState* ms, const void* actions, int traj_steps = 
     } else {
         // eager steps follow each other on the stream: programmatic dependent launch hides the launch-to-launch gap
         // (k_task_chain waits with griddepcontrol.wait before it touches memory)
-        cudaLaunchConfig_t lc = {};
-        lc.gridDim = dim3((unsigned)grid);
-        lc.blockDim = dim3((unsigned)block);
-        lc.dynamicSmemBytes = 0;
-        lc.stream = s->stream;
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = 1;
-        lc.attrs = attr;
-        lc.numAttrs = 1;
-        B2_CUDA(cudaLaunchKernelEx(&lc, b2::k_task_chain<TASK, T, false>, a));
+        B2_CUDA(b2::launch_pdl(b2::k_task_chain<TASK, T, false>, grid, block, 0, s->stream, true, a));
     }
     ++s->launches;
     B2_CUDA(cudaGetLastError());
@@ -499,9 +495,7 @@ int launch_panda(b2sim* s, ModelState* ms, const void* actions, int observe_only
     for (int k = 0; k < 3; ++k) a.goal[k] = (T)ms->task_goal[k];
     for (int j = 0; j < nq; ++j) {
         a.q0[j] = (T)ms->task_q0[j];
-        const b2_pid& p = ms->pid[j];
-        const double g[8] = {p.p, p.i, p.d, p.i_max, p.i_min, p.cmd_max, p.cmd_min, p.cmd_offset};
-        for (int k = 0; k < 8; ++k) a.pid[j][k] = (T)g[k];
+        pack_pid(ms->pid[j], a.pid[j]);
     }
     b2::TreeTopo topo;
     int rc = tree_topology(ms, &topo);
