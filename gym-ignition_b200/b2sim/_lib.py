@@ -117,6 +117,8 @@ SYMBOLS = {
     "b2sim_set_max_generalized_force": (_i, [_vp, _i, _i, _d]),
     "b2sim_set_joint_friction": (_i, [_vp, _i, _i, _d, _d]),
     "b2sim_enable_env_params": (_i, [_vp, _i, _i]),
+    "b2sim_enable_free_body_params": (_i, [_vp, _i, _i, C.POINTER(Buffer)]),
+    "b2sim_enable_shape_friction": (_i, [_vp, _i, _i, C.POINTER(Buffer)]),
     "b2sim_set_computed_torque": (_i, [_vp, _i, _dp, _dp, _dp]),
     "b2sim_apply_link_wrench": (_i, [_vp, _i, _i64, _i, _dp, _d]),
     "b2sim_get_joint": (_i, [_vp, _i, _i, _i64, _i, _dp]),

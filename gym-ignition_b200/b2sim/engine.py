@@ -262,6 +262,31 @@ class Simulator:
         dynamics = self.tensor(model, _lib.BUF_JOINT_DYNAMICS).view(self.num_envs, nq, 2)
         return inertia, dynamics, self.tensor(model, _lib.BUF_GRAVITY)
 
+    def _enable_rows(self, fn, model, enable):
+        b = _lib.Buffer()
+        check(fn(self.handle, model, 1 if enable else 0, C.byref(b)))
+        if not enable:
+            return None
+        return DeviceArray(self, b.ptr, b.rows, b.cols, b.dtype).torch(self.device)
+
+    def enable_free_body_params(self, model, enable: bool = True):
+        """Gives every env its own mass, centre of mass and inertia of the free-floating `model`, starting from the loader's
+        values. Returns a zero-copy view [N, 10]: mass, centre of mass xyz in the root-link frame, inertia about it xx xy xz
+        yy yz zz in root-link axes; the caller writes it between runs, and every unpaused run reads it. Enabling again
+        returns the same rows unchanged. enable=False returns the body to its shared values and returns None. The view
+        does not own its memory: disabling, removing the model or closing the simulator frees it, and a view kept from
+        before must not be used afterwards (enable again for a new view). Gravity, the link-level inertial data (ModelInfo
+        tables) and the dynamics of an articulated model in the same world stay nominal."""
+        return self._enable_rows(self.lib.b2sim_enable_free_body_params, model, enable)
+
+    def enable_shape_friction(self, model, enable: bool = True):
+        """Gives every env its own Coulomb friction coefficient of each collision shape of `model` (free, static or
+        articulated), starting from the loader's values. Returns a zero-copy view [N, nshapes] (column k: shape k of the
+        ModelInfo tables); a contact uses the smaller of its two shapes' values in its env. Same lifetime as
+        enable_free_body_params: enable=False frees the rows and returns None, and a view kept from before must not be
+        used after disabling, removing the model or closing the simulator."""
+        return self._enable_rows(self.lib.b2sim_enable_shape_friction, model, enable)
+
     # ---- fused task path ----
     def set_task(self, model, task, seed=0, env_offset=0, max_episode_steps=5000):
         self.run_count = getattr(self, "run_count", 0) + 1  # the per-object view drops what it cached

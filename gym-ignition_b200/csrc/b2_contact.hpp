@@ -64,6 +64,79 @@ struct alignas(16) WorldDev {
     long long ext_env[kMaxFree];
 };
 
+// Where the inertial data of the free bodies and the friction coefficients of the collision shapes come from (the world's
+// counterpart of NominalParams / EnvParams, b2_rbd.hpp). WorldNominal: the shared world description.
+template <typename T>
+struct WorldNominal {
+    B2_HD T mass(const FreeBodyDev<T>& fb, int) const { return fb.mass; }
+    B2_HD V3<T> com(const FreeBodyDev<T>& fb, int) const { return ld3(fb.com); }
+    B2_HD M3<T> Ic(const FreeBodyDev<T>& fb, int) const { return ld9(fb.Ic); }
+    B2_HD M3<T> Ic_inv(const FreeBodyDev<T>& fb, int) const { return ld9(fb.Ic_inv); }
+    // shape s of free body i, static shape k, shape r of the articulated model
+    B2_HD T body_mu(const ShapeDev<T>& sh, int, int) const { return sh.mu; }
+    B2_HD T stat_mu(const ShapeDev<T>& sh, int) const { return sh.mu; }
+    B2_HD T robot_mu(const ShapeDev<T>& sh, int) const { return sh.mu; }
+};
+
+// Per-env rows of a world (b2sim_enable_free_body_params / b2sim_enable_shape_friction), resolved per slot by the host on
+// every launch: env 0's row of free body i ([N][kFreeBodyCols]: mass, centre of mass xyz, inertia about it xx xy xz yy yz
+// zz, root-link frame), and env 0's friction coefficient of every shape slot in its model's [N][nshapes] rows with that
+// row's stride. Null: the slot reads the shared world description.
+constexpr int kFreeBodyCols = 10;
+
+template <typename T>
+struct WorldRows {
+    const T* body[kMaxFree];
+    const T* body_mu[kMaxFree][kMaxBodyShapes];
+    const T* stat_mu[kMaxStaticShapes];
+    const T* robot_mu[kMaxRobotShapes];
+    int body_mu_stride[kMaxFree];
+    int stat_mu_stride[kMaxStaticShapes];
+    int robot_mu_stride;
+};
+
+// WorldEnv: env e's rows wherever the slot has them, the shared value otherwise.
+template <typename T>
+struct WorldEnv {
+    const WorldRows<T>& rows;
+    long long e;
+    B2_HD const T* row(int i) const { return rows.body[i] + e * kFreeBodyCols; }
+    B2_HD T mass(const FreeBodyDev<T>& fb, int i) const { return rows.body[i] ? row(i)[0] : fb.mass; }
+    B2_HD V3<T> com(const FreeBodyDev<T>& fb, int i) const { return rows.body[i] ? ld3(row(i) + 1) : ld3(fb.com); }
+    B2_HD M3<T> Ic(const FreeBodyDev<T>& fb, int i) const
+    {
+        if (!rows.body[i]) return ld9(fb.Ic);
+        const T* r = row(i);
+        return M3<T>{{r[4], r[5], r[6], r[5], r[7], r[8], r[6], r[8], r[9]}};
+    }
+    // adjugate over determinant, as upload_world inverts the shared inertia on the host (b2_sim.cu)
+    B2_HD M3<T> Ic_inv(const FreeBodyDev<T>& fb, int i) const
+    {
+        if (!rows.body[i]) return ld9(fb.Ic_inv);
+        const M3<T> M = Ic(fb, i);
+        const T* I = M.m;
+        const T det = I[0] * (I[4] * I[8] - I[5] * I[7]) - I[1] * (I[3] * I[8] - I[5] * I[6]) + I[2] * (I[3] * I[7] - I[4] * I[6]);
+        return M3<T>{{(I[4] * I[8] - I[5] * I[7]) / det, (I[2] * I[7] - I[1] * I[8]) / det, (I[1] * I[5] - I[2] * I[4]) / det,
+                      (I[5] * I[6] - I[3] * I[8]) / det, (I[0] * I[8] - I[2] * I[6]) / det, (I[2] * I[3] - I[0] * I[5]) / det,
+                      (I[3] * I[7] - I[4] * I[6]) / det, (I[1] * I[6] - I[0] * I[7]) / det, (I[0] * I[4] - I[1] * I[3]) / det}};
+    }
+    B2_HD T body_mu(const ShapeDev<T>& sh, int i, int s) const
+    {
+        const T* p = rows.body_mu[i][s];
+        return p ? p[e * rows.body_mu_stride[i]] : sh.mu;
+    }
+    B2_HD T stat_mu(const ShapeDev<T>& sh, int k) const
+    {
+        const T* p = rows.stat_mu[k];
+        return p ? p[e * rows.stat_mu_stride[k]] : sh.mu;
+    }
+    B2_HD T robot_mu(const ShapeDev<T>& sh, int r) const
+    {
+        const T* p = rows.robot_mu[r];
+        return p ? p[e * rows.robot_mu_stride] : sh.mu;
+    }
+};
+
 template <typename T> B2_HD M3<T> quat_to_rot(const T* q)
 {
     const T w = q[0], x = q[1], y = q[2], z = q[3];
@@ -251,8 +324,9 @@ B2_HD void apply_impulse(BodyWork<T>* bw, RobotWork<T>* rw, const Contact<T>& c,
 }
 
 // Loads the free bodies of one world and applies the unconstrained velocity update (gravity, gyroscopic torque).
-template <typename T>
-B2_HD void bodies_begin(const WorldDev<T>& W, const T* X, BodyWork<T>* bw, long long env = -1)
+// P: where the inertial data and friction coefficients come from (WorldNominal / WorldEnv), here and below.
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void bodies_begin(const WorldDev<T>& W, const T* X, BodyWork<T>* bw, long long env = -1, const P& prm = P())
 {
     const T dt = W.dt;
     const V3<T> g = ld3(W.g);
@@ -261,13 +335,13 @@ B2_HD void bodies_begin(const WorldDev<T>& W, const T* X, BodyWork<T>* bw, long 
         const T* x = X + 13 * i;
         BodyWork<T>& b = bw[i];
         b.R = quat_to_rot(x + 3);
-        const V3<T> rc = mul(b.R, ld3(fb.com));
+        const V3<T> rc = mul(b.R, prm.com(fb, i));
         b.xc = ld3(x) + rc;
         b.w = ld3(x + 10);
         b.vc = ld3(x + 7) + cross(b.w, rc);
-        b.inv_mass = T(1) / fb.mass;
-        b.Iinv = mulBt(mul(b.R, ld9(fb.Ic_inv)), b.R);
-        const M3<T> Iw = mulBt(mul(b.R, ld9(fb.Ic)), b.R);
+        b.inv_mass = T(1) / prm.mass(fb, i);
+        b.Iinv = mulBt(mul(b.R, prm.Ic_inv(fb, i)), b.R);
+        const M3<T> Iw = mulBt(mul(b.R, prm.Ic(fb, i)), b.R);
         b.vc = b.vc + dt * g;
         b.w = b.w - dt * mul(b.Iinv, cross(b.w, mul(Iw, b.w)));
         if (W.ext_env[i] == -1 || (W.ext_env[i] >= 0 && W.ext_env[i] == env)) {
@@ -279,18 +353,18 @@ B2_HD void bodies_begin(const WorldDev<T>& W, const T* X, BodyWork<T>* bw, long 
 }
 
 // Contact points of the free bodies against static shapes and against each other.
-template <typename T>
-B2_HD void free_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, Contact<T>* cs, int& nc)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void free_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, Contact<T>* cs, int& nc, const P& prm = P())
 {
     for (int i = 0; i < W.nfree; ++i) {
         const FreeBodyDev<T>& fb = W.body[i];
         for (int s = 0; s < fb.nshapes; ++s) {
             const ShapeDev<T>& sa = fb.shape[s];
             const M3<T> Ra = mul(bw[i].R, ld9(sa.R));
-            const V3<T> pa = bw[i].xc + mul(bw[i].R, ld3(sa.p) - ld3(fb.com));
+            const V3<T> pa = bw[i].xc + mul(bw[i].R, ld3(sa.p) - prm.com(fb, i));
             for (int k = 0; k < W.nstatic; ++k) {
                 const ShapeDev<T>& sb = W.stat[k];
-                const T mu = sa.mu < sb.mu ? sa.mu : sb.mu;
+                const T mu = prm.body_mu(sa, i, s) < prm.stat_mu(sb, k) ? prm.body_mu(sa, i, s) : prm.stat_mu(sb, k);
                 if (sa.type == kShapeBox) box_vs_shape(cs, nc, i, s, -1 - k, Ra, pa, sa.size, sb, ld9(sb.R), ld3(sb.p), mu);
                 else if (sa.type == kShapeSphere) sphere_vs_shape(cs, nc, i, s, -1 - k, pa, sa.size[0], sb, ld9(sb.R), ld3(sb.p), mu);
             }
@@ -301,8 +375,8 @@ B2_HD void free_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, Contact<T>
                     const ShapeDev<T>& sb = fj.shape[u];
                     if (sb.type != kShapeBox) continue;
                     const M3<T> Rb = mul(bw[j].R, ld9(sb.R));
-                    const V3<T> pb = bw[j].xc + mul(bw[j].R, ld3(sb.p) - ld3(fj.com));
-                    const T mu = sa.mu < sb.mu ? sa.mu : sb.mu;
+                    const V3<T> pb = bw[j].xc + mul(bw[j].R, ld3(sb.p) - prm.com(fj, j));
+                    const T mu = prm.body_mu(sa, i, s) < prm.body_mu(sb, j, u) ? prm.body_mu(sa, i, s) : prm.body_mu(sb, j, u);
                     if (sa.type == kShapeBox) box_vs_shape(cs, nc, i, s, j, Ra, pa, sa.size, sb, Rb, pb, mu);
                     else if (sa.type == kShapeSphere) sphere_vs_shape(cs, nc, i, s, j, pa, sa.size[0], sb, Rb, pb, mu);
                 }
@@ -314,8 +388,9 @@ B2_HD void free_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, Contact<T>
 // Contact points of the articulated model's link shapes against static shapes and free bodies (both directions
 // for box pairs: corners of either box against the reference face of the other). Self-collisions are disabled by
 // the reference on insertion (cpp/scenario/gazebo/src/Model.cpp:175-178).
-template <typename T>
-B2_HD void robot_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, const RobotWork<T>& rw, Contact<T>* cs, int& nc)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void robot_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, const RobotWork<T>& rw, Contact<T>* cs, int& nc,
+                          const P& prm = P())
 {
     for (int r = 0; r < W.nrobot; ++r) {
         const ShapeDev<T>& sr = W.rshape[r];
@@ -325,7 +400,7 @@ B2_HD void robot_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, const Rob
         const int side = kRobotSide - r;
         for (int k = 0; k < W.nstatic; ++k) {
             const ShapeDev<T>& sb = W.stat[k];
-            const T mu = sr.mu < sb.mu ? sr.mu : sb.mu;
+            const T mu = prm.robot_mu(sr, r) < prm.stat_mu(sb, k) ? prm.robot_mu(sr, r) : prm.stat_mu(sb, k);
             if (sr.type == kShapeBox) box_vs_shape(cs, nc, side, r, -1 - k, Rr, pr, sr.size, sb, ld9(sb.R), ld3(sb.p), mu);
             else if (sr.type == kShapeSphere) sphere_vs_shape(cs, nc, side, r, -1 - k, pr, sr.size[0], sb, ld9(sb.R), ld3(sb.p), mu);
         }
@@ -334,8 +409,8 @@ B2_HD void robot_contacts(const WorldDev<T>& W, const BodyWork<T>* bw, const Rob
             for (int u = 0; u < fj.nshapes; ++u) {
                 const ShapeDev<T>& sb = fj.shape[u];
                 const M3<T> Rb = mul(bw[j].R, ld9(sb.R));
-                const V3<T> pb = bw[j].xc + mul(bw[j].R, ld3(sb.p) - ld3(fj.com));
-                const T mu = sr.mu < sb.mu ? sr.mu : sb.mu;
+                const V3<T> pb = bw[j].xc + mul(bw[j].R, ld3(sb.p) - prm.com(fj, j));
+                const T mu = prm.robot_mu(sr, r) < prm.body_mu(sb, j, u) ? prm.robot_mu(sr, r) : prm.body_mu(sb, j, u);
                 if (sb.type == kShapeBox) {  // robot shape against the free box
                     if (sr.type == kShapeBox) box_vs_shape(cs, nc, side, r, j, Rr, pr, sr.size, sb, Rb, pb, mu);
                     else if (sr.type == kShapeSphere) sphere_vs_shape(cs, nc, side, r, j, pr, sr.size[0], sb, Rb, pb, mu);
@@ -453,8 +528,8 @@ B2_HD void joint_row_sweep(RobotWork<T>& rw)
 }
 
 // Integrates the poses of the free bodies (rotation by the exponential map) and stores them back.
-template <typename T>
-B2_HD void body_end(const WorldDev<T>& W, int i, T* x /* the body's 13 state values */, BodyWork<T>& b)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void body_end(const WorldDev<T>& W, int i, T* x /* the body's 13 state values */, BodyWork<T>& b, const P& prm = P())
 {
     const T dt = W.dt;
     {
@@ -475,7 +550,7 @@ B2_HD void body_end(const WorldDev<T>& W, int i, T* x /* the body's 13 state val
         }
         b.xc = b.xc + dt * b.vc;
         const M3<T> Rn = quat_to_rot(q);
-        const V3<T> rc = mul(Rn, ld3(fb.com));
+        const V3<T> rc = mul(Rn, prm.com(fb, i));
         const V3<T> p = b.xc - rc, v = b.vc - cross(b.w, rc);
         x[0] = p.x; x[1] = p.y; x[2] = p.z;
         x[3] = q[0]; x[4] = q[1]; x[5] = q[2]; x[6] = q[3];
@@ -483,26 +558,26 @@ B2_HD void body_end(const WorldDev<T>& W, int i, T* x /* the body's 13 state val
         x[10] = b.w.x; x[11] = b.w.y; x[12] = b.w.z;
     }
 }
-template <typename T>
-B2_HD void bodies_end(const WorldDev<T>& W, T* X, BodyWork<T>* bw)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void bodies_end(const WorldDev<T>& W, T* X, BodyWork<T>* bw, const P& prm = P())
 {
-    for (int i = 0; i < W.nfree; ++i) body_end(W, i, X + 13 * i, bw[i]);
+    for (int i = 0; i < W.nfree; ++i) body_end(W, i, X + 13 * i, bw[i], prm);
 }
 
 // One step of every free body of one world. X: nfree x 13 (position, quaternion wxyz, linear and angular velocity
 // of the body frame, world coordinates). cs: caller-provided contact workspace (kMaxContacts). Returns the number
 // of contacts; their impulses divided by dt are the contact forces on body a.
-template <typename T>
-B2_HD int world_step(const WorldDev<T>& W, T* X, Contact<T>* cs, long long env = -1)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD int world_step(const WorldDev<T>& W, T* X, Contact<T>* cs, long long env = -1, const P& prm = P())
 {
     BodyWork<T> bw[kMaxFree];
-    bodies_begin(W, X, bw, env);
+    bodies_begin(W, X, bw, env, prm);
     int nc = 0;
-    free_contacts(W, bw, cs, nc);
+    free_contacts(W, bw, cs, nc, prm);
     contact_frames(cs, nc);
     contact_rows<false>(W, bw, (const RobotWork<T>*)nullptr, cs, nc);
     for (int it = 0; it < W.iterations; ++it) contact_sweep<false>(bw, (RobotWork<T>*)nullptr, cs, nc);
-    bodies_end(W, X, bw);
+    bodies_end(W, X, bw, prm);
     return nc;
 }
 
@@ -548,9 +623,9 @@ B2_HD void spd_inverse(int n, T* M, T* Minv)
 // in one LCP. On entry q holds the joint positions and dq the joint velocities after the unconstrained update
 // (dq += ddq dt); on return dq holds the constrained velocities. Positions are integrated by the caller.
 // servo_bits / servo_target: joints under a velocity servo. Returns the number of contacts.
-template <typename T>
+template <typename T, typename P = WorldNominal<T>>
 B2_HD int coupled_step(const WorldDev<T>& W, const ModelDev<T>& m, const T* q, T* dq, unsigned servo_bits,
-                       const T* servo_target, T* X, Contact<T>* cs, RobotWork<T>& rw, long long env = -1);
+                       const T* servo_target, T* X, Contact<T>* cs, RobotWork<T>& rw, long long env = -1, const P& prm = P());
 
 // ---------------------------------------------------------------------------------------------------------
 // Dense-row form of the same constraint problem, for the warp-cooperative solver (b2_kernels.cuh k_pgs_solve):
@@ -668,9 +743,10 @@ B2_HD void write_dense_rows(const WorldDev<T>& W, const ModelDev<T>* m, int nq, 
 
 // Everything of a coupled step before the solve: kinematics, unconstrained free-body velocities, contact points,
 // joint rows, M^-1, the robot-side contact rows and effective masses. Same sequence as coupled_step.
-template <typename T>
+template <typename T, typename P = WorldNominal<T>>
 B2_HD int coupled_prepare(const WorldDev<T>& W, const ModelDev<T>& m, const T* q, const T* dq, unsigned servo_bits,
-                          const T* servo_target, const T* X, BodyWork<T>* bw, Contact<T>* cs, RobotWork<T>& rw, long long env = -1)
+                          const T* servo_target, const T* X, BodyWork<T>* bw, Contact<T>* cs, RobotWork<T>& rw, long long env = -1,
+                          const P& prm = P())
 {
     const int nq = m.nq;
     const T dt = W.dt, inf = T(INFINITY);
@@ -678,10 +754,10 @@ B2_HD int coupled_prepare(const WorldDev<T>& W, const ModelDev<T>& m, const T* q
     rw.nrc = 0;
     for (int j = 0; j < nq; ++j) rw.dq[j] = dq[j];
     forward_kinematics<T, kMaxDofs>(m, q, rw.Rw, rw.pw);
-    bodies_begin(W, X, bw, env);
+    bodies_begin(W, X, bw, env, prm);
     int nc = 0;
-    free_contacts(W, bw, cs, nc);
-    robot_contacts(W, bw, rw, cs, nc);
+    free_contacts(W, bw, cs, nc, prm);
+    robot_contacts(W, bw, rw, cs, nc, prm);
     int nr = 0;
     for (int j = 0; j < nq; ++j) {
         if ((servo_bits >> j) & 1u) {
@@ -710,20 +786,20 @@ B2_HD int coupled_prepare(const WorldDev<T>& W, const ModelDev<T>& m, const T* q
 // What the three-launch pipeline needs of a coupled step before its solver: kinematics, unconstrained free-body
 // velocities, contact points and tangents, joint rows and M^-1 (only when a joint row or a robot contact exists).
 // M_known: the joint-space mass matrix at q when the caller already has it (the computed-torque controller), or null.
-template <typename T>
+template <typename T, typename P = WorldNominal<T>>
 B2_HD int coupled_prepare_rows(const WorldDev<T>& W, const ModelDev<T>& m, const T* q, const T* dq, unsigned servo_bits,
                                const T* servo_target, const T* X, const T* M_known, BodyWork<T>* bw, Contact<T>* cs,
-                               RobotWork<T>& rw, bool with_minv = true, long long env = -1)
+                               RobotWork<T>& rw, bool with_minv = true, long long env = -1, const P& prm = P())
 {
     const int nq = m.nq;
     const T dt = W.dt, inf = T(INFINITY);
     rw.nq = nq;
     for (int j = 0; j < nq; ++j) rw.dq[j] = dq[j];
     forward_kinematics<T, kMaxDofs>(m, q, rw.Rw, rw.pw);
-    bodies_begin(W, X, bw, env);
+    bodies_begin(W, X, bw, env, prm);
     int nc = 0;
-    free_contacts(W, bw, cs, nc);
-    robot_contacts(W, bw, rw, cs, nc);
+    free_contacts(W, bw, cs, nc, prm);
+    robot_contacts(W, bw, rw, cs, nc, prm);
     int nr = 0;
     for (int j = 0; j < nq; ++j) {
         if ((servo_bits >> j) & 1u) {
@@ -749,32 +825,32 @@ B2_HD int coupled_prepare_rows(const WorldDev<T>& W, const ModelDev<T>& m, const
 }
 
 // Pose part of bodies_begin only (no velocity update): what the finishing kernel needs to integrate the bodies.
-template <typename T>
-B2_HD void body_pose(const WorldDev<T>& W, int i, const T* x, BodyWork<T>& b)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void body_pose(const WorldDev<T>& W, int i, const T* x, BodyWork<T>& b, const P& prm = P())
 {
     b.R = quat_to_rot(x + 3);
-    b.xc = ld3(x) + mul(b.R, ld3(W.body[i].com));
+    b.xc = ld3(x) + mul(b.R, prm.com(W.body[i], i));
 }
-template <typename T>
-B2_HD void bodies_pose(const WorldDev<T>& W, const T* X, BodyWork<T>* bw)
+template <typename T, typename P = WorldNominal<T>>
+B2_HD void bodies_pose(const WorldDev<T>& W, const T* X, BodyWork<T>* bw, const P& prm = P())
 {
-    for (int i = 0; i < W.nfree; ++i) body_pose(W, i, X + 13 * i, bw[i]);
+    for (int i = 0; i < W.nfree; ++i) body_pose(W, i, X + 13 * i, bw[i], prm);
 }
 
 // One step of a world that couples an articulated model with free bodies through contacts, solved by one thread
 // (host tests, worlds too large for the warp-cooperative solver).
-template <typename T>
+template <typename T, typename P>
 B2_HD int coupled_step(const WorldDev<T>& W, const ModelDev<T>& m, const T* q, T* dq, unsigned servo_bits,
-                       const T* servo_target, T* X, Contact<T>* cs, RobotWork<T>& rw, long long env)
+                       const T* servo_target, T* X, Contact<T>* cs, RobotWork<T>& rw, long long env, const P& prm)
 {
     BodyWork<T> bw[kMaxFree];
-    const int nc = coupled_prepare(W, m, q, dq, servo_bits, servo_target, X, bw, cs, rw, env);
+    const int nc = coupled_prepare(W, m, q, dq, servo_bits, servo_target, X, bw, cs, rw, env, prm);
     for (int it = 0; it < W.iterations; ++it) {
         joint_row_sweep(rw);
         contact_sweep<true>(bw, &rw, cs, nc);
     }
     for (int j = 0; j < m.nq; ++j) dq[j] = rw.dq[j];
-    bodies_end(W, X, bw);
+    bodies_end(W, X, bw, prm);
     return nc;
 }
 

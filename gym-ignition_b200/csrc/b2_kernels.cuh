@@ -1304,8 +1304,31 @@ __device__ __forceinline__ void write_base_accel(const WorldBuffers<T>& b, int i
     for (int k = 0; k < 6; ++k) o[k] = (after[7 + k] - vel_before[k]) * idt;
 }
 
-template <typename T>
-__global__ void __launch_bounds__(64) k_world_free(const WorldDev<T>* __restrict__ world, const WorldBuffers<T> b)
+// ENV: the world kernels read the per-env rows of `rows` (WorldEnv) wherever a slot has them; otherwise the shared world
+// description (WorldNominal), and `rows` is not read. The rows come last, so the ENV = false kernels keep their parameter
+// layout; __grid_constant__: the coupled stages reach them through a pointer without a local copy.
+template <bool ENV, typename T>
+__device__ __forceinline__ auto world_params(const WorldRows<T>& rows, int64_t e)
+{
+    if constexpr (ENV) return WorldEnv<T>{rows, (long long)e};
+    else return WorldNominal<T>{};
+}
+template <typename T, bool ENV> struct WorldRowsRef {
+    __device__ __forceinline__ WorldNominal<T> params(int64_t) const { return {}; }
+};
+template <typename T> struct WorldRowsRef<T, true> {
+    const WorldRows<T>* rows;
+    __device__ __forceinline__ WorldEnv<T> params(int64_t e) const { return WorldEnv<T>{*rows, (long long)e}; }
+};
+template <bool ENV, typename T> __device__ __forceinline__ WorldRowsRef<T, ENV> rows_ref(const WorldRows<T>& rows)
+{
+    if constexpr (ENV) return WorldRowsRef<T, true>{&rows};
+    else return WorldRowsRef<T, false>{};
+}
+
+template <typename T, bool ENV = false>
+__global__ void __launch_bounds__(64) k_world_free(const WorldDev<T>* __restrict__ world, const WorldBuffers<T> b,
+                                                   const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ WorldDev<T> W;
     stage_world(world, W);
@@ -1319,7 +1342,7 @@ __global__ void __launch_bounds__(64) k_world_free(const WorldDev<T>* __restrict
         for (int i = 0; i < W.nfree; ++i)
             for (int k = 0; k < 6; ++k) before[6 * i + k] = X[13 * i + 7 + k];
         Contact<T> cs[kMaxContacts];
-        const int nc = world_step(W, X, cs, (long long)e);
+        const int nc = world_step(W, X, cs, (long long)e, world_params<ENV>(rows, e));
         write_contact_records(b, e, cs, nc, W.dt);
         for (int i = 0; i < W.nfree; ++i) write_base_accel(b, i, e, before + 6 * i, X + 13 * i, W.dt);
     }
@@ -1334,8 +1357,8 @@ __global__ void __launch_bounds__(64) k_world_free(const WorldDev<T>* __restrict
 // of the free bodies -> contact points -> ONE projected Gauss-Seidel solve over the tree's joint rows and every
 // contact (b2_contact.hpp coupled_step) -> position integration -> contact records.
 // ---------------------------------------------------------------------------------------------------------
-template <typename T>
-struct CoupledWorld {
+template <typename T, bool ENV = false>
+struct CoupledWorld : WorldRowsRef<T, ENV> {
     static constexpr bool active = true;
     static constexpr bool deferred = false;
     static constexpr bool keeps_M = false;
@@ -1360,7 +1383,7 @@ struct CoupledWorld {
         T vel_before[kMaxFree * 6];
         for (int i = 0; i < W.nfree; ++i)
             for (int k = 0; k < 6; ++k) vel_before[6 * i + k] = X[13 * i + 7 + k];
-        const int nc = coupled_step(W, m, q, dq, servo_bits, vel_target_row, X, cs, rw, (long long)e);
+        const int nc = coupled_step(W, m, q, dq, servo_bits, vel_target_row, X, cs, rw, (long long)e, this->params(e));
         for (int i = 0; i < W.nfree; ++i) write_base_accel(wb, i, e, vel_before + 6 * i, X + 13 * i, dt);
         for (int j = 0; j < nq; ++j) {
             w[kSlotsPerBody * j + SL_DQ] = dq[j];
@@ -1372,10 +1395,11 @@ struct CoupledWorld {
 
 // Single-thread variant: the whole coupled step, solve included, in one launch (worlds whose generalized velocity
 // does not fit the warp-cooperative solver).
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(64) k_world_coupled(const ModelDev<T>* __restrict__ tables, const RunCfg<T> cfg,
                                                       const RunBuffers<T> b, const TreeTopo topo,
-                                                      const WorldDev<T>* __restrict__ world, const WorldBuffers<T> wb)
+                                                      const WorldDev<T>* __restrict__ world, const WorldBuffers<T> wb,
+                                                      const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     __shared__ WorldDev<T> W;
@@ -1386,7 +1410,7 @@ __global__ void __launch_bounds__(64) k_world_coupled(const ModelDev<T>* __restr
     T X[kMaxFree * 13];
     load_free_bodies(W, wb, e, X);
     T buf[kSlotsPerBody * kMaxDofs + kSlotsPerBranch * kMaxBranch];
-    CoupledWorld<T> cw{W, wb, e, X};
+    CoupledWorld<T, ENV> cw{rows_ref<ENV>(rows), W, wb, e, X};
     run_tree_env(m, cfg, b, topo, e, Scratch<T, 1>{buf, 1}, cw);
     for (int i = 0; i < W.nfree; ++i)
         for (int k = 0; k < 13; ++k) wb.base_state[i][e * 13 + k] = X[13 * i + k];
@@ -1436,9 +1460,9 @@ __device__ __forceinline__ void write_contact_geometry(const WorldBuffers<T>& b,
     }
 }
 
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(64) k_world_prepare(const WorldDev<T>* __restrict__ world, const WorldBuffers<T> b,
-                                                      const PgsBuffers<T> g)
+                                                      const PgsBuffers<T> g, const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ WorldDev<T> W;
     stage_world(world, W);
@@ -1452,16 +1476,17 @@ __global__ void __launch_bounds__(64) k_world_prepare(const WorldDev<T>* __restr
     if (b.paused) return;
     BodyWork<T> bw[kMaxFree];
     Contact<T> cs[kMaxContacts];
-    bodies_begin(W, X, bw, (long long)e);
+    const auto prm = world_params<ENV>(rows, e);
+    bodies_begin(W, X, bw, (long long)e, prm);
     int nc = 0;
-    free_contacts(W, bw, cs, nc);
+    free_contacts(W, bw, cs, nc, prm);
     contact_frames(cs, nc);
     write_dense_rows(W, (const ModelDev<T>*)nullptr, 0, (const RobotWork<T>*)nullptr, bw, cs, nc, pgs_env(g, e));
     write_contact_geometry(b, e, cs, nc);
 }
 
-template <typename T>
-struct CoupledPrepare {
+template <typename T, bool ENV = false>
+struct CoupledPrepare : WorldRowsRef<T, ENV> {
     static constexpr bool active = true;
     static constexpr bool deferred = true;
     static constexpr bool keeps_M = true;
@@ -1487,18 +1512,19 @@ struct CoupledPrepare {
         BodyWork<T> bw[kMaxFree];
         Contact<T> cs[kMaxContacts];
         RobotWork<T> rw;
-        int nc = coupled_prepare_rows(W, m, q, dq, servo_bits, vel_target_row, X, have_M ? Mq : (const T*)nullptr, bw, cs, rw, true, (long long)e);
+        int nc = coupled_prepare_rows(W, m, q, dq, servo_bits, vel_target_row, X, have_M ? Mq : (const T*)nullptr, bw, cs, rw, true, (long long)e,
+                                      this->params(e));
         write_dense_rows(W, &m, nq, &rw, bw, cs, nc, pgs_env(g, e));
         write_contact_geometry(wb, e, cs, nc);
         have_M = false;
     }
 };
 
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(64) k_coupled_prepare(const ModelDev<T>* __restrict__ tables, const RunCfg<T> cfg,
                                                         const RunBuffers<T> b, const TreeTopo topo,
                                                         const WorldDev<T>* __restrict__ world, const WorldBuffers<T> wb,
-                                                        const PgsBuffers<T> g)
+                                                        const PgsBuffers<T> g, const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     __shared__ WorldDev<T> W;
@@ -1511,7 +1537,7 @@ __global__ void __launch_bounds__(64) k_coupled_prepare(const ModelDev<T>* __res
     for (int i = 0; i < W.nfree; ++i)
         for (int k = 0; k < 13; ++k) wb.base_state[i][e * 13 + k] = X[13 * i + k];
     T buf[kSlotsPerBody * kMaxDofs + kSlotsPerBranch * kMaxBranch];
-    CoupledPrepare<T> cp{W, wb, g, e, X, false};
+    CoupledPrepare<T, ENV> cp{rows_ref<ENV>(rows), W, wb, g, e, X, false};
     // leaves q (not yet integrated), the unconstrained dq and ddq in the state / acceleration buffers
     run_tree_env(m, cfg, b, topo, e, Scratch<T, 1>{buf, 1}, cp);
 }
@@ -1569,10 +1595,11 @@ __device__ __forceinline__ uint32_t load_positions(const RunBuffers<T>& b, int n
     return mask;
 }
 
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(64) k_coupled_rows(const ModelDev<T>* __restrict__ tables, const RunCfg<T> cfg,
                                                      const RunBuffers<T> b, const WorldDev<T>* __restrict__ world,
-                                                     const WorldBuffers<T> wb, const PgsBuffers<T> g)
+                                                     const WorldBuffers<T> wb, const PgsBuffers<T> g,
+                                                     const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ ModelDev<T> m;
     __shared__ WorldDev<T> W;
@@ -1598,7 +1625,8 @@ __global__ void __launch_bounds__(64) k_coupled_rows(const ModelDev<T>* __restri
     BodyWork<T> bw[kMaxFree];
     Contact<T> cs[kMaxContacts];
     RobotWork<T> rw;
-    int nc = coupled_prepare_rows(W, m, q, dq, servo_bits, b.vel_target + e * nq, X, (const T*)nullptr, bw, cs, rw, false, (long long)e);
+    int nc = coupled_prepare_rows(W, m, q, dq, servo_bits, b.vel_target + e * nq, X, (const T*)nullptr, bw, cs, rw, false, (long long)e,
+                                  world_params<ENV>(rows, e));
     write_dense_rows(W, &m, nq, &rw, bw, cs, nc, pgs_env(g, e), false);
     write_contact_geometry(wb, e, cs, nc);
 }
@@ -1958,10 +1986,11 @@ __global__ void __launch_bounds__(64, 7) k_pgs_solve(const PgsBuffers<T> g, int 
 // kFinishLanes threads per env: the stage is a handful of dependent loads per joint / body / contact, so its duration is
 // the longest of those chains; lanes take them side by side (lane = joint, lane = free body, lane = contact).
 constexpr int kFinishLanes = 16;
-template <typename T>
+template <typename T, bool ENV = false>
 __global__ void __launch_bounds__(128) k_world_finish(const WorldDev<T>* __restrict__ world, const WorldBuffers<T> b,
                                                       const PgsBuffers<T> g, T* __restrict__ state, T* __restrict__ accel,
-                                                      int nq, uint32_t* __restrict__ robot_reset_mask)
+                                                      int nq, uint32_t* __restrict__ robot_reset_mask,
+                                                      const __grid_constant__ WorldRows<T> rows)
 {
     __shared__ WorldDev<T> W;
     stage_world(world, W);
@@ -1986,11 +2015,12 @@ __global__ void __launch_bounds__(128) k_world_finish(const WorldDev<T>* __restr
         BodyWork<T> bw;
         for (int k = 0; k < 13; ++k) X[k] = b.base_state[i][e * 13 + k];
         for (int k = 0; k < 6; ++k) before[k] = X[7 + k];
-        body_pose(W, i, X, bw);
+        const auto prm = world_params<ENV>(rows, e);
+        body_pose(W, i, X, bw, prm);
         const T* vb = v + nq + 6 * i;
         bw.vc = v3(vb[0], vb[1], vb[2]);
         bw.w = v3(vb[3], vb[4], vb[5]);
-        body_end(W, i, X, bw);
+        body_end(W, i, X, bw, prm);
         for (int k = 0; k < 13; ++k) b.base_state[i][e * 13 + k] = X[k];
         write_base_accel(b, i, e, before, X, dt);
     }

@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
+#include <array>
 #include <fstream>
 #include <memory>
 #include <sstream>
@@ -98,6 +99,8 @@ struct ModelState {
     int max_episode_steps = 5000;
     double rand_mass_delta = 0, rand_gravity_sigma = 0;
     bool env_params = false;  // B2_BUF_BODY_INERTIA / JOINT_DYNAMICS / GRAVITY allocated (b2sim_enable_env_params)
+    void* body_rows = nullptr;  // [N, b2::kFreeBodyCols] per-env inertial data of a free body (b2sim_enable_free_body_params)
+    void* mu_rows = nullptr;    // [N, nshapes] per-env friction coefficient of every collision shape (b2sim_enable_shape_friction)
     unsigned long long* d_step = nullptr;  // device-side step counter of the fused task (next Philox step index)
     unsigned int* d_ticket = nullptr;
     bool graph_recorded = false;
@@ -133,6 +136,9 @@ struct b2sim {
     std::vector<int> static_shape_model, static_shape_link;
     int robot_model = -1;                                // articulated model whose link shapes take part in contacts
     std::vector<int> robot_shape_link;                   // link of each robot shape (reporting)
+    // loader shape (column of the model's friction rows) of every shape slot of the world description
+    std::vector<std::array<int, b2::kMaxBodyShapes>> free_shape_col;
+    std::vector<int> static_shape_col, robot_shape_col;
     int32_t* contact_count = nullptr;
     int32_t* contact_ids = nullptr;
     void* contact_data = nullptr;
@@ -750,6 +756,9 @@ int upload_world(b2sim* s)
     s->static_shape_model.clear();
     s->static_shape_link.clear();
     s->robot_shape_link.clear();
+    s->free_shape_col.clear();
+    s->static_shape_col.clear();
+    s->robot_shape_col.clear();
     s->robot_model = -1;
     W.iterations = s->contact_iterations;
     W.dt = (T)((double)s->dt_ns / 1e9);
@@ -773,9 +782,14 @@ int upload_world(b2sim* s)
                                    (I[3] * I[7] - I[4] * I[6]) / det, (I[1] * I[6] - I[0] * I[7]) / det, (I[0] * I[4] - I[1] * I[3]) / det};
             for (int k = 0; k < 9; ++k) { fb.Ic[k] = (T)I[k]; fb.Ic_inv[k] = (T)inv[k]; }
             for (int k = 0; k < 3; ++k) fb.com[k] = (T)t.body_com[k];
+            std::array<int, b2::kMaxBodyShapes> cols;
+            cols.fill(-1);
             for (int k = 0; k < t.nshapes && fb.nshapes < b2::kMaxBodyShapes; ++k)
-                if (t.shape_type[k] == B2_SHAPE_BOX || t.shape_type[k] == B2_SHAPE_SPHERE)
+                if (t.shape_type[k] == B2_SHAPE_BOX || t.shape_type[k] == B2_SHAPE_SPHERE) {
+                    cols[fb.nshapes] = k;
                     fill_shape(fb.shape[fb.nshapes++], t, k, b2::Pose(), (int)id, false);
+                }
+            s->free_shape_col.push_back(cols);
         } else if (ms->kind == B2_KIND_STATIC) {
             for (int k = 0; k < t.nshapes; ++k) {
                 if (t.shape_type[k] != B2_SHAPE_BOX && t.shape_type[k] != B2_SHAPE_PLANE) continue;
@@ -783,6 +797,7 @@ int upload_world(b2sim* s)
                 fill_shape(W.stat[W.nstatic++], t, k, ms->base, (int)id, true);
                 s->static_shape_model.push_back((int)id);
                 s->static_shape_link.push_back(t.shape_link[k]);
+                s->static_shape_col.push_back(k);
             }
         } else if (t.nq > 0 && s->robot_model < 0) {
             // articulated model: box / sphere shapes on its moving links collide with the free bodies and the static
@@ -794,6 +809,7 @@ int upload_world(b2sim* s)
                 fill_shape(W.rshape[W.nrobot], t, k, b2::Pose(), (int)id, false);  // pose in the body frame
                 W.rbody[W.nrobot++] = body;
                 s->robot_shape_link.push_back(t.shape_link[k]);
+                s->robot_shape_col.push_back(k);
             }
             if (W.nrobot > 0) s->robot_model = (int)id;
         }
@@ -876,6 +892,38 @@ b2::WorldBuffers<T> world_buffers(b2sim* s, int paused)
     return b;
 }
 
+// Per-env rows of the world's slots (b2sim_enable_free_body_params, b2sim_enable_shape_friction), resolved on every launch so
+// that enabling or disabling rows needs no world rebuild. *any: some model of the world has rows (the ENV kernels run).
+template <typename T>
+b2::WorldRows<T> world_rows(const b2sim* s, bool* any)
+{
+    b2::WorldRows<T> r;
+    memset(&r, 0, sizeof r);
+    *any = false;
+    for (const auto& ms : s->models)
+        if (!ms->removed && (ms->body_rows || ms->mu_rows)) *any = true;
+    if (!*any) return r;
+    for (size_t i = 0; i < s->free_models.size(); ++i) {
+        const ModelState* ms = s->models[s->free_models[i]].get();
+        r.body[i] = (const T*)ms->body_rows;
+        r.body_mu_stride[i] = ms->model->t.nshapes;
+        for (int k = 0; k < b2::kMaxBodyShapes; ++k)
+            if (ms->mu_rows && s->free_shape_col[i][k] >= 0) r.body_mu[i][k] = (const T*)ms->mu_rows + s->free_shape_col[i][k];
+    }
+    for (size_t k = 0; k < s->static_shape_col.size(); ++k) {
+        const ModelState* ms = s->models[s->static_shape_model[k]].get();
+        r.stat_mu_stride[k] = ms->model->t.nshapes;
+        if (ms->mu_rows) r.stat_mu[k] = (const T*)ms->mu_rows + s->static_shape_col[k];
+    }
+    if (s->robot_model >= 0) {
+        const ModelState* ms = s->models[s->robot_model].get();
+        r.robot_mu_stride = ms->model->t.nshapes;
+        for (size_t k = 0; k < s->robot_shape_col.size(); ++k)
+            if (ms->mu_rows) r.robot_mu[k] = (const T*)ms->mu_rows + s->robot_shape_col[k];
+    }
+    return r;
+}
+
 // Solve + finish launches that follow a prepare kernel (not on paused runs).
 template <typename T>
 int launch_solve_finish(b2sim* s, ModelState* robot, bool clear_robot_mask = false)
@@ -893,10 +941,12 @@ int launch_solve_finish(b2sim* s, ModelState* robot, bool clear_robot_mask = fal
         b2::k_pgs_solve<T, 32><<<grid_for(s->n, 2), 64, smem, s->stream>>>(g, s->contact_iterations);
     }
     B2_CUDA(cudaGetLastError());
-    b2::k_world_finish<T><<<grid_for(s->n * b2::kFinishLanes, 128), 128, 0, s->stream>>>(
+    bool env = false;
+    const b2::WorldRows<T> rows = world_rows<T>(s, &env);
+    (env ? b2::k_world_finish<T, true> : b2::k_world_finish<T, false>)<<<grid_for(s->n * b2::kFinishLanes, 128), 128, 0, s->stream>>>(
         (const b2::WorldDev<T>*)s->d_world, world_buffers<T>(s, 0), g, robot ? (T*)robot->buf[B2_BUF_STATE] : nullptr,
         robot ? (T*)robot->buf[B2_BUF_ACCELERATION] : nullptr, robot ? robot->model->t.nq : 0,
-        robot && clear_robot_mask ? (uint32_t*)robot->buf[B2_BUF_RESET_MASK] : nullptr);
+        robot && clear_robot_mask ? (uint32_t*)robot->buf[B2_BUF_RESET_MASK] : nullptr, rows);
     B2_CUDA(cudaGetLastError());
     s->launches += 2;
     return B2_OK;
@@ -913,15 +963,18 @@ int launch_world(b2sim* s, int paused)
     static const char* solver = getenv("B2_CONTACT_SOLVER");
     const bool forced_thread = solver && !strcmp(solver, "thread");
     const bool forced_warp = solver && !strcmp(solver, "warp");
+    bool env = false;
+    const b2::WorldRows<T> rows = world_rows<T>(s, &env);
     if (s->pgs_nvp && !forced_thread && (forced_warp || s->n <= kWarpSolverMaxEnvs)) {
         const int block = s->n <= kWarpSolverMaxEnvs ? 32 : 64;  // small batches: one warp per SM
-        b2::k_world_prepare<T><<<grid_for(s->n, block), block, 0, s->stream>>>((const b2::WorldDev<T>*)s->d_world,
-                                                                             world_buffers<T>(s, paused), pgs_buffers<T>(s));
+        (env ? b2::k_world_prepare<T, true> : b2::k_world_prepare<T, false>)<<<grid_for(s->n, block), block, 0, s->stream>>>(
+            (const b2::WorldDev<T>*)s->d_world, world_buffers<T>(s, paused), pgs_buffers<T>(s), rows);
         ++s->launches;
         B2_CUDA(cudaGetLastError());
         return paused ? B2_OK : launch_solve_finish<T>(s, nullptr);
     }
-    b2::k_world_free<T><<<grid_for(s->n, 64), 64, 0, s->stream>>>((const b2::WorldDev<T>*)s->d_world, world_buffers<T>(s, paused));
+    (env ? b2::k_world_free<T, true> : b2::k_world_free<T, false>)<<<grid_for(s->n, 64), 64, 0, s->stream>>>(
+        (const b2::WorldDev<T>*)s->d_world, world_buffers<T>(s, paused), rows);
     ++s->launches;
     B2_CUDA(cudaGetLastError());
     return B2_OK;
@@ -936,6 +989,8 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
     int rc = tree_topology(ms, &topo);
     if (rc != B2_OK) return rc;
     const char* split_env = getenv("B2_COUPLED_SPLIT");  // read per launch: tests compare the two pipelines in one process
+    bool env = false;
+    const b2::WorldRows<T> rows = world_rows<T>(s, &env);
     if (s->pgs_nvp && !paused && !(split_env && !strcmp(split_env, "0"))) {
         // Unpaused step: the three independent parts of the prepare stage run concurrently on forked streams
         // (b2_kernels.cuh, "Split prepare"); the solve waits for all of them. 32-thread blocks: at the 4,096-env size of
@@ -950,7 +1005,8 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
             // and 65 us). The same explicit split for all three (64 KB shared, the rest L1 for their per-thread scratch).
             const int carve = b2::kCoupledCarveout;
             B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_dynamics<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
-            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_rows<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_rows<T, false>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
+            B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_rows<T, true>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
             B2_CUDA(cudaFuncSetAttribute(b2::k_coupled_minv<T>, cudaFuncAttributePreferredSharedMemoryCarveout, carve));
         }
         const b2::RunBuffers<T> rb = run_buffers<T>(s, ms);
@@ -968,8 +1024,8 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
         B2_CUDA(cudaStreamWaitEvent(s->fork[0], s->fork_ev[0], 0));
         B2_CUDA(cudaStreamWaitEvent(s->fork[1], s->fork_ev[0], 0));
         // launch order = block dispatch order: the longest kernel (rows) first, the lane-parallel dynamics last
-        b2::k_coupled_rows<T><<<grid_for(s->n, 32), 32, 0, s->fork[0]>>>(tb, cfg, rb, (const b2::WorldDev<T>*)s->d_world,
-                                                                        world_buffers<T>(s, 0), g);
+        (env ? b2::k_coupled_rows<T, true> : b2::k_coupled_rows<T, false>)<<<grid_for(s->n, 32), 32, 0, s->fork[0]>>>(
+            tb, cfg, rb, (const b2::WorldDev<T>*)s->d_world, world_buffers<T>(s, 0), g, rows);
         if (tr) cudaEventRecord(tev[2], s->fork[0]);
         b2::k_coupled_minv<T><<<grid_for(s->n, 32), 32, 0, s->fork[1]>>>(tb, rb, g);
         if (tr) cudaEventRecord(tev[3], s->fork[1]);
@@ -1001,16 +1057,16 @@ int launch_coupled(b2sim* s, ModelState* ms, int paused, uint32_t compute_bit, u
     }
     if (s->pgs_nvp) {
         // 32-thread blocks: at the 4,096-env size of this configuration every warp gets an SM (and its L1) of its own
-        b2::k_coupled_prepare<T><<<grid_for(s->n, 32), 32, 0, s->stream>>>(
+        (env ? b2::k_coupled_prepare<T, true> : b2::k_coupled_prepare<T, false>)<<<grid_for(s->n, 32), 32, 0, s->stream>>>(
             (const b2::ModelDev<T>*)ms->d_tables, cfg, run_buffers<T>(s, ms), topo, (const b2::WorldDev<T>*)s->d_world,
-            world_buffers<T>(s, paused), pgs_buffers<T>(s));
+            world_buffers<T>(s, paused), pgs_buffers<T>(s), rows);
         ++s->launches;
         B2_CUDA(cudaGetLastError());
         return paused ? B2_OK : launch_solve_finish<T>(s, ms);
     }
-    b2::k_world_coupled<T><<<grid_for(s->n, 64), 64, 0, s->stream>>>((const b2::ModelDev<T>*)ms->d_tables, cfg, run_buffers<T>(s, ms),
-                                                                   topo, (const b2::WorldDev<T>*)s->d_world,
-                                                                   world_buffers<T>(s, paused));
+    (env ? b2::k_world_coupled<T, true> : b2::k_world_coupled<T, false>)<<<grid_for(s->n, 64), 64, 0, s->stream>>>(
+        (const b2::ModelDev<T>*)ms->d_tables, cfg, run_buffers<T>(s, ms), topo, (const b2::WorldDev<T>*)s->d_world,
+        world_buffers<T>(s, paused), rows);
     ++s->launches;
     B2_CUDA(cudaGetLastError());
     return B2_OK;
@@ -1036,6 +1092,8 @@ void free_model_buffers(ModelState* ms)
     for (auto& b : ms->buf)
         if (b) { cudaFree(b); b = nullptr; }
     if (ms->force_read) { cudaFree(ms->force_read); ms->force_read = nullptr; }
+    if (ms->body_rows) { cudaFree(ms->body_rows); ms->body_rows = nullptr; }
+    if (ms->mu_rows) { cudaFree(ms->mu_rows); ms->mu_rows = nullptr; }
     if (ms->d_tables) { cudaFree(ms->d_tables); ms->d_tables = nullptr; }
     if (ms->d_step) { cudaFree(ms->d_step); ms->d_step = nullptr; }
     if (ms->d_ticket) { cudaFree(ms->d_ticket); ms->d_ticket = nullptr; }
@@ -1044,6 +1102,32 @@ void free_model_buffers(ModelState* ms)
         if (*p) { cudaFreeHost(*p); *p = nullptr; }
 }
 
+// Shared part of b2sim_enable_free_body_params / b2sim_enable_shape_friction: `rows` is the model's [N, cols] allocation,
+// `init` its first row, copied into every env.
+int enable_rows(b2sim* s, void*& rows, int enable, int cols, const double* init, b2_buffer* out)
+{
+    if (!enable) {
+        if (rows) {
+            B2_CUDA(cudaStreamSynchronize(s->stream));  // runs still queued read the rows
+            cudaFree(rows);
+            rows = nullptr;
+        }
+        return B2_OK;
+    }
+    if (!rows) {
+        B2_CUDA(cudaMalloc(&rows, (size_t)s->n * cols * s->esize()));
+        for (int k = 0; k < cols; ++k) {
+            const int rc = col_fill_any(s, rows, cols, k, init[k]);
+            if (rc != B2_OK) {
+                cudaFree(rows);
+                rows = nullptr;
+                return rc;
+            }
+        }
+    }
+    if (out) *out = b2_buffer{rows, s->n, cols, s->dtype, (int32_t)s->esize()};
+    return B2_OK;
+}
 }  // namespace
 
 // =====================================================================================================
@@ -1948,6 +2032,30 @@ int b2sim_enable_env_params(b2sim* s, int model, int enable)
         return fail(rc, "%s", msg.c_str());
     }
     return B2_OK;
+}
+
+int b2sim_enable_free_body_params(b2sim* s, int model, int enable, b2_buffer* out)
+{
+    ModelState* ms = get_model(s, model);
+    if (!ms) return fail(B2_ERR_NOT_FOUND, "model %d not found", model);
+    DeviceGuard guard__(s->device);
+    if (enable && ms->kind != B2_KIND_FREE)
+        return fail(B2_ERR_UNSUPPORTED, "model '%s' is not a free-floating body", ms->name.c_str());
+    const b2_model_tables& t = ms->model->t;
+    double init[b2::kFreeBodyCols] = {t.body_mass, t.body_com[0], t.body_com[1], t.body_com[2]};
+    const int sym[6] = {0, 1, 2, 4, 5, 8};
+    for (int k = 0; k < 6; ++k) init[4 + k] = t.body_Ic[sym[k]];
+    return enable_rows(s, ms->body_rows, enable, b2::kFreeBodyCols, init, out);
+}
+
+int b2sim_enable_shape_friction(b2sim* s, int model, int enable, b2_buffer* out)
+{
+    ModelState* ms = get_model(s, model);
+    if (!ms) return fail(B2_ERR_NOT_FOUND, "model %d not found", model);
+    DeviceGuard guard__(s->device);
+    const b2_model_tables& t = ms->model->t;
+    if (enable && t.nshapes == 0) return fail(B2_ERR_UNSUPPORTED, "model '%s' has no collision shape", ms->name.c_str());
+    return enable_rows(s, ms->mu_rows, enable, t.nshapes, t.shape_mu, out);
 }
 
 // ---- zero-copy view --------------------------------------------------------------------------------------------

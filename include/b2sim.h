@@ -247,6 +247,29 @@ int b2sim_set_joint_friction(b2sim* s, int model, int joint, double coulomb, dou
  * or static model, a model with a pendulum / cart-pole task, and a world with free bodies (also from b2sim_run when a
  * free body is inserted later); b2sim_set_task refuses a pendulum / cart-pole task on a model with per-env parameters. */
 int b2sim_enable_env_params(b2sim* s, int model, int enable);
+/* Per-env parameters of a world's free bodies and contacts (domain randomisation of the objects a robot manipulates and of
+ * the surfaces they touch). Both entry points follow b2sim_enable_env_params: enable != 0 allocates the rows in the
+ * simulator dtype, fills every row with the model's current values and returns the view in `out` (which may be NULL);
+ * enabling rows that exist returns the same view and does not refill it. The caller owns the rows: a write on the
+ * simulator stream between runs acts from the next unpaused run on. Nothing checks them on the device: they must stay
+ * physically valid (mass > 0, a symmetric positive-definite inertia, mu >= 0). enable = 0 synchronises the stream and
+ * frees the rows, and the model returns to the shared values; removing the model or destroying the simulator frees them
+ * too, and views taken before are then invalid. Rows may be enabled before a free body is inserted: they are read once
+ * the world has a contact stage, and they survive the rebuilds of the world description when other models are inserted or
+ * removed. What stays nominal: gravity (the world's), the dynamics of an articulated model that shares the world with free
+ * bodies (b2sim_enable_env_params refuses such a world), and the link-level inertial data of the loader (b2model_tables:
+ * link_com, which a wrench applied at a link's centre of mass uses, and total_mass).
+ *
+ * Free-body rows: [N, 10] for a B2_KIND_FREE model: mass, centre of mass xyz in the root-link frame, inertia about the
+ * centre of mass in root-link axes (xx xy xz yy yz zz), the record of one body of B2_BUF_BODY_INERTIA; every row starts
+ * from body_mass, body_com and body_Ic of b2model_tables. B2_ERR_UNSUPPORTED for any other kind of model. */
+int b2sim_enable_free_body_params(b2sim* s, int model, int enable, b2_buffer* out);
+/* Friction rows: [N, nshapes], column k = the Coulomb friction coefficient of collision shape k of b2model_tables in each
+ * env, starting from shape_mu[k]; for a free, static (ground plane, table) or articulated model (the finger pads). A
+ * contact's coefficient is the smaller of its two shapes' values in that env. Columns of shapes the contact stage does not
+ * use (cylinders, shapes beyond the per-body / per-model limits, shapes on links welded to the base) are kept and never
+ * read. B2_ERR_UNSUPPORTED for a model without collision shapes. */
+int b2sim_enable_shape_friction(b2sim* s, int model, int enable, b2_buffer* out);
 
 /* ---- custom controller: ComputedTorqueFixedBase run by ControllerRunner -------------------------------- */
 /* Model::insertModelPlugin("ControllerRunner", ...) with a <controller name="ComputedTorqueFixedBase"> context

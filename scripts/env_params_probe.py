@@ -12,7 +12,13 @@ the fingers held mid-range, 16,384 envs with the fingers driven into their lower
 damped rows (the dense constraint solve) and with undamped ones (the lane-parallel stage), 65,536 envs on k_task_panda. Last, the cost of redrawing every row of 16,384 envs once (the per-episode pattern: new
 rows after the step that reports done) with torch, against the step it precedes.
 
-    python scripts/env_params_probe.py [runs_per_block]
+Worlds with free bodies (Simulator.enable_free_body_params / enable_shape_friction), timed the same way: the pick scene's
+grasp step at 4,096 envs (the forked coupled pipeline), two stacked cubes at 4,096 envs (k_world_prepare / k_pgs_solve /
+k_world_finish) and at 65,536 envs (k_world_free). "on": the cubes' masses x U(0.8, 1.2), centres of mass within 2 mm,
+inertias x U(0.8, 1.2), and friction U(0.6, 1.2) on every shape that takes part (cube, table, finger pads; cubes, ground);
+"untouched": the same rows enabled and left at their initial values (the kernels' cost without a change of the physics).
+
+    python scripts/env_params_probe.py [runs_per_block] [all|world]
 """
 import os
 import subprocess
@@ -143,6 +149,91 @@ def reach(runs):
     env.close()
 
 
+def world_rows(sim, cubes, shaped, gen):
+    """Random free-body rows on `cubes` and friction rows on every model of `shaped` (rows "on")."""
+    import torch
+    for m in cubes:
+        rows = sim.enable_free_body_params(m)
+        opts = dict(device=rows.device, dtype=rows.dtype)
+        n = rows.shape[0]
+        s = 0.8 + 0.4 * torch.rand(n, 1, generator=gen, **opts)
+        rows[:, 0:1] *= s
+        rows[:, 1:4] = 0.002 * (2 * torch.rand(n, 3, generator=gen, **opts) - 1) / 3 ** 0.5
+        rows[:, 4:] *= s
+    for m in shaped:
+        mu = sim.enable_shape_friction(m)
+        mu.copy_(0.6 + 0.6 * torch.rand(mu.shape, generator=gen, device=mu.device, dtype=mu.dtype))
+
+
+def pick_world(n, rows_on, seed):
+    import torch
+    import b2sim
+    sc = b2sim.PandaPickScene(n, seed=seed)
+    if rows_on == "untouched":
+        sc.sim.enable_free_body_params(sc.cube)
+        for m in (sc.cube, sc.table, sc.panda):
+            sc.sim.enable_shape_friction(m)
+    elif rows_on:
+        gen = torch.Generator(device="cuda")
+        gen.manual_seed(seed)
+        world_rows(sc.sim, [sc.cube], [sc.cube, sc.table, sc.panda], gen)
+    sc.step(30)
+    sc.set_fingers(0.0)
+    sc.step(150)  # grasping from here on
+    return sc.sim, sc
+
+
+def stacked_world(n, rows_on, seed):
+    import torch
+    import b2sim
+    import gym_ignition_models
+    from b2sim import _lib as L
+    sim = b2sim.Simulator(n, 0.001, 1)
+    ground = sim.insert_model_file(gym_ignition_models.get_model_file("ground_plane"))
+    cube = """<robot name="cube"><link name="cube"><inertial><mass value="5.0"/>
+      <inertia ixx="0.0333" ixy="0" ixz="0" iyy="0.0333" iyz="0" izz="0.0333"/></inertial>
+      <collision><geometry><box size="0.2 0.2 0.2"/></geometry></collision></link></robot>"""
+    cubes = [sim.insert_model(cube, pose=(0, 0, z, 1, 0, 0, 0), name=f"c{k}") for k, z in enumerate((0.1, 0.3))]
+    if rows_on == "untouched":
+        for m in cubes:
+            sim.enable_free_body_params(m)
+        for m in [ground] + cubes:
+            sim.enable_shape_friction(m)
+    elif rows_on:
+        gen = torch.Generator(device="cuda")
+        gen.manual_seed(seed)
+        world_rows(sim, cubes, [ground] + cubes, gen)
+    for _ in range(300):  # settle
+        sim.run()
+    assert sim.tensor(cubes[1], L.BUF_BASE_STATE)[:, 2].min().item() > 0.25
+    return sim, None
+
+
+def worlds(runs):
+    import numpy as np
+    import torch
+    for name, n, kernels, make in (("pick grasp step", 4096, "forked coupled pipeline", pick_world),
+                                   ("two stacked cubes", 4096, "k_world_prepare/k_pgs_solve/k_world_finish", stacked_world),
+                                   ("two stacked cubes", 65536, "k_world_free", stacked_world)):
+        worlds_ = {"off": make(n, False, 3), "untouched": make(n, "untouched", 3), "on": make(n, True, 3)}
+        for sim, _ in worlds_.values():  # warm-up
+            for _ in range(100):
+                sim.run()
+        torch.cuda.synchronize()
+        times = {k: [] for k in worlds_}
+        for block in range(5):
+            for key, (sim, _) in worlds_.items():
+                times[key].append(timed(sim.run, runs))
+        med = {k: float(np.median(v)) for k, v in times.items()}
+        contacts = {k: np.mean([len(sim.contacts(e)) for e in range(0, n, max(1, n // 64))]) for k, (sim, _) in worlds_.items()}
+        print(f"world {name:17s} n={n:6d} {kernels:43s} " + "  ".join(
+            f"{k} {med[k]:8.2f} us/step (blocks {min(v):.2f}-{max(v):.2f}, {contacts[k]:.1f} contacts)"
+            for k, v in times.items()) + f"  untouched/off {med['untouched'] / med['off']:.3f}  on/off {med['on'] / med['off']:.3f}",
+            flush=True)
+        for sim, sc in worlds_.values():
+            (sc or sim).close()
+
+
 def main():
     sys.path.insert(0, ROOT)
     import __graft_entry__
@@ -150,7 +241,11 @@ def main():
     import numpy as np
     import torch
     runs = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
+    section = sys.argv[2] if len(sys.argv) > 2 else "all"
     print(f"card: {card()}", flush=True)
+    if section == "world":
+        worlds(max(1, runs // 5))
+        return
     for n, kernel in SIZES.items():
         sims = {"off": panda_sim(n, False, 3), "on": panda_sim(n, True, 3)}
         for sim in sims.values():  # warm-up: module loads, clocks
@@ -174,6 +269,7 @@ def main():
         for sim in sims.values():
             sim.close()
     reach(runs)
+    worlds(max(1, runs // 5))
 
 
 if __name__ == "__main__":
